@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: LightweightUNet de-glaring inference, images/sec (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
 
@@ -180,6 +180,24 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm), "source": "nvidia-smi -lms 100"}
 
 
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_output(d, y):
+    """Write the timed forward's output `y` [N,C,H,W] as <d>/output.npy, float32.  An output larger than DUMP_BYTES keeps its leading
+    images that fit (or, when one image does not, the leading rows of the first), so element [n,c,h,w] of the file is element [n,c,h,w]
+    of the output and two builds run with the same arguments compare element for element."""
+    import numpy as np
+    y = y.detach().float()
+    cap = (DUMP_BYTES - 4096) // 4     # elements; room for the .npy header
+    if y.numel() > cap:
+        per_image = y[0].numel()
+        y = y[:cap // per_image] if per_image <= cap else y[:1, :, :cap // (y.shape[1] * y.shape[3])]
+    y = y.cpu()
+    os.makedirs(d, exist_ok=True)
+    np.save(os.path.join(d, "output.npy"), y.numpy())
+
+
 ORT_NOTE = "onnxruntime unavailable \u2014 not installed, no network"
 
 
@@ -249,8 +267,10 @@ def run_reference(args, rank, world):
             fwd(x)
         t = time.perf_counter()
         for _ in range(args.steps):
-            fwd(x)
+            y = fwd(x)
         dt = time.perf_counter() - t
+    if args.dump_outputs:
+        dump_output(args.dump_outputs, y)
     rate = batch * args.steps / dt
     sample = (f"{args.steps} steps x {batch} images of 1x{args.hw}x{args.hw}, fp32, torch CPU {cores} threads"
               + ("" if batch == args.batch else f"; a bounded sample of the GPU arm's batch of {args.batch} (per-image CPU cost is flat in "
@@ -273,7 +293,7 @@ def run_reference(args, rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline forward (the side measurements use their own counts)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--storage", default="fp16", choices=["fp16", "bf16", "fp32"])
@@ -284,7 +304,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-train", action="store_true", help="skip the configs[3] training-step measurement")
     ap.add_argument("--no-extras", action="store_true", help="skip the configs[0] latency and configs[4] wide-variant side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the measurements, write what the last timed step computed (rank 0's "
+                    "output images, float32) as DIR/output.npy; above 64 MB, the leading images that fit")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -754,6 +778,8 @@ def main():
                         "batch1_ms": (1e3 / rate1 if rate1 else None),
                         "onnxruntime_cpu": onnxruntime_status()}
 
+    if rank == 0 and args.dump_outputs:
+        dump_output(args.dump_outputs, y)
     if rank == 0:
         print(json.dumps({
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": args.warmup,

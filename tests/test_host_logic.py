@@ -23,7 +23,13 @@ def test_library_exports_every_declared_symbol():
         assert hasattr(lib, name), f"{name} declared in include/deglare.h but not exported"
     assert declared == set(_lib.SYMBOLS), (declared ^ set(_lib.SYMBOLS))
     assert lib.dg_version() >= 100
-    assert lib.dg_launch_count() == 0  # nothing may launch without a GPU
+    # nothing may launch without a GPU; the counter is per process and GPU tests may already have run in this one, so it is read
+    # in a fresh process that sees no device
+    import subprocess
+    out = subprocess.run([sys.executable, "-c", "from image_enhancement_deglaring_b200 import _lib; print(_lib.load().dg_launch_count())"],
+                         cwd=ROOT, env={**os.environ, "CUDA_VISIBLE_DEVICES": ""}, capture_output=True, text=True, timeout=300)
+    assert out.returncode == 0, out.stderr[-500:]
+    assert int(out.stdout.split()[-1]) == 0
 
 
 def test_struct_layouts_match_header_sizes(tmp_path):

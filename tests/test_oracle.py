@@ -167,17 +167,24 @@ def test_optimized_train_step_oracle_matches_reference(golden):
         assert np.abs(got[:32] - g["gy_ghead/" + k]).max() <= 1e-9 + 1e-3 * np.abs(g["gy_ghead/" + k]).max(), k
 
 
-# ---- second oracle: the shipped ONNX artefact itself (what api/app.py:84,171 and evaluate.py:95,122 execute through onnxruntime) ------
-ONNX_PATH = "/root/reference/best_model.onnx"     # build container only; absent on the GPU box
-
-
-@pytest.mark.skipif(not os.path.exists(ONNX_PATH), reason="the reference mount (best_model.onnx) exists only in the build container")
-def test_onnx_artefact_interpreter_matches_reference_goldens(best_sd, golden):
+# ---- second oracle: the exported ONNX graph (what api/app.py:84,171 and evaluate.py:95,122 execute through onnxruntime) ----------
+def test_onnx_artefact_interpreter_matches_reference_goldens(best_sd, golden, tmp_path):
     """oracle/onnx_interp.py evaluates the exported graph (opset 11, 229 nodes, eleven operator types) with the ONNX operator
-    semantics: it must land on the outputs the reference MODULE produced (golden vectors), i.e. artefact == module == oracle."""
+    semantics: it must land on the outputs the reference MODULE produced (golden vectors), i.e. artefact == module == oracle.
+    The graph is tests/golden/make_onnx_golden.py's export of the reference module, stored without its weights; the initializers
+    are re-attached from weights/best_model.pth, each checked against the sha256 the export recorded."""
+    import hashlib
     from oracle.onnx_interp import OnnxGraph
-    g = OnnxGraph(ONNX_PATH)
-    assert g.opset == 11 and g.inputs == ["input"] and g.outputs == ["output"]
+    store = golden("onnx_graph.npz")
+    path = tmp_path / "best_model.onnx"
+    path.write_bytes(store["model"].tobytes())
+    g = OnnxGraph(str(path))
+    assert not g.inits
+    for name, key, shape, digest in zip(store["init_names"], store["init_keys"], store["init_shapes"], store["init_sha256"]):
+        v = best_sd[key].numpy().reshape([int(s) for s in shape.split(",")])
+        assert hashlib.sha256(v.astype("<f4").tobytes()).hexdigest() == digest, name
+        g.inits[name] = v
+    assert g.opset == 11 and g.inputs == ["input"] and g.outputs == ["output"] and len(g.nodes) == 229
     assert g.op_types() == ["Add", "AveragePool", "Concat", "Constant", "Conv", "ConvTranspose", "InstanceNormalization", "Mul",
                             "Reshape", "Shape", "Sigmoid"]
     png = golden("lw_png.npz")
@@ -202,9 +209,10 @@ def test_onnx_artefact_interpreter_matches_reference_goldens(best_sd, golden):
     with torch.no_grad():
         want = tpo.lightweight_forward(x, best_sd).numpy()
     assert np.abs(g.run(x.numpy()) - want).max() <= 1e-5
-    # the artefact's initializers are the 486,409 weights of weights/best_model.pth
+    # the initializers are the 486,409 weights of weights/best_model.pth, every state_dict entry exactly once
     named = {k: v for k, v in g.inits.items() if not k.startswith("onnx::")}
     assert sum(v.size for v in g.inits.values() if v.dtype == np.float32) == 486409
+    assert sorted(store["init_keys"]) == sorted(best_sd)
     for k, v in named.items():
         assert np.array_equal(v, best_sd[k].numpy()), k
 
