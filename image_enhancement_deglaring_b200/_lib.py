@@ -32,9 +32,7 @@ class DgConv3x3Args(C.Structure):
         ("src", DgSrc * 2), ("nsrc", C.c_int32), ("dtype", C.c_int32),
         ("N", C.c_int32), ("H", C.c_int32), ("W", C.c_int32), ("cout", C.c_int32),
         ("weight", C.c_void_p), ("weight_tc", C.c_void_p), ("out", C.c_void_p), ("out_stats", C.c_void_p),
-        ("act_sum", C.c_void_p), ("out_coef", C.c_void_p), ("out_counter", C.c_void_p), ("out_gamma", C.c_void_p),
-        ("out_beta", C.c_void_p), ("out_groups", C.c_int32), ("reserved", C.c_int32), ("eps", C.c_float),
-        ("path", C.c_int32), ("weight_comp", C.c_void_p),
+        ("act_sum", C.c_void_p), ("eps", C.c_float), ("path", C.c_int32), ("weight_comp", C.c_void_p),
     ]
 
 

@@ -48,6 +48,17 @@ static const char* const kConvNames[18] = {"enc1.0", "enc1.3", "enc2.0", "enc2.3
                                            "bottleneck.3", "up4+dec4.0", "dec4.3", "up3+dec3.0", "dec3.3", "up2+dec2.0", "dec2.3",
                                            "up1+dec1.0", "dec1.3"};
 
+// Path bits 2-6 selected kernel variants that measured slower and were removed.  A caller that still sets one gets an error rather
+// than different kernels than it asked for.
+constexpr int32_t kRemovedPathBits = 0x7c;
+static int check_path(int32_t path, const char* who) {
+    if (path & kRemovedPathBits) {
+        set_error("%s: path %d sets bit %d, whose kernel variant was removed", who, path, __builtin_ctz(path & kRemovedPathBits));
+        return 2;
+    }
+    return 0;
+}
+
 static int validate_src(const dg_src& s, const char* who) {
     if (s.raw == nullptr) { set_error("%s: null source pointer", who); return 2; }
     if (s.channels < 1) { set_error("%s: bad channel count %d", who, s.channels); return 2; }
@@ -70,9 +81,9 @@ static int validate_src(const dg_src& s, const char* who) {
 struct LwPlan {
     int f[5];
     int conv_c[18], conv_h[18], conv_w[18];
-    size_t raw_off[18], stats_off[18], counter_off[18], coef_off[18];
+    size_t raw_off[18], stats_off[18];
     size_t up_off[4];  // scratch for a materialised upconvK output (deep decoder levels, 16-bit storage)
-    size_t stats_bytes, total_bytes;  // stats_bytes = the zero-initialised prefix (statistics + arrival counters)
+    size_t stats_bytes, total_bytes;  // stats_bytes = the zero-initialised prefix (statistics)
 };
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -81,6 +92,7 @@ static inline int block_level(int b) { return b < 5 ? b : 8 - b; }
 
 static int make_plan(const dg_lw_params* p, int N, int H, int W, LwPlan* pl) {
     if (p == nullptr) { set_error("null params"); return 2; }
+    if (int rc = check_path(p->path, "lw")) return rc;
     if (N < 1 || H < 16 || W < 16 || (H % 16) || (W % 16)) {
         // 500x500 raises at the first torch.cat in the reference (src/model.py:116); here it is an error too
         set_error("input %dx%dx%d: H and W must be positive multiples of 16", N, H, W);
@@ -98,16 +110,8 @@ static int make_plan(const dg_lw_params* p, int N, int H, int W, LwPlan* pl) {
         pl->stats_off[i] = off;
         off += (size_t)N * pl->conv_c[i] * 2 * sizeof(double);
     }
-    for (int i = 0; i < 18; ++i) {
-        pl->counter_off[i] = off;
-        off += align_up((size_t)N * sizeof(int32_t), 8);
-    }
     pl->stats_bytes = off;
     off = align_up(off, 256);
-    for (int i = 0; i < 18; ++i) {
-        pl->coef_off[i] = off;
-        off += align_up((size_t)N * pl->conv_c[i] * 2 * sizeof(float), 256);
-    }
     for (int i = 0; i < 18; ++i) {
         pl->raw_off[i] = off;
         off += align_up((size_t)N * pl->conv_h[i] * pl->conv_w[i] * pl->conv_c[i] * dtype_size(p->dtype), 256);
@@ -124,10 +128,8 @@ static int make_plan(const dg_lw_params* p, int N, int H, int W, LwPlan* pl) {
 
 // Decoder levels whose ConvTranspose output is materialised by a stand-alone tensor-core GEMM (16-bit tiers) and read by the
 // consuming conv as an identity source: every level with C_up >= 32 -- upconv4 / upconv3 of the shipped model, ALL levels of the
-// wide variant (features_start = 64) -- plus upconv2 with path bit 5.  The concat itself is never stored.
-static inline bool lw_up_materialised(const dg_lw_params* p, const LwPlan& pl, int u) {
-    return pl.f[3 - u] >= 32 || (u == 2 && (p->path & 32));
-}
+// wide variant (features_start = 64).  The concat itself is never stored.
+static inline bool lw_up_materialised(const LwPlan& pl, int u) { return pl.f[3 - u] >= 32; }
 
 // n0: first image of the sub-batch the descriptor is for (every per-image tensor is contiguous over the batch)
 static dg_src gn_src(const dg_lw_params* p, const LwPlan& pl, char* ws, int conv_idx, int xform, int n0 = 0) {
@@ -137,10 +139,6 @@ static dg_src gn_src(const dg_lw_params* p, const LwPlan& pl, char* ws, int conv
     const size_t img = (size_t)pl.conv_h[conv_idx] * pl.conv_w[conv_idx] * pl.conv_c[conv_idx] * dtype_size(p->dtype);
     s.raw = ws + pl.raw_off[conv_idx] + (size_t)n0 * img;
     s.stats = reinterpret_cast<const double*>(ws + pl.stats_off[conv_idx]) + (size_t)n0 * pl.conv_c[conv_idx] * 2;
-    // path bit 4: producer-side GroupNorm finalisation.  Measured SLOWER on B200 (2.87 vs 2.74 ms/batch-64 forward): the
-    // threadfence + ticket keeps every producer CTA resident until its statistics atomics have landed, which costs more
-    // than the consumers' double-precision prologue saves.  Kept selectable for experiments; off by default.
-    s.coef = (p->path & 16) ? reinterpret_cast<const float*>(ws + pl.coef_off[conv_idx]) + (size_t)n0 * pl.conv_c[conv_idx] * 2 : nullptr;
     s.gamma = p->gn_w[b][j];
     s.beta = p->gn_b[b][j];
     s.channels = pl.conv_c[conv_idx];
@@ -169,11 +167,6 @@ static int lw_forward_range(const dg_lw_params* p, const LwPlan& pl, char* ws, c
         a.weight_tc = p->conv_w_tc[b][i % 2];
         a.out = ws + pl.raw_off[i] + (size_t)n0 * a.H * a.W * a.cout * esz;
         a.out_stats = reinterpret_cast<double*>(ws + pl.stats_off[i]) + (size_t)n0 * a.cout * 2;
-        a.out_coef = (p->path & 16) ? reinterpret_cast<float*>(ws + pl.coef_off[i]) + (size_t)n0 * a.cout * 2 : nullptr;
-        a.out_counter = reinterpret_cast<int32_t*>(ws + pl.counter_off[i]) + n0;
-        a.out_gamma = p->gn_w[b][i % 2];
-        a.out_beta = p->gn_b[b][i % 2];
-        a.out_groups = p->groups[b];
         a.eps = 1e-5f;
         a.path = p->path;
         a.nsrc = 1;
@@ -197,12 +190,12 @@ static int lw_forward_range(const dg_lw_params* p, const LwPlan& pl, char* ws, c
             a.src[1] = gn_src(p, pl, ws, 2 * lvl + 1, DG_X_SAME, n0);  // skip: torch.cat((up, skip), 1)
             a.nsrc = 2;
             a.weight_comp = p->dec_comp[u];
-            // deep levels (upconv4, upconv3; upconv2 with path bit 5): run the transposed conv as its own tensor-core GEMM and
+            // deep levels (upconv4, upconv3): run the transposed conv as its own tensor-core GEMM and
             // feed its output as an identity source -- see convt_tc.cu for why this beats fusing there
             // composite weights present for a level the tcgen05 decoder mode covers (C_up >= 16): ConvTranspose, concat and conv run
             // as one low-resolution conv in conv3x3_t5.cu -- no stand-alone ConvTranspose, no `up` tensor
             const bool dec_t5 = p->dec_comp[u] != nullptr && !(p->path & (128 | 1024)) && pl.f[lvl] >= 16;
-            const bool unfuse = p->dtype != DG_F32 && (p->path & 3) != 1 && lw_up_materialised(p, pl, u) && !dec_t5;
+            const bool unfuse = p->dtype != DG_F32 && (p->path & 3) != 1 && lw_up_materialised(pl, u) && !dec_t5;
             if (unfuse) {
                 bool handled = false;
                 void* up = ws + pl.up_off[u] + (size_t)n0 * a.H * a.W * pl.f[lvl] * esz;
@@ -247,7 +240,7 @@ static int lw_forward_range(const dg_lw_params* p, const LwPlan& pl, char* ws, c
 // 2.25 -> 2.09 ms per forward (two streams; four: 2.12); batch 32: 1.20 -> 1.08 ms, batch 16: 0.675 -> 0.599 ms, batch 8: no
 // change (hence the default threshold of 16).  Outputs are bit-identical (nothing depends on the batch size).
 struct FwdFork {
-    static constexpr int MAXF = 4;
+    static constexpr int MAXF = 2;   // the two halves of a batch
     bool ready = false;
     int device = -1;
     cudaStream_t s[MAXF];
@@ -445,20 +438,16 @@ static int lw_backward(const dg_lw_params* p, const float* x, const float* grad_
     if (e == cudaSuccess) e = cudaMemsetAsync(grads, 0, gl.total * sizeof(float), st);
     if (e != cudaSuccess) { set_error("memset: %s", cudaGetErrorString(e)); return 10; }
     const int split = g_split.load();
-    if (split > 0 && N >= split && N >= 2) {   // concurrent sub-batches, as in lw_forward (DG_BWD_FORKS = 2..4 of them; default 2)
+    if (split > 0 && N >= split && N >= 2) {   // two concurrent sub-batches, as in lw_forward
         if ((rc = fork_init())) return rc;
         FwdFork& F = g_forks[0];
-        static const int want = [] { const char* e = getenv("DG_BWD_FORKS"); const int v = e ? atoi(e) : 2; return v < 2 ? 2 : (v > FwdFork::MAXF ? FwdFork::MAXF : v); }();
-        const int nf = N >= 8 * want ? want : 2;
         cudaEventRecord(F.fork, st);
-        int n0 = 0;
-        for (int k = 0; k < nf; ++k) {
-            const int nn = (N - n0) / (nf - k);
+        const int half = N / 2;
+        for (int k = 0; k < 2; ++k) {
             cudaStreamWaitEvent(F.s[k], F.fork, 0);
-            rc = lw_backward_range(p, pl, bp, gl, x, grad_y, n0, nn, H, W, fw, bw, grads, F.s[k], l1);
+            rc = lw_backward_range(p, pl, bp, gl, x, grad_y, k ? half : 0, k ? N - half : half, H, W, fw, bw, grads, F.s[k], l1);
             cudaEventRecord(F.join[k], F.s[k]);
             cudaStreamWaitEvent(st, F.join[k], 0);
-            n0 += nn;
             if (rc) return rc;
         }
         return 0;
@@ -529,7 +518,7 @@ static int lw_backward_range(const dg_lw_params* p, const LwPlan& pl, const BwdP
             if (a.nsrc == 2) {
                 const int lvl = block_level(b), u = b - 5;
                 void* up = fw + pl.up_off[u] + (size_t)n0 * Hi * Wi * pl.f[lvl] * esz;
-                const bool have_up = lw_up_materialised(p, pl, u);
+                const bool have_up = lw_up_materialised(pl, u);
                 if (!have_up) {
                     rc = convt_tc_launch(a.src[0], p->dtype, N, Hi, Wi, up, 1e-5f, p->path, st, &ok);
                     if (rc) return rc;
@@ -721,6 +710,7 @@ uint64_t dg_launch_count(void) { return g_launches.load(std::memory_order_relaxe
 
 int dg_conv3x3_fused(const dg_conv3x3_args* a, dg_stream_t stream) {
     if (a == nullptr) { set_error("conv3x3: null args"); return 2; }
+    if (int rc = check_path(a->path, "conv3x3")) return rc;
     if (a->nsrc < 1 || a->nsrc > 2) { set_error("conv3x3: nsrc %d", a->nsrc); return 2; }
     if (a->N < 1 || a->H < 1 || a->W < 1 || a->cout < 1) { set_error("conv3x3: bad shape"); return 3; }
     if (a->weight == nullptr || a->out == nullptr) { set_error("conv3x3: null weight/out"); return 2; }
@@ -742,9 +732,6 @@ int dg_conv3x3_fused(const dg_conv3x3_args* a, dg_stream_t stream) {
         rc = conv3x3_t5_launch(*a, st, &handled);     // warp-specialised tcgen05 + TMEM kernel: every C_out >= 32 layer
         if (rc) return rc;
         if (handled) return 0;
-        rc = conv3x3_umma_launch(*a, st, &handled);   // round-1 tcgen05 kernel (opt-in, path bit 6)
-        if (rc) return rc;
-        if (handled) return 0;
         rc = conv3x3_dec_launch(*a, st, &handled);    // upconv1 + dec1.0 with the ConvTranspose folded into the conv taps
         if (rc) return rc;
         if (handled) return 0;
@@ -762,6 +749,7 @@ int dg_conv3x3_fused(const dg_conv3x3_args* a, dg_stream_t stream) {
 int dg_conv3x3_wgrad(const dg_conv3x3_args* a, const float* dR, float* dW, int32_t s_tap, int32_t s_ci, int32_t s_co,
                      dg_stream_t stream) {
     if (a == nullptr || dR == nullptr || dW == nullptr) { set_error("wgrad: null pointer"); return 2; }
+    if (int rc = check_path(a->path, "wgrad")) return rc;
     if (a->nsrc < 1 || a->nsrc > 2) { set_error("wgrad: nsrc %d", a->nsrc); return 2; }
     for (int s = 0; s < a->nsrc; ++s) {
         int rc = validate_src(a->src[s], "wgrad");
@@ -879,7 +867,9 @@ int dg_lw_forward(const dg_lw_params* p, const float* x, float* y, int32_t N, in
 int dg_convt2x2_fused(const dg_src* src, int32_t dtype, int32_t N, int32_t H, int32_t W, void* out, float eps, int32_t path,
                       dg_stream_t stream) {
     if (src == nullptr || out == nullptr || N < 1 || H < 2 || W < 2) { set_error("convt2x2: bad arguments"); return 2; }
-    int rc = validate_src(*src, "convt2x2");
+    int rc = check_path(path, "convt2x2");
+    if (rc) return rc;
+    rc = validate_src(*src, "convt2x2");
     if (rc) return rc;
     bool handled = false;
     rc = convt_tc_launch(*src, dtype, N, H, W, out, eps, path, reinterpret_cast<cudaStream_t>(stream), &handled);

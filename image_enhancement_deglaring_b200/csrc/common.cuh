@@ -122,41 +122,6 @@ __device__ __forceinline__ void gn_coef(const double* __restrict__ stats, const 
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;"); }
 
-// ---- producer-side GroupNorm finalisation --------------------------------------------------------------------------
-// Every CTA of a conv adds its partial (sum, sumsq) to stats[n] with double atomics; the CTA that arrives last at the
-// per-image counter (threadfence + atomic ticket) sees the complete sums and writes the affine (a, b) of the GroupNorm
-// that follows, so consumer CTAs start with two float loads per channel instead of a double-precision prologue.
-__device__ __forceinline__ bool last_cta_of_image(int* counter, int ctas_per_image) {
-    __shared__ int s_last;
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) s_last = (atomicAdd(counter, 1) == ctas_per_image - 1) ? 1 : 0;
-    __syncthreads();
-    return s_last != 0;
-}
-
-__device__ __forceinline__ void gn_finalize(const double* stats, const float* __restrict__ gamma, const float* __restrict__ beta,
-                                            int n, int C, int groups, double plane, float eps, float* __restrict__ coef) {
-    __threadfence();
-    const int cpg = C / groups;
-    for (int c = threadIdx.x; c < C; c += blockDim.x) {
-        const int g0 = (c / cpg) * cpg;
-        double s1 = 0.0, s2 = 0.0;
-        for (int k = 0; k < cpg; ++k) {
-            s1 += __ldcg(stats + (size_t)(n * C + g0 + k) * 2);
-            s2 += __ldcg(stats + (size_t)(n * C + g0 + k) * 2 + 1);
-        }
-        const double cnt = plane * cpg;
-        const double mean = s1 / cnt;
-        double var = s2 / cnt - mean * mean;
-        if (var < 0.0) var = 0.0;
-        const double rstd = rsqrt(var + (double)eps);
-        const double a = rstd * (double)gamma[c];
-        coef[(size_t)(n * C + c) * 2] = (float)a;
-        coef[(size_t)(n * C + c) * 2 + 1] = (float)((double)beta[c] - mean * a);
-    }
-}
-
 }  // namespace dg
 
 // ---- host side ---------------------------------------------------------------------------
@@ -183,7 +148,6 @@ int check_launch(const char* what);
 int conv3x3_generic_launch(const dg_conv3x3_args& a, cudaStream_t stream);
 int conv3x3_tc_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* handled);
 int conv_first_tc_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* handled);
-int conv3x3_umma_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* handled);
 int conv3x3_t5_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* handled);
 int conv3x3_ring_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* handled);
 int conv3x3_dec_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* handled);

@@ -79,7 +79,7 @@ __device__ __forceinline__ void dc_mbar_wait(uint32_t bar, uint32_t parity) {
     }
 }
 
-template <typename T, int ACT>
+template <typename T>
 __global__ void __launch_bounds__(DC_THREADS, 2) dec8_ring_kernel(const __grid_constant__ DecArgs p) {
     extern __shared__ __align__(1024) unsigned char smem[];
     unsigned char* sact = smem + DC_OFF_SACT;
@@ -94,8 +94,6 @@ __global__ void __launch_bounds__(DC_THREADS, 2) dec8_ring_kernel(const __grid_c
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int cb = warp & 1, rb = warp >> 1;      // warp tile: output rows 4 rb .. 4 rb + 3, columns 32 cb .. 32 cb + 31
     const int H = p.H, W = p.W, Hl = H >> 1, Wl = W >> 1;
-    constexpr int FACT = ACT == ACT_HALF2 ? ACT_TANH : ACT;
-    constexpr bool H2 = ACT == ACT_HALF2 && std::is_same<T, __half>::value;   // packed-half affine + tanh + fma
 
     pdl_launch_dependents();
     if (tid == 0) {
@@ -202,7 +200,7 @@ __global__ void __launch_bounds__(DC_THREADS, 2) dec8_ring_kernel(const __grid_c
                 float a, b;
                 if (tid < DC_CL) gn_coef(p.st_l, p.g_l, p.b_l, n, DC_CL, p.groups_l, tid, (double)Hl * Wl, p.eps, a, b);
                 else gn_coef(p.st_s, p.g_s, p.b_s, n, DC_CU, p.groups_s, tid - DC_CL, (double)H * W, p.eps, a, b);
-                if constexpr (FACT != ACT_EXACT) { a *= 0.5f; b *= 0.5f; }
+                a *= 0.5f; b *= 0.5f;
                 coef[tid] = make_float2(a, b);
             }
             cur_n = n;
@@ -214,18 +212,9 @@ __global__ void __launch_bounds__(DC_THREADS, 2) dec8_ring_kernel(const __grid_c
         const unsigned char* lraw = sraw + DC_OFF_LRAW;
         const bool interior = y0 >= 2 && x0 >= 2 && y0 + DC_TH + 2 <= H && x0 + DC_TW + 2 <= W;
         {   // skip: 18 x 66 pixels, de-interleaved by column parity (global x = x0 - 1 + c; x0 is even)
-            float2 cf[H2 ? 1 : 8];
-            uint32_t ah[H2 ? 4 : 1], bh[H2 ? 4 : 1];
-            if constexpr (H2) {
+            float2 cf[8];
 #pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    ah[e] = pack2<__half>(coef[DC_CL + 2 * e].x, coef[DC_CL + 2 * e + 1].x);
-                    bh[e] = pack2<__half>(coef[DC_CL + 2 * e].y, coef[DC_CL + 2 * e + 1].y);
-                }
-            } else {
-#pragma unroll
-                for (int e = 0; e < 8; ++e) cf[e] = coef[DC_CL + e];
-            }
+            for (int e = 0; e < 8; ++e) cf[e] = coef[DC_CL + e];
             constexpr int NPIX = DC_PH * DC_PW;
             constexpr int SLOTS = (NPIX + DC_THREADS - 1) / DC_THREADS;   // 5
             uint4 q[SLOTS];
@@ -243,31 +232,18 @@ __global__ void __launch_bounds__(DC_THREADS, 2) dec8_ring_kernel(const __grid_c
                 if (!interior) ok = (unsigned)(y0 - 1 + r) < (unsigned)H && (unsigned)(x0 - 1 + c) < (unsigned)W;
                 uint4 o = make_uint4(0u, 0u, 0u, 0u);
                 if (ok) {
-                    if constexpr (H2) {
-                        o = act8_h2(q[i], ah, bh);
-                    } else {
-                        float yv[8];
-                        act8<T, FACT>(q[i], cf, yv);
-                        o = pack8<T>(yv);
-                    }
+                    float yv[8];
+                    act8<T>(q[i], cf, yv);
+                    o = pack8<T>(yv);
                 }
                 *reinterpret_cast<uint4*>(sact + ((c & 1) ^ 1) * DC_SPLANE + (r * DC_SW + ((c + 1) >> 1)) * 16) = o;
             }
         }
         {   // low: 10 x 34 pixels x 2 chunks of 8 channels -> two channel planes
             const int c8 = tid & 1;
-            float2 cf[H2 ? 1 : 8];
-            uint32_t ah[H2 ? 4 : 1], bh[H2 ? 4 : 1];
-            if constexpr (H2) {
+            float2 cf[8];
 #pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    ah[e] = pack2<__half>(coef[c8 * 8 + 2 * e].x, coef[c8 * 8 + 2 * e + 1].x);
-                    bh[e] = pack2<__half>(coef[c8 * 8 + 2 * e].y, coef[c8 * 8 + 2 * e + 1].y);
-                }
-            } else {
-#pragma unroll
-                for (int e = 0; e < 8; ++e) cf[e] = coef[c8 * 8 + e];
-            }
+            for (int e = 0; e < 8; ++e) cf[e] = coef[c8 * 8 + e];
             constexpr int NSL = DC_LH * DC_LW * 2;                          // 680
             constexpr int SLOTS = (NSL + DC_THREADS - 1) / DC_THREADS;     // 3
             uint4 q[SLOTS];
@@ -288,13 +264,9 @@ __global__ void __launch_bounds__(DC_THREADS, 2) dec8_ring_kernel(const __grid_c
                 }
                 uint4 o = make_uint4(0u, 0u, 0u, 0u);
                 if (ok) {
-                    if constexpr (H2) {
-                        o = act8_h2(q[i], ah, bh);
-                    } else {
-                        float yv[8];
-                        act8<T, FACT>(q[i], cf, yv);
-                        o = pack8<T>(yv);
-                    }
+                    float yv[8];
+                    act8<T>(q[i], cf, yv);
+                    o = pack8<T>(yv);
                 }
                 *reinterpret_cast<uint4*>(lact + c8 * DC_LPLANE + lp * 16) = o;
             }
@@ -457,9 +429,9 @@ __global__ void pack_dec_composite_kernel(const float* __restrict__ ct_w, const 
     }
 }
 
-template <typename T, int ACT>
+template <typename T>
 int launch_dec(const DecArgs& a, cudaStream_t st) {
-    auto kern = dec8_ring_kernel<T, ACT>;
+    auto kern = dec8_ring_kernel<T>;
     static bool done = false;
     if (!done) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, DC_SMEM);
@@ -603,12 +575,7 @@ int conv3x3_dec_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* hand
     if (total > 0x7fffffffLL) return 0;
     r.total = (int)total;
     *handled = true;
-    const int flavour = (a.path >> 2) & 3;
-    if (a.dtype == DG_F16) {
-        if (flavour == 2) return launch_dec<__half, ACT_HALF2>(r, stream);
-        return flavour == 1 ? launch_dec<__half, ACT_EXACT>(r, stream) : launch_dec<__half, ACT_TANH>(r, stream);
-    }
-    return flavour == 1 ? launch_dec<__nv_bfloat16, ACT_EXACT>(r, stream) : launch_dec<__nv_bfloat16, ACT_TANH>(r, stream);
+    return a.dtype == DG_F16 ? launch_dec<__half>(r, stream) : launch_dec<__nv_bfloat16>(r, stream);
 }
 
 }  // namespace dg

@@ -385,10 +385,6 @@ __global__ void __launch_bounds__(NTHREADS) conv3x3_generic_kernel(const dg_conv
             const int co = co_cta + (tid >> 1);
             if (co < Cout) atomicAdd(p.out_stats + ((size_t)n * Cout + co) * 2 + (tid & 1), statsm[tid]);
         }
-        if (p.out_coef != nullptr && p.out_counter != nullptr && p.out_gamma != nullptr && p.out_groups > 0) {
-            if (last_cta_of_image(p.out_counter + n, gridDim.x * gridDim.y * cfg.cobatches))
-                gn_finalize(p.out_stats, p.out_gamma, p.out_beta, n, Cout, p.out_groups, (double)H * W, p.eps, p.out_coef);
-        }
     }
 }
 

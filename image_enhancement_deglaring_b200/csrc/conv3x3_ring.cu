@@ -59,7 +59,7 @@ __device__ __forceinline__ void rg_mbar_wait(uint32_t bar, uint32_t parity) {
     }
 }
 
-template <typename T, int ACT>
+template <typename T>
 __global__ void __launch_bounds__(RG_THREADS, 3) conv8_ring_kernel(const __grid_constant__ RingArgs p) {
     extern __shared__ __align__(1024) unsigned char smem[];
     float2* coef = reinterpret_cast<float2*>(smem + RG_OFF_COEF);
@@ -70,8 +70,6 @@ __global__ void __launch_bounds__(RG_THREADS, 3) conv8_ring_kernel(const __grid_
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int seg = warp & 3, rb = warp >> 2;
     const int H = p.H, W = p.W;
-    constexpr int FACT = ACT == ACT_HALF2 ? ACT_TANH : ACT;
-    constexpr bool H2 = ACT == ACT_HALF2 && std::is_same<T, __half>::value;
 
     pdl_launch_dependents();
     if (tid == 0) {
@@ -151,7 +149,7 @@ __global__ void __launch_bounds__(RG_THREADS, 3) conv8_ring_kernel(const __grid_
                 float a, b;
                 if (p.cf) { a = __ldg(p.cf + (size_t)(n * RG_C + tid) * 2); b = __ldg(p.cf + (size_t)(n * RG_C + tid) * 2 + 1); }
                 else gn_coef(p.st, p.g, p.b, n, RG_C, p.groups, tid, (double)H * W, p.eps, a, b);
-                if constexpr (FACT != ACT_EXACT) { a *= 0.5f; b *= 0.5f; }
+                a *= 0.5f; b *= 0.5f;
                 coef[tid] = make_float2(a, b);
             }
             cur_n = n;
@@ -161,18 +159,9 @@ __global__ void __launch_bounds__(RG_THREADS, 3) conv8_ring_kernel(const __grid_
         rg_mbar_wait(bar0 + 8 * stage, (uint32_t)((k / RG_NS) & 1));
         unsigned char* act = smem + stage * RG_STAGE_BYTES;
         {
-            float2 cf[H2 ? 1 : 8];
-            uint32_t ah[H2 ? 4 : 1], bh[H2 ? 4 : 1];
-            if constexpr (H2) {
+            float2 cf[8];
 #pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    ah[e] = pack2<__half>(coef[2 * e].x, coef[2 * e + 1].x);
-                    bh[e] = pack2<__half>(coef[2 * e].y, coef[2 * e + 1].y);
-                }
-            } else {
-#pragma unroll
-                for (int e = 0; e < 8; ++e) cf[e] = coef[e];
-            }
+            for (int e = 0; e < 8; ++e) cf[e] = coef[e];
             const bool interior = y0 >= 1 && x0 >= 1 && y0 + RG_TH + 1 <= H && x0 + RG_TW + 1 <= W;
             constexpr int NPIX = RG_PH * RG_PW;
             constexpr int SLOTS = (NPIX + RG_THREADS - 1) / RG_THREADS;   // 5
@@ -192,13 +181,9 @@ __global__ void __launch_bounds__(RG_THREADS, 3) conv8_ring_kernel(const __grid_
                     ok = (unsigned)(y0 - 1 + r) < (unsigned)H && (unsigned)(x0 - 1 + c) < (unsigned)W;
                 }
                 if (ok) {
-                    if constexpr (H2) {
-                        *reinterpret_cast<uint4*>(act + px * 16) = act8_h2(q[i], ah, bh);
-                    } else {
-                        float yv[8];
-                        act8<T, FACT>(q[i], cf, yv);
-                        *reinterpret_cast<uint4*>(act + px * 16) = pack8<T>(yv);
-                    }
+                    float yv[8];
+                    act8<T>(q[i], cf, yv);
+                    *reinterpret_cast<uint4*>(act + px * 16) = pack8<T>(yv);
                 }
             }
         }
@@ -255,9 +240,9 @@ __global__ void __launch_bounds__(RG_THREADS, 3) conv8_ring_kernel(const __grid_
     if (cur_n >= 0) flush_stats(cur_n);
 }
 
-template <typename T, int ACT>
+template <typename T>
 int launch_ring(const RingArgs& a, cudaStream_t st) {
-    auto kern = conv8_ring_kernel<T, ACT>;
+    auto kern = conv8_ring_kernel<T>;
     static bool done = false;
     if (!done) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, RG_SMEM);
@@ -289,7 +274,6 @@ int conv3x3_ring_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* han
     const dg_src& s0 = a.src[0];
     if (s0.xform != DG_X_SAME || s0.channels != RG_C || s0.stats == nullptr || !s0.silu || s0.scale != nullptr) return 0;
     if ((reinterpret_cast<uintptr_t>(s0.raw) | reinterpret_cast<uintptr_t>(a.out) | reinterpret_cast<uintptr_t>(a.weight_tc)) & 15) return 0;
-    if (a.out_coef != nullptr && (a.path & 16)) return 0;   // producer-side finalisation stays with the per-tile kernel
     RingArgs r;
     memset(&r, 0, sizeof(r));
     if (!tma_map_nhwc16(&r.tmap, s0.raw, a.N, a.H, a.W, RG_PW, RG_PH)) return 0;   // no driver entry point: per-tile kernel
@@ -302,12 +286,7 @@ int conv3x3_ring_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* han
     if (total > 0x7fffffffLL) return 0;
     r.total = (int)total;
     *handled = true;
-    const int flavour = (a.path >> 2) & 3;
-    if (a.dtype == DG_F16) {
-        if (flavour == 2) return launch_ring<__half, ACT_HALF2>(r, stream);
-        return flavour == 1 ? launch_ring<__half, ACT_EXACT>(r, stream) : launch_ring<__half, ACT_TANH>(r, stream);
-    }
-    return flavour == 1 ? launch_ring<__nv_bfloat16, ACT_EXACT>(r, stream) : launch_ring<__nv_bfloat16, ACT_TANH>(r, stream);
+    return a.dtype == DG_F16 ? launch_ring<__half>(r, stream) : launch_ring<__nv_bfloat16>(r, stream);
 }
 
 }  // namespace dg

@@ -85,7 +85,6 @@ struct T5Args {
     int cl;           // T5_DEC: channels of the low-resolution source
     const float* bias;   // T5_CONVT: [cu];  T5_DEC: [9 border kinds][cu] ConvTranspose bias seen through the valid conv taps
     int items;
-    int dbg;
     long long* trace;   // DG_T5_TRACE=1: per-role clock64 timestamps of CTA 0 (debug aid, see t5_trace_dump)
 };
 
@@ -223,11 +222,10 @@ __device__ __forceinline__ T5Item t5_item(const T5Args& p, int item) {
     return it;
 }
 
-template <typename T, int MODE, int ACT>
+template <typename T, int MODE>
 __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_constant__ T5Args p) {
     extern __shared__ __align__(1024) unsigned char smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    constexpr int FACT = ACT == ACT_HALF2 ? ACT_TANH : ACT;
 
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + p.off_bar);
     // barrier table: a_full[R] a_empty[R] b_full[R] b_empty[R] t_full[2] t_empty[2], R = T5_MAX_RING
@@ -330,7 +328,7 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
                         const int ky = p.ntaps == 1 ? 1 : tap / 3, kx = p.ntaps == 1 ? 1 : tap - ky * 3;
                         const uint64_t da = da_chunk + (uint32_t)(ky * p.pitch + kx);
                         const uint64_t db = t5_desc(b_base + (uint32_t)sb * p.b_stage_bytes, (uint32_t)p.nb * 16u, 128);
-                        if (cnt > 0 && !(p.dbg & 1)) {
+                        if (cnt > 0) {
                             const uint32_t acc = (ch | tap) ? 1u : 0u;
                             const uint32_t dc0 = dcol + (uint32_t)(mw * p.nb);
                             const uint64_t da0 = da + (uint32_t)(mw * 128);
@@ -404,7 +402,7 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
             mbar_wait_relaxed(T_FULL(tsg), tph);
             tc_fence_after();
             if (warp == T5_EPI_WARP0 && lane == 0) T5_TRACE(1, 2 * k);
-            for (int m = 0; m < ((p.dbg & 2) ? 0 : it.mt_cur); ++m) {
+            for (int m = 0; m < it.mt_cur; ++m) {
                 const int q = (it.m0 + m) * 128 + wq * 32 + lane;
                 const int y = q / p.pitch, xl = q - y * p.pitch, x = it.xs + xl;
                 const bool valid = xl < p.tw && x < p.W && y < p.H;
@@ -605,22 +603,11 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
                 if (cu.c >= p.pitch) { cu.c -= p.pitch; cu.r += 1; }
             }
         };
-        constexpr bool H2 = ACT == ACT_HALF2 && std::is_same<T, __half>::value && MODE != T5_POOL;   // packed-half affine + tanh + fma
-        float2 cf[H2 ? 1 : 8];
-        uint32_t ah[H2 ? 4 : 1], bh[H2 ? 4 : 1];
+        float2 cf[8];
         auto load_coefs = [&](const Job& jb) {
             if (jb.ident) return;
-            if constexpr (H2) {
 #pragma unroll
-                for (int e = 0; e < 4; ++e) {
-                    const float2 c0 = coef[jb.cs + 2 * e], c1 = coef[jb.cs + 2 * e + 1];
-                    ah[e] = pack2<__half>(c0.x, c1.x);
-                    bh[e] = pack2<__half>(c0.y, c1.y);
-                }
-            } else {
-#pragma unroll
-                for (int e = 0; e < 8; ++e) cf[e] = coef[jb.cs + e];
-            }
+            for (int e = 0; e < 8; ++e) cf[e] = coef[jb.cs + e];
         };
         auto proc_batch = [&](const Job& jb, const Batch& q, unsigned char* dst) {
 #pragma unroll
@@ -630,16 +617,14 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
                 if (q.ok[b]) {
                     if (jb.ident) {
                         o = q.v[b][0];
-                    } else if constexpr (H2) {
-                        o = act8_h2(q.v[b][0], ah, bh);
                     } else {
                         float yv[8];
-                        act8<T, FACT>(q.v[b][0], cf, yv);
+                        act8<T>(q.v[b][0], cf, yv);
                         if constexpr (MODE == T5_POOL) {
                             float t[8];
 #pragma unroll
                             for (int j = 1; j < 4; ++j) {
-                                act8<T, FACT>(q.v[b][j], cf, t);
+                                act8<T>(q.v[b][j], cf, t);
 #pragma unroll
                                 for (int e = 0; e < 8; ++e) yv[e] += t[e];
                             }
@@ -649,8 +634,7 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
                         o = pack8<T>(yv);
                     }
                 }
-                if (!(p.dbg & 4)) *reinterpret_cast<uint4*>(dst + (size_t)q.ss[b] * 16) = o;
-                else if (o.x == 0x12345u) *reinterpret_cast<uint4*>(dst + (size_t)q.ss[b] * 16) = o;
+                *reinterpret_cast<uint4*>(dst + (size_t)q.ss[b] * 16) = o;
             }
         };
         auto ensure_coefs = [&](int n, int& coef_n) {
@@ -670,7 +654,7 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
                     if (p.cf0) { a = __ldg(p.cf0 + (size_t)(n * p.ncoef + c) * 2); b = __ldg(p.cf0 + (size_t)(n * p.ncoef + c) * 2 + 1); }
                     else gn_coef(p.st0, p.g0, p.b0, n, p.ncoef, p.groups0, c, plane, p.eps, a, b);
                 }
-                if constexpr (FACT != ACT_EXACT) { a *= 0.5f; b *= 0.5f; }
+                a *= 0.5f; b *= 0.5f;
                 coef[c] = make_float2(a, b);
             }
             coef_n = n;
@@ -813,9 +797,9 @@ void t5_trace_dump(const T5Args& t, long long* dev, cudaStream_t st) {
                 h[1024 + 4 * k + 1] - t0, h[1024 + 4 * k + 2] - t0, h[1024 + 4 * k + 3] - t0, h[1536 + 2 * k] - t0, h[1536 + 2 * k + 1] - t0);
 }
 
-template <typename T, int MODE, int ACT>
+template <typename T, int MODE>
 int launch_t5(const T5Args& t, cudaStream_t st) {
-    auto kern = conv3x3_t5_kernel<T, MODE, ACT>;
+    auto kern = conv3x3_t5_kernel<T, MODE>;
     static bool done = false;
     if (!done) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
@@ -839,13 +823,13 @@ int launch_t5(const T5Args& t, cudaStream_t st) {
     return check_launch("conv3x3_t5");
 }
 
-template <typename T, int ACT>
+template <typename T>
 int dispatch_t5(const T5Args& t, int mode, cudaStream_t st) {
-    if (mode == T5_SAME) return launch_t5<T, T5_SAME, ACT>(t, st);
-    if (mode == T5_POOL) return launch_t5<T, T5_POOL, ACT>(t, st);
-    if (mode == T5_CONVT) return launch_t5<T, T5_CONVT, ACT>(t, st);
-    if (mode == T5_DEC) return launch_t5<T, T5_DEC, ACT>(t, st);
-    return launch_t5<T, T5_CAT2, ACT>(t, st);
+    if (mode == T5_SAME) return launch_t5<T, T5_SAME>(t, st);
+    if (mode == T5_POOL) return launch_t5<T, T5_POOL>(t, st);
+    if (mode == T5_CONVT) return launch_t5<T, T5_CONVT>(t, st);
+    if (mode == T5_DEC) return launch_t5<T, T5_DEC>(t, st);
+    return launch_t5<T, T5_CAT2>(t, st);
 }
 }  // namespace
 
@@ -910,14 +894,8 @@ int conv3x3_t5_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* handl
     // measured on par or faster (enc3.0 0.071 vs 0.100 ms, enc3.3 0.079 vs 0.083 ms at batch 64); the concat conv (K = 576) wins here
     if (!forced && a.cout == 32 && mode != T5_CAT2 && mode != T5_DEC) return 0;
     if (!t5_plan(t, mode)) return decline("shape does not fit the tcgen05 plan");
-    { const char* e = getenv("DG_T5_DBG"); t.dbg = e ? atoi(e) : 0; }
     *handled = true;
-    const int flavour = (a.path >> 2) & 3;
-    if (a.dtype == DG_F16) {
-        if (flavour == 2) return dispatch_t5<__half, ACT_HALF2>(t, mode, stream);
-        return flavour == 1 ? dispatch_t5<__half, ACT_EXACT>(t, mode, stream) : dispatch_t5<__half, ACT_TANH>(t, mode, stream);
-    }
-    return flavour == 1 ? dispatch_t5<__nv_bfloat16, ACT_EXACT>(t, mode, stream) : dispatch_t5<__nv_bfloat16, ACT_TANH>(t, mode, stream);
+    return a.dtype == DG_F16 ? dispatch_t5<__half>(t, mode, stream) : dispatch_t5<__nv_bfloat16>(t, mode, stream);
 }
 
 
@@ -944,10 +922,7 @@ int convt_t5_launch(const dg_src& s, int dtype, int N, int H, int W, void* out, 
     t.cu = s.ct_cout;
     if (!t5_plan(t, T5_CONVT)) return 0;
     *handled = true;
-    const int flavour = (path >> 2) & 3;
-    if (dtype == DG_F16)
-        return flavour == 1 ? dispatch_t5<__half, ACT_EXACT>(t, T5_CONVT, st) : dispatch_t5<__half, ACT_TANH>(t, T5_CONVT, st);
-    return flavour == 1 ? dispatch_t5<__nv_bfloat16, ACT_EXACT>(t, T5_CONVT, st) : dispatch_t5<__nv_bfloat16, ACT_TANH>(t, T5_CONVT, st);
+    return dtype == DG_F16 ? dispatch_t5<__half>(t, T5_CONVT, st) : dispatch_t5<__nv_bfloat16>(t, T5_CONVT, st);
 }
 
 
@@ -1018,7 +993,7 @@ int convt_dgrad_t5_launch(const float* dCat, int stride, void* scratch_bf16, con
     int rc = check_launch("up_half_pos_bf16");
     if (rc) return rc;
     *handled = true;
-    return launch_t5<__nv_bfloat16, T5_IDENT, ACT_TANH>(t, st);
+    return launch_t5<__nv_bfloat16, T5_IDENT>(t, st);
 }
 
 int conv3x3_dgrad_t5_launch(const float* dR, const void* dR_bf16, void* scratch_bf16, const void* wflip_tc_bf16, float* out, int N,
@@ -1048,7 +1023,7 @@ int conv3x3_dgrad_t5_launch(const float* dR, const void* dR_bf16, void* scratch_
         if (rc) return rc;
     }
     *handled = true;
-    return launch_t5<__nv_bfloat16, T5_IDENT, ACT_TANH>(t, st);
+    return launch_t5<__nv_bfloat16, T5_IDENT>(t, st);
 }
 
 }  // namespace dg

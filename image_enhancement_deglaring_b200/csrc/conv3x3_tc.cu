@@ -36,7 +36,6 @@ struct TcArgs {
     void* out; double* out_stats;
     int N, H, W; float eps;
     const float* cf0; const float* cf1;   // optional finished (a, b) of src0 / src1 ([N,C,2]), else computed from st0 / st1
-    float* out_coef; int* out_counter; const float* out_gamma; const float* out_beta; int out_groups;
 };
 
 // ---- compile-time geometry -------------------------------------------------------------------------
@@ -120,7 +119,7 @@ struct Geo {
 // SYNC_FIRST: the GroupNorm coefficients `cfs` are still being written by other threads when this is called; the CTA barrier
 // that publishes them is taken here, AFTER the first batch of global loads has been issued, so the coefficient chain
 // (statistics load -> double math -> shared memory) and the first tile loads overlap instead of running back to back.
-template <typename T, typename G, int C, bool POOL, int ACT, bool IDENT = false, bool SYNC_FIRST = false>
+template <typename T, typename G, int C, bool POOL, bool IDENT = false, bool SYNC_FIRST = false>
 __device__ __forceinline__ void stage_planes(unsigned char* act, const unsigned char* __restrict__ src,
                                              const float2* __restrict__ cfs, int plane0, int y0, int x0, int H, int W) {
     constexpr int NC = C / 8;
@@ -131,25 +130,13 @@ __device__ __forceinline__ void stage_planes(unsigned char* act, const unsigned 
     constexpr int ITERS = (NSLOT + MAXB - 1) / MAXB;
     constexpr int BATCH = (NSLOT + ITERS - 1) / ITERS;
     constexpr int DR = PSTRIDE / G::PW, DC = PSTRIDE % G::PW;      // slot-to-slot advance of (row, column)
-    constexpr bool H2 = (ACT == ACT_HALF2) && !POOL && std::is_same<T, __half>::value;
-    constexpr int FACT = H2 ? ACT_TANH : ACT;                      // float flavour used when half2 does not apply
     static_assert(G::THREADS % NC == 0, "chunk ownership");
     const int c8 = threadIdx.x % NC;
     const int p0 = threadIdx.x / NC;
-    float2 cf[H2 ? 1 : 8];
-    uint32_t ah[H2 ? 4 : 1], bh[H2 ? 4 : 1];
+    float2 cf[8];
     auto read_coefs = [&]() {
-        if constexpr (H2) {
 #pragma unroll
-            for (int k = 0; k < 4; ++k) {
-                const float2 c0 = cfs[c8 * 8 + 2 * k], c1 = cfs[c8 * 8 + 2 * k + 1];
-                ah[k] = pack2<__half>(c0.x, c1.x);
-                bh[k] = pack2<__half>(c0.y, c1.y);
-            }
-        } else {
-#pragma unroll
-            for (int k = 0; k < 8; ++k) cf[k] = cfs[c8 * 8 + k];
-        }
+        for (int k = 0; k < 8; ++k) cf[k] = cfs[c8 * 8 + k];
     };
     if constexpr (!SYNC_FIRST && !IDENT) read_coefs();
     unsigned char* dst = act + (size_t)(plane0 + c8) * G::PLANE * 16;
@@ -200,16 +187,14 @@ __device__ __forceinline__ void stage_planes(unsigned char* act, const unsigned 
                 if (ok[b]) {
                     if constexpr (IDENT) {
                         o = q[b][0];  // already-final values (materialised ConvTranspose output): plain copy
-                    } else if constexpr (H2) {
-                        o = act8_h2(q[b][0], ah, bh);
                     } else {
                         float y[8];
-                        act8<T, FACT>(q[b][0], cf, y);
+                        act8<T>(q[b][0], cf, y);
                         if constexpr (POOL) {
                             float t[8];
 #pragma unroll
                             for (int j = 1; j < 4; ++j) {
-                                act8<T, FACT>(q[b][j], cf, t);
+                                act8<T>(q[b][j], cf, t);
 #pragma unroll
                                 for (int k = 0; k < 8; ++k) y[k] += t[k];
                             }
@@ -227,7 +212,7 @@ __device__ __forceinline__ void stage_planes(unsigned char* act, const unsigned 
     else run(std::false_type{});
 }
 
-template <typename T, typename G, int ACT>
+template <typename T, typename G>
 __global__ void __launch_bounds__(G::THREADS, G::MIN_CTAS) conv3x3_tc_kernel(const TcArgs p) {
     extern __shared__ __align__(128) unsigned char smem[];
     unsigned char* act = smem + G::OFF_ACT;
@@ -270,7 +255,7 @@ __global__ void __launch_bounds__(G::THREADS, G::MIN_CTAS) conv3x3_tc_kernel(con
                 if (p.cf1) { a = __ldg(p.cf1 + (size_t)(n * G::CU + cc) * 2); b = __ldg(p.cf1 + (size_t)(n * G::CU + cc) * 2 + 1); }
                 else gn_coef(p.st1, p.g1, p.b1, n, G::CU, p.groups1, cc, (double)H * W, p.eps, a, b);
             }
-            if constexpr (ACT != ACT_EXACT) { a *= 0.5f; b *= 0.5f; }  // silu(y) = h + h*tanh(h), h = y/2
+            a *= 0.5f; b *= 0.5f;  // silu(y) = h + h*tanh(h), h = y/2
             coef[c] = make_float2(a, b);
         }
         float* ctb = reinterpret_cast<float*>(smem + G::OFF_CTB);
@@ -297,7 +282,7 @@ __global__ void __launch_bounds__(G::THREADS, G::MIN_CTAS) conv3x3_tc_kernel(con
             float a, b;
             if (p.cf1) { a = __ldg(p.cf1 + (size_t)(n * G::COUT + c) * 2); b = __ldg(p.cf1 + (size_t)(n * G::COUT + c) * 2 + 1); }
             else gn_coef(p.st1, p.g1, p.b1, n, G::COUT, p.groups1, c, (double)H * W, p.eps, a, b);
-            if constexpr (ACT != ACT_EXACT) { a *= 0.5f; b *= 0.5f; }
+            a *= 0.5f; b *= 0.5f;
             coef[c] = make_float2(a, b);
         }
     } else {
@@ -306,7 +291,7 @@ __global__ void __launch_bounds__(G::THREADS, G::MIN_CTAS) conv3x3_tc_kernel(con
             float a, b;
             if (p.cf0) { a = __ldg(p.cf0 + (size_t)(n * G::CIN + c) * 2); b = __ldg(p.cf0 + (size_t)(n * G::CIN + c) * 2 + 1); }
             else gn_coef(p.st0, p.g0, p.b0, n, G::CIN, p.groups0, c, plane, p.eps, a, b);
-            if constexpr (ACT != ACT_EXACT) { a *= 0.5f; b *= 0.5f; }
+            a *= 0.5f; b *= 0.5f;
             coef[c] = make_float2(a, b);
         }
     }
@@ -314,19 +299,19 @@ __global__ void __launch_bounds__(G::THREADS, G::MIN_CTAS) conv3x3_tc_kernel(con
 
     // ---- (2) stage the activated halo tile ------------------------------------------------------------
     if constexpr (G::MODE == M_SAME) {
-        stage_planes<T, G, G::CIN, false, ACT, false, true>(act, reinterpret_cast<const unsigned char*>(p.src0) + (size_t)n * H * W * G::CIN * 2,
+        stage_planes<T, G, G::CIN, false, false, true>(act, reinterpret_cast<const unsigned char*>(p.src0) + (size_t)n * H * W * G::CIN * 2,
                                                              coef, 0, y0, x0, H, W);
     } else if constexpr (G::MODE == M_CAT2) {
-        stage_planes<T, G, G::COUT, false, ACT, true>(act, reinterpret_cast<const unsigned char*>(p.src0) + (size_t)n * H * W * G::COUT * 2,
+        stage_planes<T, G, G::COUT, false, true>(act, reinterpret_cast<const unsigned char*>(p.src0) + (size_t)n * H * W * G::COUT * 2,
                                                       coef, 0, y0, x0, H, W);
-        stage_planes<T, G, G::COUT, false, ACT, false, true>(act, reinterpret_cast<const unsigned char*>(p.src1) + (size_t)n * H * W * G::COUT * 2,
+        stage_planes<T, G, G::COUT, false, false, true>(act, reinterpret_cast<const unsigned char*>(p.src1) + (size_t)n * H * W * G::COUT * 2,
                                                               coef, G::COUT / 8, y0, x0, H, W);
     } else if constexpr (G::MODE == M_POOL) {
-        stage_planes<T, G, G::CIN, true, ACT, false, true>(act, reinterpret_cast<const unsigned char*>(p.src0) + (size_t)n * H * W * G::CIN * 8,
+        stage_planes<T, G, G::CIN, true, false, true>(act, reinterpret_cast<const unsigned char*>(p.src0) + (size_t)n * H * W * G::CIN * 8,
                                                             coef, 0, y0, x0, H, W);
     } else {
         // skip -> planes [CU/8, 2CU/8)
-        stage_planes<T, G, G::CU, false, ACT, false, true>(act, reinterpret_cast<const unsigned char*>(p.src1) + (size_t)n * H * W * G::CU * 2,
+        stage_planes<T, G, G::CU, false, false, true>(act, reinterpret_cast<const unsigned char*>(p.src1) + (size_t)n * H * W * G::CU * 2,
                                                             coef + G::CL, G::CU / 8, y0, x0, H, W);
         // activated low-res tile -> low planes
         unsigned char* low = smem + G::OFF_LOW;
@@ -362,7 +347,7 @@ __global__ void __launch_bounds__(G::THREADS, G::MIN_CTAS) conv3x3_tc_kernel(con
                     uint4 o = make_uint4(0u, 0u, 0u, 0u);
                     if (ok[b]) {
                         float y[8];
-                        act8<T, (ACT == ACT_HALF2 ? ACT_TANH : ACT)>(q[b], cf, y);
+                        act8<T>(q[b], cf, y);
                         o = pack8<T>(y);
                     }
                     *reinterpret_cast<uint4*>(low + ((size_t)c8 * G::LPLANE + lp) * 16) = o;
@@ -659,10 +644,6 @@ __global__ void __launch_bounds__(G::THREADS, G::MIN_CTAS) conv3x3_tc_kernel(con
             for (int w = 0; w < G::WM; ++w) t += (double)statf[w * G::COUT * 2 + c];
             atomicAdd(p.out_stats + (size_t)n * G::COUT * 2 + c, t);
         }
-    if (p.out_coef != nullptr && p.out_stats != nullptr) {
-        if (last_cta_of_image(p.out_counter + n, gridDim.x * gridDim.y))
-            gn_finalize(p.out_stats, p.out_gamma, p.out_beta, n, G::COUT, p.out_groups, (double)H * W, p.eps, p.out_coef);
-    }
 }
 
 // ---- weight packing kernels ------------------------------------------------------------------------------
@@ -743,9 +724,9 @@ int pack_convt_tc(const float* w, void* out, int cl, int cu, int dtype, cudaStre
 }
 
 // ---- dispatch -----------------------------------------------------------------------------------------------
-template <typename T, typename G, int ACT>
+template <typename T, typename G>
 static int launch_geo(const TcArgs& t, cudaStream_t st) {
-    auto kern = conv3x3_tc_kernel<T, G, ACT>;
+    auto kern = conv3x3_tc_kernel<T, G>;
     static bool attr_done = false;  // per instantiation
     if (!attr_done) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM_BYTES);
@@ -759,12 +740,12 @@ static int launch_geo(const TcArgs& t, cudaStream_t st) {
     return check_launch("conv3x3_tc");
 }
 
-template <typename T, int ACT>
+template <typename T>
 static int dispatch(const dg_conv3x3_args& a, const TcArgs& t, int mode, int cin, cudaStream_t st, bool* handled) {
     *handled = true;
     const int cout = a.cout;
 #define DG_TC(CI, CO, MD, TH, TW, WM, WN, ST) \
-    if (cin == CI && cout == CO && mode == MD) return launch_geo<T, Geo<CI, CO, MD, TH, TW, WM, WN, ST>, ACT>(t, st);
+    if (cin == CI && cout == CO && mode == MD) return launch_geo<T, Geo<CI, CO, MD, TH, TW, WM, WN, ST>>(t, st);
     DG_TC(8, 8, M_SAME, 16, 32, 4, 1, false)      // enc1.3, dec1.3 (128-thread CTAs: 8 independent phase streams per SM)
     DG_TC(8, 16, M_POOL, 16, 64, 8, 1, false)     // enc2.0 (ROLL measured slower: .135 vs .112 ms, pooled staging wants the wide tile)
     DG_TC(16, 16, M_SAME, 16, 64, 8, 1, false)    // enc2.3, dec2.3 (ROLL at 16x32 measured slower: .117 vs .099 ms)
@@ -825,22 +806,11 @@ int conv3x3_tc_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* handl
     t.src0 = s0.raw; t.st0 = s0.stats; t.g0 = s0.gamma; t.b0 = s0.beta; t.groups0 = s0.groups;
     t.cf0 = s0.coef;
     if (a.nsrc == 2) t.cf1 = a.src[1].coef;
-    if (a.out_coef && a.out_counter && a.out_gamma && a.out_beta && a.out_groups > 0) {
-        t.out_coef = a.out_coef; t.out_counter = a.out_counter; t.out_gamma = a.out_gamma; t.out_beta = a.out_beta;
-        t.out_groups = a.out_groups;
-    }
     t.wgt = a.weight_tc;
     t.out = a.out; t.out_stats = a.out_stats;
     t.N = a.N; t.H = a.H; t.W = a.W; t.eps = a.eps;
-    // path bits 2-3 pick the prologue flavour: 0 = tanh.approx.f32 (default), 4 = exact ex2/rcp, 8 = packed half2 (fp16 only)
-    const int flavour = (a.path >> 2) & 3;
-    if (a.dtype == DG_F16) {
-        if (flavour == 1) return dispatch<__half, ACT_EXACT>(a, t, mode, cin, stream, handled);
-        if (flavour == 2) return dispatch<__half, ACT_HALF2>(a, t, mode, cin, stream, handled);
-        return dispatch<__half, ACT_TANH>(a, t, mode, cin, stream, handled);
-    }
-    if (flavour == 1) return dispatch<__nv_bfloat16, ACT_EXACT>(a, t, mode, cin, stream, handled);
-    return dispatch<__nv_bfloat16, ACT_TANH>(a, t, mode, cin, stream, handled);
+    if (a.dtype == DG_F16) return dispatch<__half>(a, t, mode, cin, stream, handled);
+    return dispatch<__nv_bfloat16>(a, t, mode, cin, stream, handled);
 }
 
 }  // namespace dg

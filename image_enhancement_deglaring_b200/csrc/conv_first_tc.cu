@@ -22,7 +22,6 @@ constexpr int F_THREADS = 256;
 struct FirstArgs {
     const float* x; const float* w; void* out; double* out_stats;
     int N, H, W;
-    float* out_coef; int* out_counter; const float* out_gamma; const float* out_beta; int out_groups; float eps;
     int x_u8;  // x points at uint8 pixels, normalised as float32(u) / 255.0f (api/app.py:153) -- IEEE divide, bit-exact
 };
 
@@ -182,10 +181,6 @@ __global__ void __launch_bounds__(F_THREADS) conv_first_tc_kernel(const FirstArg
         for (int w8 = 0; w8 < 8; ++w8) t += (double)statw[w8][tid];
         atomicAdd(p.out_stats + (size_t)n * COUT * 2 + tid, t);
     }
-    if (p.out_coef != nullptr && p.out_stats != nullptr) {
-        if (last_cta_of_image(p.out_counter + n, gridDim.x * gridDim.y))
-            gn_finalize(p.out_stats, p.out_gamma, p.out_beta, n, COUT, p.out_groups, (double)H * W, p.eps, p.out_coef);
-    }
 }
 }  // namespace
 
@@ -197,12 +192,7 @@ int conv_first_tc_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* ha
     if (a.cout != 8 && a.cout != 16) return 0;
     if (a.act_sum != nullptr || a.N > 65535) return 0;
     if (reinterpret_cast<uintptr_t>(a.out) & 3) return 0;
-    FirstArgs f{reinterpret_cast<const float*>(s.raw), a.weight, a.out, a.out_stats, a.N, a.H, a.W,
-                nullptr, nullptr, nullptr, nullptr, 0, a.eps, s.xform == DG_X_IMAGE_U8 ? 1 : 0};
-    if (a.out_coef && a.out_counter && a.out_gamma && a.out_beta && a.out_groups > 0) {
-        f.out_coef = a.out_coef; f.out_counter = a.out_counter; f.out_gamma = a.out_gamma; f.out_beta = a.out_beta;
-        f.out_groups = a.out_groups;
-    }
+    FirstArgs f{reinterpret_cast<const float*>(s.raw), a.weight, a.out, a.out_stats, a.N, a.H, a.W, s.xform == DG_X_IMAGE_U8 ? 1 : 0};
     dim3 grid((a.W + F_TW - 1) / F_TW, (a.H + F_TH - 1) / F_TH, a.N);
     cudaError_t le = cudaSuccess;
     if (a.dtype == DG_F16) {

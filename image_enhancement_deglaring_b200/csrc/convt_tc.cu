@@ -29,7 +29,7 @@ struct ConvtArgs {
     int N, h, w; float eps;  // h, w: LOW resolution
 };
 
-template <typename T, int CL, int CU, int ACT>
+template <typename T, int CL, int CU>
 __global__ void __launch_bounds__(CT_THREADS) convt_tc_kernel(const ConvtArgs p) {
     constexpr int NCL8 = CL / 8, LPLANE = ct_pad_plane(CT_MP, NCL8);
     constexpr int CHUNKS = CL / 16, CT_N = 4 * CU, CT_NT = CT_N / 8, NTG = CT_NT < 8 ? CT_NT : 8;
@@ -58,7 +58,7 @@ __global__ void __launch_bounds__(CT_THREADS) convt_tc_kernel(const ConvtArgs p)
         float a, b;
         if (p.coef) { a = __ldg(p.coef + (size_t)(n * CL + c) * 2); b = __ldg(p.coef + (size_t)(n * CL + c) * 2 + 1); }
         else gn_coef(p.stats, p.gamma, p.beta, n, CL, p.groups, c, (double)hw, p.eps, a, b);
-        if constexpr (ACT != ACT_EXACT) { a *= 0.5f; b *= 0.5f; }
+        a *= 0.5f; b *= 0.5f;
         coef[c] = make_float2(a, b);
     }
     for (int c = tid; c < CU; c += CT_THREADS) bias[c] = p.ctb[c];
@@ -78,7 +78,7 @@ __global__ void __launch_bounds__(CT_THREADS) convt_tc_kernel(const ConvtArgs p)
             if (p_base + lp < hw) {
                 float y[8];
                 const uint4 q = __ldg(reinterpret_cast<const uint4*>(raw + (size_t)(p_base + lp) * CL + c8 * 8));
-                act8<T, (ACT == ACT_HALF2 ? ACT_TANH : ACT)>(q, cf, y);
+                act8<T>(q, cf, y);
                 o = pack8<T>(y);
             }
             *reinterpret_cast<uint4*>(low + ((size_t)c8 * LPLANE + lp) * 16) = o;
@@ -136,11 +136,11 @@ __global__ void __launch_bounds__(CT_THREADS) convt_tc_kernel(const ConvtArgs p)
     }
 }
 
-template <typename T, int CL, int CU, int ACT>
+template <typename T, int CL, int CU>
 int launch_convt(const ConvtArgs& a, cudaStream_t st) {
     constexpr int NCL8 = CL / 8, LPLANE = ct_pad_plane(CT_MP, NCL8);
     constexpr int SMEM = NCL8 * LPLANE * 16 + (CL / 16) * 2 * 4 * CU * 16 + CL * 8 + CU * 4;
-    auto kern = convt_tc_kernel<T, CL, CU, ACT>;
+    auto kern = convt_tc_kernel<T, CL, CU>;
     static bool done = false;
     if (!done) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM);
@@ -154,13 +154,13 @@ int launch_convt(const ConvtArgs& a, cudaStream_t st) {
     return check_launch("convt_tc");
 }
 
-template <typename T, int ACT>
+template <typename T>
 int dispatch_convt(const ConvtArgs& a, int cl, int cu, cudaStream_t st, bool* handled) {
     *handled = true;
-    if (cl == 128 && cu == 64) return launch_convt<T, 128, 64, ACT>(a, st);   // upconv4
-    if (cl == 64 && cu == 32) return launch_convt<T, 64, 32, ACT>(a, st);     // upconv3
-    if (cl == 32 && cu == 16) return launch_convt<T, 32, 16, ACT>(a, st);     // upconv2
-    if (cl == 16 && cu == 8) return launch_convt<T, 16, 8, ACT>(a, st);       // upconv1 (training: wgrad of dec1.0 reads `up`)
+    if (cl == 128 && cu == 64) return launch_convt<T, 128, 64>(a, st);   // upconv4
+    if (cl == 64 && cu == 32) return launch_convt<T, 64, 32>(a, st);     // upconv3
+    if (cl == 32 && cu == 16) return launch_convt<T, 32, 16>(a, st);     // upconv2
+    if (cl == 16 && cu == 8) return launch_convt<T, 16, 8>(a, st);       // upconv1 (training: wgrad of dec1.0 reads `up`)
     *handled = false;
     return 0;
 }
@@ -184,12 +184,8 @@ int convt_tc_launch(const dg_src& s, int dtype, int N, int H, int W, void* out, 
     if ((reinterpret_cast<uintptr_t>(s.raw) | reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(s.ct_w_tc)) & 15) return 0;
     if (N > 65535) return 0;
     ConvtArgs a{s.raw, s.stats, s.gamma, s.beta, s.coef, s.groups, s.ct_w_tc, s.ct_b, out, N, H / 2, W / 2, eps};
-    const int flavour = (path >> 2) & 3;
-    if (dtype == DG_F16)
-        return flavour == 1 ? dispatch_convt<__half, ACT_EXACT>(a, s.channels, s.ct_cout, st, handled)
-                            : dispatch_convt<__half, ACT_TANH>(a, s.channels, s.ct_cout, st, handled);
-    return flavour == 1 ? dispatch_convt<__nv_bfloat16, ACT_EXACT>(a, s.channels, s.ct_cout, st, handled)
-                        : dispatch_convt<__nv_bfloat16, ACT_TANH>(a, s.channels, s.ct_cout, st, handled);
+    if (dtype == DG_F16) return dispatch_convt<__half>(a, s.channels, s.ct_cout, st, handled);
+    return dispatch_convt<__nv_bfloat16>(a, s.channels, s.ct_cout, st, handled);
 }
 
 }  // namespace dg

@@ -63,56 +63,31 @@ template <> __device__ __forceinline__ float2 unpack2<__nv_bfloat16>(uint32_t v)
     return __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&v));
 }
 
-// ---- SiLU of the GroupNorm affine, two flavours --------------------------------------------------------
-//  TANH:  silu(y) = h + h*tanh(h), h = y/2 with the 1/2 folded into the affine coefficients: FFMA + MUFU.TANH
-//         + FFMA (tanh.approx.f32: max rel. error 2^-11, the same size as the fp16 rounding of the result);
-//  exact: y * rcp(1 + ex2(-y*log2e)): FFMA, FMUL, MUFU.EX2, FADD, MUFU.RCP, FMUL (rel. error ~2^-22).
+// ---- SiLU of the GroupNorm affine --------------------------------------------------------------------
+//  silu(y) = h + h*tanh(h), h = y/2 with the 1/2 folded into the affine coefficients: FFMA + MUFU.TANH + FFMA
+//  (tanh.approx.f32: max rel. error 2^-11, the same size as the fp16 rounding of the result).
 //  (__expf/__fdividef cost ~12 instructions per element because of their range handling -- profile r1.)
 __device__ __forceinline__ float tanh_approx(float x) {
     float y;
     asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
 }
-// activation flavours of the tensor-core prologue
-enum { ACT_EXACT = 0, ACT_TANH = 1, ACT_HALF2 = 2 };
 
-template <int ACT>
 __device__ __forceinline__ float silu_affine(float x, float a, float b) {
     const float y = fmaf(x, a, b);
-    if constexpr (ACT != ACT_EXACT) {
-        return fmaf(y, tanh_approx(y), y);  // (a, b) pre-halved by the caller
-    } else {
-        float e, r;
-        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(y * -1.4426950408889634f));
-        asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(1.f + e));
-        return y * r;
-    }
+    return fmaf(y, tanh_approx(y), y);  // (a, b) pre-halved by the caller
 }
 
-// GroupNorm apply + SiLU on 8 packed 16-bit channels; cf = (a, b) pairs of those channels (registers)
-template <typename T, int ACT>
+// GroupNorm apply + SiLU on 8 packed 16-bit channels; cf = (a, b) pairs of those channels (registers), pre-halved
+template <typename T>
 __device__ __forceinline__ void act8(const uint4& raw, const float2 (&cf)[8], float (&y)[8]) {
     const uint32_t w[4] = {raw.x, raw.y, raw.z, raw.w};
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
         const float2 v = unpack2<T>(w[k]);
-        y[2 * k] = silu_affine<ACT>(v.x, cf[2 * k].x, cf[2 * k].y);
-        y[2 * k + 1] = silu_affine<ACT>(v.y, cf[2 * k + 1].x, cf[2 * k + 1].y);
+        y[2 * k] = silu_affine(v.x, cf[2 * k].x, cf[2 * k].y);
+        y[2 * k + 1] = silu_affine(v.y, cf[2 * k + 1].x, cf[2 * k + 1].y);
     }
-}
-
-// ACT_HALF2 (fp16 storage only): the whole prologue in packed half precision -- h = a'x + b' (HFMA2), t = tanh(h)
-// (MUFU.TANH.F16x2), y = h*t + h (HFMA2): 3 instructions per PAIR of channels and no unpack / pack at all.
-__device__ __forceinline__ uint32_t silu_affine_h2(uint32_t x, uint32_t a, uint32_t b) {
-    uint32_t h, t, y;
-    asm("fma.rn.f16x2 %0, %1, %2, %3;" : "=r"(h) : "r"(x), "r"(a), "r"(b));
-    asm("tanh.approx.f16x2 %0, %1;" : "=r"(t) : "r"(h));
-    asm("fma.rn.f16x2 %0, %1, %2, %1;" : "=r"(y) : "r"(h), "r"(t));
-    return y;
-}
-__device__ __forceinline__ uint4 act8_h2(const uint4& raw, const uint32_t (&a)[4], const uint32_t (&b)[4]) {
-    return make_uint4(silu_affine_h2(raw.x, a[0], b[0]), silu_affine_h2(raw.y, a[1], b[1]),
-                      silu_affine_h2(raw.z, a[2], b[2]), silu_affine_h2(raw.w, a[3], b[3]));
 }
 
 template <typename T>

@@ -184,14 +184,14 @@ wgrad_tc_kernel(const WgArgs p) {
                         const size_t rowb = (size_t)(2 * W) * CS * 2;
                         const unsigned char* q0 = base + (size_t)(2 * gy) * rowb + (size_t)(2 * gx) * CS * 2;
                         float y[8], t[8];
-                        act8<T, ACT_TANH>(__ldg(reinterpret_cast<const uint4*>(q0)), cf, y);
-                        act8<T, ACT_TANH>(__ldg(reinterpret_cast<const uint4*>(q0 + CS * 2)), cf, t);
+                        act8<T>(__ldg(reinterpret_cast<const uint4*>(q0)), cf, y);
+                        act8<T>(__ldg(reinterpret_cast<const uint4*>(q0 + CS * 2)), cf, t);
 #pragma unroll
                         for (int k = 0; k < 8; ++k) y[k] += t[k];
-                        act8<T, ACT_TANH>(__ldg(reinterpret_cast<const uint4*>(q0 + rowb)), cf, t);
+                        act8<T>(__ldg(reinterpret_cast<const uint4*>(q0 + rowb)), cf, t);
 #pragma unroll
                         for (int k = 0; k < 8; ++k) y[k] += t[k];
-                        act8<T, ACT_TANH>(__ldg(reinterpret_cast<const uint4*>(q0 + rowb + CS * 2)), cf, t);
+                        act8<T>(__ldg(reinterpret_cast<const uint4*>(q0 + rowb + CS * 2)), cf, t);
 #pragma unroll
                         for (int k = 0; k < 8; ++k) y[k] = 0.25f * (y[k] + t[k]);
                         o = pack8<BF>(y);
@@ -201,7 +201,7 @@ wgrad_tc_kernel(const WgArgs p) {
                             o = to_bf16x8<T>(q);
                         } else {
                             float y[8];
-                            act8<T, ACT_TANH>(q, cf, y);
+                            act8<T>(q, cf, y);
                             o = pack8<BF>(y);
                         }
                     }
@@ -437,7 +437,7 @@ __global__ void __launch_bounds__(WG_THREADS) convt_wgrad_tc_kernel(const CtWgAr
                 uint4 o = make_uint4(0u, 0u, 0u, 0u);
                 if (gy < Hl && gx < Wl) {
                     float y[8];
-                    act8<T, ACT_TANH>(__ldg(reinterpret_cast<const uint4*>(base + ((size_t)gy * Wl + gx) * CL * 2)), cf, y);
+                    act8<T>(__ldg(reinterpret_cast<const uint4*>(base + ((size_t)gy * Wl + gx) * CL * 2)), cf, y);
                     o = pack8<BF>(y);
                 }
                 *reinterpret_cast<uint4*>(dst + (size_t)pix * 16) = o;

@@ -63,8 +63,8 @@ typedef struct {
     const float* ct_w;    /* DG_X_CONVT2: weights packed [2][2][channels][ct_cout] fp32    */
     const float* ct_b;    /* DG_X_CONVT2: bias [ct_cout]                                   */
     const void* ct_w_tc;  /* DG_X_CONVT2: optional tensor-core packing (dg_pack_convt2x2_tc) */
-    const float* coef;    /* optional [N,channels,2] finished GroupNorm affine (a, b) written by the producer's
-                             last CTA (dg_conv3x3_args.out_coef); consumers prefer it over `stats`   */
+    const float* coef;    /* optional [N,channels,2] finished GroupNorm affine (a, b), e.g. from dg_gn_affine;
+                             consumers prefer it over `stats`                                */
     int32_t channels;
     int32_t groups;       /* GroupNorm groups over `channels`                              */
     int32_t xform;        /* DG_X_*                                                        */
@@ -91,22 +91,13 @@ typedef struct {
     double* out_stats;    /* [N,cout,2], must be zero on entry; accumulated atomically     */
     double* act_sum;      /* optional [N,src[0].channels]: sum over pixels of the ACTIVATED
                              src[0] (for ChannelAttention's global average); zero on entry  */
-    /* optional: the LAST CTA to finish an image turns its statistics into the GroupNorm affine of the norm that
-       follows this conv, so consumers load two floats per channel instead of redoing double-precision math per CTA */
-    float* out_coef;          /* [N,cout,2] (a = rstd*gamma, b = beta - mean*a)                  */
-    int32_t* out_counter;     /* [N] arrival counters, zero on entry                              */
-    const float* out_gamma;   /* [cout] weight / bias / groups of the GroupNorm applied to `out`  */
-    const float* out_beta;
-    int32_t out_groups;
-    int32_t reserved;
     float eps;            /* GroupNorm eps of the sources (1e-5)                           */
     int32_t path;         /* bits 0-1: 0 = auto, 1 = force generic CUDA-core path, 2 = force tensor-core path;
-                             bits 2-3: SiLU flavour of the tensor-core prologue (0 tanh.approx, 1 exact ex2/rcp, 2 half2);
-                             bit 4: producer-side GroupNorm finalisation; bit 5: un-fuse upconv2 as well;
-                             bit 6: round-1 tcgen05 kernel (opt-in); bit 7: do not use the round-2 tcgen05 kernel (conv3x3_t5.cu);
-                             bit 8: insist on it (tests); bit 9 / bit 10: do not use the persistent TMA-fed 8 -> 8 kernel
-                             (conv3x3_ring.cu) / the composite decoder kernels (conv3x3_dec.cu, conv3x3_t5.cu decoder mode);
-                             bit 11 (module level): also pack the composite blobs of the 32 -> 16 ... 128 -> 64 decoders           */
+                             bit 7: do not use the tcgen05 kernel (conv3x3_t5.cu); bit 8: insist on it (tests);
+                             bit 9 / bit 10: do not use the persistent TMA-fed 8 -> 8 kernel (conv3x3_ring.cu) / the composite
+                             decoder kernels (conv3x3_dec.cu, conv3x3_t5.cu decoder mode);
+                             bit 11 (module level): also pack the composite blobs of the 32 -> 16 ... 128 -> 64 decoders.
+                             Bits 2-6 are unused: a call that sets one fails with 2.                                        */
     const void* weight_comp;  /* optional, decoder conv over (DG_X_CONVT2 low, DG_X_SAME skip) only: dg_pack_dec_composite blob --
                                  the ConvTranspose folded into the conv's taps (conv3x3_dec.cu); NULL = stage `up` in the CTA  */
 } dg_conv3x3_args;
@@ -249,7 +240,7 @@ typedef struct {
                                                weights; the tensor-core dgrad reads it transposed (NULL = CUDA-core dgrad) */
     const float* head_w;                    /* output_conv.weight [out][f0]                */
     const float* head_b;
-    int32_t path;                           /* 0 auto, 1 generic, 2 tensor-core            */
+    int32_t path;                           /* dg_conv3x3_args.path: 0 auto, 1 generic, 2 tensor-core, ... */
     int32_t reserved;
     const void* dec_comp[4];                /* optional: dg_pack_dec_composite blobs of (upconv4..1, dec4..1 `.0`) for the
                                                levels the composite decoder kernel covers (upconv1 + dec1.0 of the shipped

@@ -299,8 +299,8 @@ def test_tc_first_layer(dtype, cout, H, W):
 
 
 @pytest.mark.parametrize("dtype", TC_DTYPES)
-def test_tc_exact_and_tanh_silu_agree(dtype):
-    """path bit 2 selects the ex2/rcp SiLU in the staging prologue instead of tanh.approx."""
+def test_tc_tanh_silu_matches_oracle(dtype):
+    """The tanh.approx SiLU of the staging prologue (h + h*tanh(h), h = y/2) against the fp32 oracle."""
     rs = _rs(15)
     N, cin, cout, H, W = 2, 16, 16, 32, 64
     raw = torch.from_numpy((rs.standard_normal((N, cin, H, W)) * 3 + 1).astype(np.float32))
@@ -311,12 +311,10 @@ def test_tc_exact_and_tanh_silu_agree(dtype):
     wtc = ops.pack_conv3x3_tc(wp, dtype)
     src = ops.make_src(q, cin, stats=_stats(seen), gamma=g.cuda(), beta=b.cuda(), groups=8)
     o_t, _ = ops.conv3x3_fused([src], wp, cout, N, H, W, dtype, path=2, weight_tc=wtc)
-    o_e, _ = ops.conv3x3_fused([src], wp, cout, N, H, W, dtype, path=6, weight_tc=wtc)
     torch.cuda.synchronize()
     ref = F.conv2d(tpo.gn_silu(seen, 8, g, b), w, None, 1, 1)
     tol = (4e-3 if dtype == ops.DG_F16 else 3e-2) * max(1.0, float(ref.abs().max()))
-    for o in (o_t, o_e):
-        assert float((o.float().cpu().permute(0, 3, 1, 2) - ref).abs().max()) <= tol
+    assert float((o_t.float().cpu().permute(0, 3, 1, 2) - ref).abs().max()) <= tol
 
 
 @pytest.mark.parametrize("dtype", TC_DTYPES)
@@ -384,19 +382,13 @@ def _deep_case(rs, dtype, mode, cin, cout, N, H, W, groups=8):
 @pytest.mark.parametrize("mode,cin,cout,H,W", [("same", 64, 64, 16, 64), ("same", 64, 64, 8, 32), ("same", 64, 64, 12, 40),
                                                  ("pool", 32, 64, 16, 32), ("pool", 32, 64, 6, 10), ("cat2", 64, 32, 16, 64),
                                                  ("cat2", 64, 32, 10, 36)])
-def test_umma_matches_hmma_and_generic(dtype, mode, cin, cout, H, W):
-    """round-1 tcgen05/TMEM kernel (path 2 | 64, with the round-2 kernel disabled by bit 7) vs the mma.sync kernel (path 2 | 128)
-    vs the generic kernel on identical inputs."""
+def test_hmma_matches_generic(dtype, mode, cin, cout, H, W):
+    """The mma.sync kernel (path 2 | 128: the tcgen05 kernel disabled) vs the generic kernel on identical inputs."""
     srcs, wp, wtc, _ = _deep_case(_rs(17), dtype, mode, cin, cout, 3, H, W)
     o_gen, s_gen = ops.conv3x3_fused(srcs, wp, cout, 3, H, W, dtype, path=1)
-    o_um, s_um = ops.conv3x3_fused(srcs, wp, cout, 3, H, W, dtype, path=2 | 64 | 128, weight_tc=wtc)
     o_hm, s_hm = ops.conv3x3_fused(srcs, wp, cout, 3, H, W, dtype, path=2 | 128, weight_tc=wtc)
     torch.cuda.synchronize()
-    _tc_check(o_um, s_um, o_gen, s_gen, dtype, f"umma {mode} {cin}->{cout}")
     _tc_check(o_hm, s_hm, o_gen, s_gen, dtype, f"hmma {mode} {cin}->{cout}")
-    # both tensor paths round the same fp16 operands: they agree far tighter than either does with the fp32-staged generic path
-    scale = max(1.0, float(o_gen.float().abs().max()))
-    assert float((o_um.float() - o_hm.float()).abs().max()) <= (2e-3 if dtype == ops.DG_F16 else 1.6e-2) * scale
 
 
 # every deep layer of LightweightUNet(features_start=8) at its real 512^2 geometry plus ragged / tiny shapes, then the channel

@@ -47,6 +47,43 @@ def test_struct_layouts_match_header_sizes(tmp_path):
     assert C.sizeof(_lib.DgSrc) == 9 * 8 + 6 * 4
 
 
+_REMOVED_PATH_BITS_PROBE = r"""
+import ctypes as C, json
+from image_enhancement_deglaring_b200 import _lib
+lib = _lib.load()
+buf = (C.c_float * 4096)()   # placeholder for every pointer: none may be dereferenced
+res = {}
+for path in (4, 8, 16, 32, 64, 0, 2 | 128):
+    p = _lib.DgLwParams()
+    p.in_channels, p.out_channels, p.features_start, p.dtype, p.path = 1, 1, 8, _lib.DG_F16, path
+    rc = lib.dg_lw_workspace_bytes(C.byref(p), 1, 16, 16, C.byref(C.c_size_t(0)))
+    res[path] = [rc, lib.dg_last_error_string().decode()]
+    if path & 0x7c:
+        a = _lib.DgConv3x3Args()
+        a.nsrc, a.dtype, a.N, a.H, a.W, a.cout, a.eps, a.path = 1, _lib.DG_F16, 1, 16, 16, 8, 1e-5, path
+        a.weight = a.out = a.out_stats = C.addressof(buf)
+        a.src[0].raw, a.src[0].channels, a.src[0].groups, a.src[0].xform = C.addressof(buf), 8, 1, _lib.DG_X_SAME
+        res[path] += [lib.dg_conv3x3_fused(C.byref(a), None), lib.dg_last_error_string().decode()]
+print(json.dumps(res))
+"""
+
+
+def test_removed_path_bits_are_rejected():
+    """Path bits 2-6 no longer select anything: dg_conv3x3_fused and the dg_lw_* planner return 2 and name the bit, before any
+    CUDA call -- run in a process that sees no CUDA device, where a call that reached the runtime would fail differently."""
+    import json
+    import subprocess
+    out = subprocess.run([sys.executable, "-c", _REMOVED_PATH_BITS_PROBE], cwd=ROOT, env={**os.environ, "CUDA_VISIBLE_DEVICES": ""},
+                         capture_output=True, text=True, timeout=300)
+    assert out.returncode == 0, out.stderr[-500:]
+    res = {int(k): v for k, v in json.loads(out.stdout.splitlines()[-1]).items()}
+    for bit in range(2, 7):
+        ws_rc, ws_err, conv_rc, conv_err = res[1 << bit]
+        assert conv_rc == 2 and f"path {1 << bit} sets bit {bit}," in conv_err, (bit, conv_rc, conv_err)
+        assert ws_rc == 2 and f"path {1 << bit} sets bit {bit}," in ws_err, (bit, ws_rc, ws_err)
+    assert res[0][0] == 0 and res[2 | 128][0] == 0, res   # the surviving bits still plan a workspace
+
+
 def test_module_surface_matches_reference_contract(best_sd, golden):
     import image_enhancement_deglaring_b200 as dg
     net = dg.LightweightUNet()

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Accuracy of storage tiers / kernel paths on the golden PNGs and a seeded random batch (GPU box).
-    python tools/accuracy_paths.py [--paths 0,8,128]
+    python tools/accuracy_paths.py [--paths 0,128]
 The reference values come from tests/golden (generated from the reference) -- no oracle import here."""
 import argparse
 import os
@@ -14,7 +14,7 @@ sys.path.insert(0, ROOT)
 import image_enhancement_deglaring_b200 as dg  # noqa: E402
 
 ap = argparse.ArgumentParser()
-ap.add_argument("--paths", default="0,8,128")
+ap.add_argument("--paths", default="0,128")
 ap.add_argument("--storage", default="fp16")
 a = ap.parse_args()
 g = np.load(os.path.join(ROOT, "tests", "golden", "lw_png.npz"))

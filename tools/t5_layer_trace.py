@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """One fused conv at a LightweightUNet layer geometry, batch 64, with the t5 kernel's role timeline (DG_T5_TRACE=1) --
-debug aid for the warp-specialised pipeline.   DG_T5_TRACE=1 [DG_T5_DBG=k] python tools/t5_layer_trace.py same 32 32 128 128"""
+debug aid for the warp-specialised pipeline.   DG_T5_TRACE=1 python tools/t5_layer_trace.py same 32 32 128 128"""
 import sys, os, time
 import numpy as np
 import torch
