@@ -59,6 +59,13 @@ class DgLwParams(C.Structure):
     ]
 
 
+class DgLwBwdRequest(C.Structure):
+    _fields_ = [
+        ("grad_y", C.c_void_p), ("y", C.c_void_p), ("target", C.c_void_p), ("loss_grad", C.c_void_p),
+        ("grads", C.c_void_p), ("param_mask", C.c_uint64), ("grad_x", C.c_void_p),
+    ]
+
+
 # every symbol include/deglare.h declares: name -> (restype, argtypes)
 SYMBOLS = {
     "dg_conv3x3_fused": (C.c_int, [C.POINTER(DgConv3x3Args), C.c_void_p]),
@@ -111,6 +118,10 @@ SYMBOLS = {
     "dg_l1_loss_sum": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
     "dg_lw_backward_l1": (C.c_int, [C.POINTER(DgLwParams), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
                                     C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
+    "dg_lw_backward_select": (C.c_int, [C.POINTER(DgLwParams), C.c_void_p, C.POINTER(DgLwBwdRequest), C.c_int32, C.c_int32,
+                                        C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dg_conv_first_dgrad": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                      C.c_void_p]),
     "dg_adamw_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_float,
                                 C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_int32, C.c_float, C.c_void_p]),
     "dg_adamw_step_graph": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p, C.c_float,

@@ -302,34 +302,50 @@ static int lw_forward(const dg_lw_params* p, const void* x, void* y, int N, int 
 // Flat gradient layout = the module's parameters() order and the parameters' own memory layouts:
 //   per block: conv0.weight [Co][Ci][3][3], gn0.weight, gn0.bias, conv1.weight, gn1.weight, gn1.bias
 //   order: enc1..enc4, bottleneck, (upconvK.weight [Ci][Co][2][2], upconvK.bias, decK block) for K=4..1, head w, head b
+// The named fields hold a tensor's index k in that order (bit k of dg_lw_bwd_request.param_mask); off[k] is its flat offset and
+// pos[k] its forward position x 2: conv i and the GroupNorm after it 2i, upconvK one below the decoder conv consuming it, head 36.
+constexpr int kLwTensors = 64;
 struct GradLayout {
-    size_t conv_w[9][2], gn_w[9][2], gn_b[9][2], up_w[4], up_b[4], head_w, head_b, total;
+    int conv_w[9][2], gn_w[9][2], gn_b[9][2], up_w[4], up_b[4], head_w, head_b;
+    size_t off[kLwTensors + 1];   // off[kLwTensors] = the total element count
+    int pos[kLwTensors];
 };
 
 static void make_grad_layout(const dg_lw_params* p, const LwPlan& pl, GradLayout* g) {
     size_t off = 0;
+    int k = 0;
+    auto add = [&](size_t count, int pos) { g->off[k] = off; g->pos[k] = pos; off += count; return k++; };
     auto block = [&](int b) {
         const int lvl = block_level(b);
         const int c = pl.f[lvl];
         const int cin0 = b == 0 ? p->in_channels : (b < 5 ? pl.f[lvl - 1] : 2 * c);
-        g->conv_w[b][0] = off; off += (size_t)c * cin0 * 9;
-        g->gn_w[b][0] = off; off += c;
-        g->gn_b[b][0] = off; off += c;
-        g->conv_w[b][1] = off; off += (size_t)c * c * 9;
-        g->gn_w[b][1] = off; off += c;
-        g->gn_b[b][1] = off; off += c;
+        g->conv_w[b][0] = add((size_t)c * cin0 * 9, 4 * b);
+        g->gn_w[b][0] = add(c, 4 * b);
+        g->gn_b[b][0] = add(c, 4 * b);
+        g->conv_w[b][1] = add((size_t)c * c * 9, 4 * b + 2);
+        g->gn_w[b][1] = add(c, 4 * b + 2);
+        g->gn_b[b][1] = add(c, 4 * b + 2);
     };
     for (int b = 0; b < 5; ++b) block(b);
     for (int b = 5; b < 9; ++b) {
         const int lvl = block_level(b), u = b - 5;
-        g->up_w[u] = off; off += (size_t)pl.f[lvl + 1] * pl.f[lvl] * 4;
-        g->up_b[u] = off; off += pl.f[lvl];
+        g->up_w[u] = add((size_t)pl.f[lvl + 1] * pl.f[lvl] * 4, 4 * b - 1);
+        g->up_b[u] = add(pl.f[lvl], 4 * b - 1);
         block(b);
     }
-    g->head_w = off; off += (size_t)p->out_channels * pl.f[0];
-    g->head_b = off; off += p->out_channels;
-    g->total = off;
+    g->head_w = add((size_t)p->out_channels * pl.f[0], 36);
+    g->head_b = add(p->out_channels, 36);
+    g->off[k] = off;
 }
+
+// What one backward computes: the parameter tensors of `mask` into `grads`, and dL/dx into grad_x when set.  `low` = the lowest
+// requested forward position x 2 (-2 = the input image): conv i's data gradient runs only when low < 2i.
+struct BwdRequest {
+    float* grads;
+    uint64_t mask;
+    float* grad_x;
+    int low;
+};
 
 struct BwdPlan {
     size_t p_off[18], g_off[18], t_off[18], gb_off[18], low_off[4], coef_off, p_bytes, total;   // gb: dR as bf16 (16-bit tiers)
@@ -406,11 +422,13 @@ static void fwd_conv_args(const dg_lw_params* p, const LwPlan& pl, char* ws, con
 struct L1Seed { const float* y; const float* target; const float* scale; float inv_numel; };
 
 static int lw_backward_range(const dg_lw_params* p, const struct LwPlan& pl, const struct BwdPlan& bp, const struct GradLayout& gl,
-                             const float* x, const float* grad_y, int n0, int N, int H, int W, char* fw, char* bw, float* grads,
-                             cudaStream_t st, const L1Seed* l1);
+                             const float* x, const float* grad_y, int n0, int N, int H, int W, char* fw, char* bw,
+                             const BwdRequest& rq, cudaStream_t st, const L1Seed* l1);
 
+// grads / mask / grad_x as in dg_lw_bwd_request; dg_lw_backward and dg_lw_backward_l1 are mask = every tensor, grad_x = NULL
 static int lw_backward(const dg_lw_params* p, const float* x, const float* grad_y, int N, int H, int W, void* fwd_ws,
-                       size_t fwd_bytes, void* bwd_ws, size_t bwd_bytes, float* grads, cudaStream_t st, const L1Seed* l1 = nullptr) {
+                       size_t fwd_bytes, void* bwd_ws, size_t bwd_bytes, float* grads, uint64_t mask, float* grad_x, cudaStream_t st,
+                       const L1Seed* l1 = nullptr) {
     LwPlan pl;
     int rc = make_plan(p, N, H, W, &pl);
     if (rc) return rc;
@@ -422,7 +440,10 @@ static int lw_backward(const dg_lw_params* p, const float* x, const float* grad_
         set_error("backward: workspace too small (fwd %zu/%zu, bwd %zu/%zu)", fwd_bytes, pl.total_bytes, bwd_bytes, bp.total);
         return 4;
     }
-    if (x == nullptr || (grad_y == nullptr && l1 == nullptr) || grads == nullptr) { set_error("backward: null pointer"); return 2; }
+    if (x == nullptr || (grad_y == nullptr && l1 == nullptr) || (mask != 0 && grads == nullptr)) { set_error("backward: null pointer"); return 2; }
+    BwdRequest rq{grads, mask, grad_x, grad_x != nullptr ? -2 : 1 << 30};
+    for (int k = 0; k < kLwTensors; ++k)
+        if (((mask >> k) & 1) && gl.pos[k] < rq.low) rq.low = gl.pos[k];
     // conv_w_flip / up_w_t feed the CUDA-core data-gradient kernels only: required where a tensor-core packing is absent
     for (int b = 0; b < 9; ++b)
         for (int j = 0; j < 2; ++j)
@@ -435,7 +456,13 @@ static int lw_backward(const dg_lw_params* p, const float* x, const float* grad_
     char* fw = static_cast<char*>(fwd_ws);
     char* bw = static_cast<char*>(bwd_ws);
     cudaError_t e = cudaMemsetAsync(bw, 0, bp.p_bytes, st);
-    if (e == cudaSuccess) e = cudaMemsetAsync(grads, 0, gl.total * sizeof(float), st);
+    for (int k = 0; k < kLwTensors && e == cudaSuccess;) {   // one memset per run of requested tensors; the others stay untouched
+        if (!((mask >> k) & 1)) { ++k; continue; }
+        int k1 = k;
+        while (k1 < kLwTensors && ((mask >> k1) & 1)) ++k1;
+        e = cudaMemsetAsync(grads + gl.off[k], 0, (gl.off[k1] - gl.off[k]) * sizeof(float), st);
+        k = k1;
+    }
     if (e != cudaSuccess) { set_error("memset: %s", cudaGetErrorString(e)); return 10; }
     const int split = g_split.load();
     if (split > 0 && N >= split && N >= 2) {   // two concurrent sub-batches, as in lw_forward
@@ -445,22 +472,24 @@ static int lw_backward(const dg_lw_params* p, const float* x, const float* grad_
         const int half = N / 2;
         for (int k = 0; k < 2; ++k) {
             cudaStreamWaitEvent(F.s[k], F.fork, 0);
-            rc = lw_backward_range(p, pl, bp, gl, x, grad_y, k ? half : 0, k ? N - half : half, H, W, fw, bw, grads, F.s[k], l1);
+            rc = lw_backward_range(p, pl, bp, gl, x, grad_y, k ? half : 0, k ? N - half : half, H, W, fw, bw, rq, F.s[k], l1);
             cudaEventRecord(F.join[k], F.s[k]);
             cudaStreamWaitEvent(st, F.join[k], 0);
             if (rc) return rc;
         }
         return 0;
     }
-    return lw_backward_range(p, pl, bp, gl, x, grad_y, 0, N, H, W, fw, bw, grads, st, l1);
+    return lw_backward_range(p, pl, bp, gl, x, grad_y, 0, N, H, W, fw, bw, rq, st, l1);
 }
 
 // Backward over images [n0, n0 + N) of a batch of N_total; every buffer was laid out for the whole batch (`N` below is the
-// sub-batch size).  Parameter gradients are accumulated atomically, so concurrent sub-batches add up.
+// sub-batch size).  Parameter gradients are accumulated atomically, so concurrent sub-batches add up; the input gradient is per
+// image.  Tensors outside rq.mask get no kernel work, and the loop ends below the lowest requested position.
 static int lw_backward_range(const dg_lw_params* p, const LwPlan& pl, const BwdPlan& bp, const GradLayout& gl, const float* x,
-                             const float* grad_y, int n0, int N, int H, int W, char* fw, char* bw, float* grads, cudaStream_t st,
-                             const L1Seed* l1) {
+                             const float* grad_y, int n0, int N, int H, int W, char* fw, char* bw, const BwdRequest& rq,
+                             cudaStream_t st, const L1Seed* l1) {
     int rc = 0;
+    auto gp = [&](int k) { return ((rq.mask >> k) & 1) ? rq.grads + gl.off[k] : nullptr; };
     const size_t esz = dtype_size(p->dtype);
     bool t_split[18] = {};   // decoder conv i: T(i) holds the two halves of the concat gradient as two compact tensors
     auto hwc = [&](int i, int c) { return (size_t)pl.conv_h[i] * pl.conv_w[i] * c; };
@@ -477,11 +506,13 @@ static int lw_backward_range(const dg_lw_params* p, const LwPlan& pl, const BwdP
     const size_t o0 = (size_t)n0 * p->out_channels * H * W;
     rc = head_bwd_launch(p->dtype, raw(17), stats(17), p->gn_w[8][1], p->gn_b[8][1],
                          grad_y ? grad_y + o0 : nullptr, p->head_w, G(17), P(17),
-                         grads + gl.head_w, grads + gl.head_b, N, H, W, pl.conv_c[17], p->out_channels, p->groups[8], 1e-5f, st,
+                         gp(gl.head_w), gp(gl.head_b), N, H, W, pl.conv_c[17], p->out_channels, p->groups[8], 1e-5f, st,
                          l1 ? l1->y + o0 : nullptr, l1 ? l1->target + o0 : nullptr, l1 ? l1->scale : nullptr, l1 ? l1->inv_numel : 0.f);
     if (rc) return rc;
-    for (int i = 17; i >= 0; --i) {
+    for (int i = 17; i >= 0 && rq.low <= 2 * i; --i) {
         const int b = i / 2, j = i % 2, C = pl.conv_c[i], Hi = pl.conv_h[i], Wi = pl.conv_w[i];
+        float* const dW = gp(gl.conv_w[b][j]);   // NULL: frozen, no weight-gradient kernel
+        const bool dgrad = rq.low < 2 * i;       // something below conv i wants a gradient (i = 0: the input image)
         char rname[32];
         snprintf(rname, sizeof(rname), "bwd %s", kConvNames[i]);
         NvtxRange range(rname);
@@ -489,9 +520,10 @@ static int lw_backward_range(const dg_lw_params* p, const LwPlan& pl, const BwdP
         dg_conv3x3_args a;
         fwd_conv_args(p, pl, fw, x, N, i, &a, n0);
         // G_i -> dR_i, dgamma / dbeta.  Where BOTH consumers of dR_i are tensor-core kernels (they round it to bf16 anyway) it is
-        // written once as bf16 instead of fp32 in place: they read half the bytes and copy the tile instead of converting it.
+        // written once as bf16 instead of fp32 in place: they read half the bytes and copy the tile instead of converting it.  A
+        // skipped weight gradient leaves the data gradient to decide alone.
         void* dRb = nullptr;
-        if (i > 0 && p->dtype != DG_F32 && (p->path & 3) != 1 && p->conv_w_tc_bf16[b][j] != nullptr) {
+        if (i > 0 && (dW != nullptr || dgrad) && p->dtype != DG_F32 && (p->path & 3) != 1 && p->conv_w_tc_bf16[b][j] != nullptr) {
             dg_conv3x3_args probe = a;
             if (probe.nsrc == 2) {   // the wgrad kernel sees a decoder conv with its ConvTranspose source materialised
                 memset(&probe.src[0], 0, sizeof(dg_src));
@@ -500,18 +532,18 @@ static int lw_backward_range(const dg_lw_params* p, const LwPlan& pl, const BwdP
                 probe.src[0].groups = 1;
                 probe.src[0].xform = DG_X_SAME;
             }
-            bool wg_ok = false, dgr_ok = false;
-            conv3x3_wgrad_tc_launch(probe, G(i), grads + gl.conv_w[b][j], 1, 9, 9 * bp.cin_tot[i], st, &wg_ok, nullptr, /*dry*/ true);
+            bool wg_ok = dW == nullptr, dgr_ok = false;
+            if (dW != nullptr) conv3x3_wgrad_tc_launch(probe, G(i), dW, 1, 9, 9 * bp.cin_tot[i], st, &wg_ok, nullptr, /*dry*/ true);
             conv3x3_dgrad_tc_launch(G(i), p->conv_w_tc_bf16[b][j], G(i), N, Hi, Wi, C, bp.cin_tot[i], st, &dgr_ok, nullptr, nullptr, true);
             if (wg_ok && dgr_ok) dRb = bw + bp.gb_off[i] + (size_t)n0 * hwc(i, C) * 2;
         }
         bool dr_bf16 = false;
-        rc = gn_bwd_apply_launch(p->dtype, raw(i), stats(i), p->gn_w[b][j], P(i), G(i), grads + gl.gn_w[b][j], grads + gl.gn_b[b][j],
+        rc = gn_bwd_apply_launch(p->dtype, raw(i), stats(i), p->gn_w[b][j], P(i), G(i), gp(gl.gn_w[b][j]), gp(gl.gn_b[b][j]),
                                  N, Hi, Wi, C, p->groups[b], 1e-5f, st, dRb, &dr_bf16);
         if (rc) return rc;
         const void* dRb_in = dr_bf16 ? dRb : nullptr;   // when set, G(i) still holds G, NOT dR: only the bf16 copy is valid
-        bool wg_done = false;
-        if (p->dtype != DG_F32 && (p->path & 3) != 1 && i > 0) {
+        bool wg_done = dW == nullptr;
+        if (dW != nullptr && p->dtype != DG_F32 && (p->path & 3) != 1 && i > 0) {
             // tensor-core wgrad (wgrad_tc.cu); a decoder conv reads the MATERIALISED ConvTranspose output: the forward left it
             // in the workspace for the deep levels, for the fused levels it is rebuilt here by the same stand-alone kernel
             bool ok = true;
@@ -532,21 +564,23 @@ static int lw_backward_range(const dg_lw_params* p, const LwPlan& pl, const BwdP
                 }
             }
             if (ok) {
-                rc = conv3x3_wgrad_tc_launch(a, G(i), grads + gl.conv_w[b][j], 1, 9, 9 * bp.cin_tot[i], st, &wg_done, dRb_in);
+                rc = conv3x3_wgrad_tc_launch(a, G(i), dW, 1, 9, 9 * bp.cin_tot[i], st, &wg_done, dRb_in);
                 if (rc) return rc;
             }
             if (!wg_done) fwd_conv_args(p, pl, fw, x, N, i, &a, n0);  // restore the fused description for the generic kernel
         }
-        if (i == 0 && (p->path & 3) != 1 && p->in_channels == 1) {   // first conv: dedicated streaming kernel (backward.cu)
-            rc = first_wgrad_launch(x + (size_t)n0 * p->in_channels * H * W, G(0), grads + gl.conv_w[0][0], N, Hi, Wi, C, st, &wg_done);
+        if (dW != nullptr && i == 0 && (p->path & 3) != 1 && p->in_channels == 1) {   // first conv: dedicated streaming kernel (backward.cu)
+            rc = first_wgrad_launch(x + (size_t)n0 * p->in_channels * H * W, G(0), dW, N, Hi, Wi, C, st, &wg_done);
             if (rc) return rc;
         }
         if (!wg_done && dRb_in != nullptr) { set_error("backward: conv %d wgrad probe / launch mismatch", i); return 11; }
         if (!wg_done) {
-            rc = conv3x3_wgrad_launch(a, G(i), grads + gl.conv_w[b][j], /*tap*/ 1, /*ci*/ 9, /*co*/ 9 * bp.cin_tot[i], st);
+            rc = conv3x3_wgrad_launch(a, G(i), dW, /*tap*/ 1, /*ci*/ 9, /*co*/ 9 * bp.cin_tot[i], st);
             if (rc) return rc;
         }
-        if (i == 0) break;
+        if (!dgrad) break;
+        if (i == 0)   // dL/dx: dR_0 is fp32 in G(0) in every tier (conv 0 never gets the bf16 copy)
+            return first_dgrad_launch(G(0), p->conv_w[0][0], rq.grad_x + (size_t)n0 * p->in_channels * H * W, N, H, W, p->in_channels, C, st);
         // dA_in = conv3x3(dR_i, flipped weights): tensor cores where covered (dgrad_tc.cu) ...
         bool dg_done = false;
         bool act_fused = false;
@@ -612,17 +646,20 @@ static int lw_backward_range(const dg_lw_params* p, const LwPlan& pl, const BwdP
             float* dlow = reinterpret_cast<float*>(bw + bp.low_off[u]) + (size_t)n0 * (Hi / 2) * (Wi / 2) * pl.f[lvl + 1];
             // the low-resolution producer feeds nothing but this ConvTranspose: with the tensor-core data gradient its activation
             // backward is fused into that kernel's epilogue, which then writes G(i-1) / P(i-1) directly
-            const bool try_fuse = p->dtype != DG_F32 && (p->path & 3) != 1 && p->up_w_tc_bf16[u] != nullptr;
+            // (the ConvTranspose's own data gradient only when something below it, at conv i-1 or lower, is requested)
+            const bool low_wanted = rq.low < 2 * i - 1;
+            const bool try_fuse = low_wanted && p->dtype != DG_F32 && (p->path & 3) != 1 && p->up_w_tc_bf16[u] != nullptr;
             DgradAct lact{raw(i - 1), stats(i - 1), p->gn_w[b - 1][1], p->gn_b[b - 1][1], P(i - 1), p->groups[b - 1], p->dtype, 1e-5f};
             bool low_fused = false;
             rc = convt_bwd_launch(p->dtype, T(i), t_split[i] ? pl.f[lvl] : 2 * pl.f[lvl], p->up_w[u], p->up_w_t[u], raw(i - 1), stats(i - 1), p->gn_w[b - 1][1],
-                                  p->gn_b[b - 1][1], try_fuse ? G(i - 1) : dlow, grads + gl.up_w[u], grads + gl.up_b[u],
+                                  p->gn_b[b - 1][1], !low_wanted ? nullptr : try_fuse ? G(i - 1) : dlow, gp(gl.up_w[u]), gp(gl.up_b[u]),
                                   reinterpret_cast<float*>(bw + bp.coef_off) + (size_t)n0 * bp.maxc * 2, N, Hi, Wi, pl.f[lvl + 1], pl.f[lvl],
                                   p->groups[b - 1], 1e-5f, st, (p->path & 3) != 1 ? p->up_w_tc_bf16[u] : nullptr,
                                   try_fuse ? &lact : nullptr, try_fuse ? &low_fused : nullptr,
                                   (p->path & 3) != 1 ? p->up_w_dgrad_tc_bf16[u] : nullptr,
                                   p->dtype != DG_F32 ? bw + bp.gb_off[i] + (size_t)n0 * hwc(i, C) * 2 : nullptr);   // conv i's bf16 dR scratch is free again
             if (rc) return rc;
+            if (!low_wanted) break;
             if (low_fused) continue;   // G(i-1), P(i-1) are done
             if (try_fuse) {            // the kernel declined: G(i-1) holds the plain gradient; act_bwd works in place on it
                 rc = act_bwd(i - 1, G(i - 1), pl.f[lvl + 1], 0, nullptr, 0, 0);
@@ -1001,7 +1038,7 @@ int dg_lw_num_params(const dg_lw_params* p, size_t* count) {
     if (rc) return rc;
     GradLayout gl;
     make_grad_layout(p, pl, &gl);
-    if (count) *count = gl.total;
+    if (count) *count = gl.off[kLwTensors];
     return 0;
 }
 
@@ -1018,7 +1055,7 @@ int dg_lw_backward_workspace_bytes(const dg_lw_params* p, int32_t N, int32_t H, 
 int dg_lw_backward(const dg_lw_params* p, const float* x, const float* grad_y, int32_t N, int32_t H, int32_t W,
                    void* fwd_workspace, size_t fwd_bytes, void* bwd_workspace, size_t bwd_bytes, float* grads,
                    dg_stream_t stream) {
-    return lw_backward(p, x, grad_y, N, H, W, fwd_workspace, fwd_bytes, bwd_workspace, bwd_bytes, grads,
+    return lw_backward(p, x, grad_y, N, H, W, fwd_workspace, fwd_bytes, bwd_workspace, bwd_bytes, grads, ~0ull, nullptr,
                        reinterpret_cast<cudaStream_t>(stream));
 }
 
@@ -1028,8 +1065,33 @@ int dg_lw_backward_l1(const dg_lw_params* p, const float* x, const float* y, con
     if (y == nullptr || target == nullptr) { set_error("backward_l1: null output / target"); return 2; }
     if (p == nullptr) { set_error("null params"); return 2; }
     L1Seed l1{y, target, loss_grad, 1.0f / ((float)N * (float)p->out_channels * (float)H * (float)W)};
-    return lw_backward(p, x, nullptr, N, H, W, fwd_workspace, fwd_bytes, bwd_workspace, bwd_bytes, grads,
+    return lw_backward(p, x, nullptr, N, H, W, fwd_workspace, fwd_bytes, bwd_workspace, bwd_bytes, grads, ~0ull, nullptr,
                        reinterpret_cast<cudaStream_t>(stream), &l1);
+}
+
+int dg_lw_backward_select(const dg_lw_params* p, const float* x, const dg_lw_bwd_request* r, int32_t N, int32_t H, int32_t W,
+                          void* fwd_workspace, size_t fwd_bytes, void* bwd_workspace, size_t bwd_bytes, dg_stream_t stream) {
+    if (r == nullptr) { set_error("backward_select: null request"); return 2; }
+    const bool l1_seed = r->y != nullptr || r->target != nullptr;
+    if ((r->grad_y != nullptr) == l1_seed) {
+        set_error("backward_select: give exactly one gradient seed, grad_y or the fused-L1 (y, target)");
+        return 2;
+    }
+    if (l1_seed && (r->y == nullptr || r->target == nullptr)) { set_error("backward_select: the fused-L1 seed needs both y and target"); return 2; }
+    if (r->param_mask != 0 && r->grads == nullptr) { set_error("backward_select: param_mask 0x%llx without a grads buffer", (unsigned long long)r->param_mask); return 2; }
+    if (r->param_mask == 0 && r->grad_x == nullptr) { set_error("backward_select: nothing requested (param_mask 0, grad_x NULL)"); return 2; }
+    if (p == nullptr) { set_error("null params"); return 2; }
+    if (int rc = check_path(p->path, "lw")) return rc;
+    if (r->grad_x != nullptr && p->conv_w[0][0] == nullptr) { set_error("backward_select: grad_x needs conv_w[0][0]"); return 2; }
+    L1Seed l1{r->y, r->target, r->loss_grad, 1.0f / ((float)N * (float)p->out_channels * (float)H * (float)W)};
+    return lw_backward(p, x, r->grad_y, N, H, W, fwd_workspace, fwd_bytes, bwd_workspace, bwd_bytes, r->grads, r->param_mask, r->grad_x,
+                       reinterpret_cast<cudaStream_t>(stream), l1_seed ? &l1 : nullptr);
+}
+
+int dg_conv_first_dgrad(const float* dR, const float* w, float* dx, int32_t N, int32_t H, int32_t W, int32_t cin, int32_t cout,
+                        dg_stream_t stream) {
+    if (dR == nullptr || w == nullptr || dx == nullptr) { set_error("first dgrad: null pointer"); return 2; }
+    return first_dgrad_launch(dR, w, dx, N, H, W, cin, cout, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int dg_l1_loss_sum(const float* y, const float* target, size_t count, double* sum, dg_stream_t stream) {

@@ -151,7 +151,7 @@ struct GnBwdArgs {
     float* G;  // in: G, out: dR (unless dRb)
     void* dRb; // vector kernel only: write dR as bf16 [N,H,W,C] HERE instead of fp32 in place -- the tensor-core wgrad / dgrad round
                // it to bf16 anyway, so they read half the bytes and copy instead of converting (bit-identical results)
-    float* dgamma; float* dbeta;
+    float* dgamma; float* dbeta;   // either NULL = not computed (frozen)
     int N, H, W, C, groups; float eps;
 };
 
@@ -173,15 +173,15 @@ __global__ void __launch_bounds__(BW_THREADS) gn_bwd_apply_kernel(const GnBwdArg
         gsm[5 * c] = m; gsm[5 * c + 1] = r; gsm[5 * c + 2] = p.gamma[c];
         gsm[5 * c + 3] = (float)(m1 / cnt); gsm[5 * c + 4] = (float)(m2 / cnt);
     }
-    if (blockIdx.x == 0 && blockIdx.y == 0 && p.dgamma != nullptr) {
+    if (blockIdx.x == 0 && blockIdx.y == 0 && (p.dgamma != nullptr || p.dbeta != nullptr)) {
         for (int c = threadIdx.x; c < C; c += BW_THREADS) {
             double dg = 0.0, db = 0.0;
             for (int i = 0; i < p.N; ++i) {
                 db += p.P[((size_t)i * C + c) * 2];
                 dg += p.P[((size_t)i * C + c) * 2 + 1];
             }
-            atomicAdd(p.dgamma + c, (float)dg);   // accumulated: concurrent sub-batches (api.cu) each add their images' share
-            atomicAdd(p.dbeta + c, (float)db);
+            if (p.dgamma) atomicAdd(p.dgamma + c, (float)dg);   // accumulated: concurrent sub-batches (api.cu) each add their images' share
+            if (p.dbeta) atomicAdd(p.dbeta + c, (float)db);
         }
     }
     __syncthreads();
@@ -339,15 +339,15 @@ __global__ void __launch_bounds__(BW_THREADS) gn_bwd_apply_vec_kernel(const GnBw
         gsm[5 * c] = m; gsm[5 * c + 1] = r; gsm[5 * c + 2] = p.gamma[c];
         gsm[5 * c + 3] = (float)(m1 / cnt); gsm[5 * c + 4] = (float)(m2 / cnt);
     }
-    if (blockIdx.x == 0 && blockIdx.y == 0 && p.dgamma != nullptr) {
+    if (blockIdx.x == 0 && blockIdx.y == 0 && (p.dgamma != nullptr || p.dbeta != nullptr)) {
         for (int c = threadIdx.x; c < C; c += BW_THREADS) {
             double dg = 0.0, db = 0.0;
             for (int i = 0; i < p.N; ++i) {
                 db += p.P[((size_t)i * C + c) * 2];
                 dg += p.P[((size_t)i * C + c) * 2 + 1];
             }
-            atomicAdd(p.dgamma + c, (float)dg);   // accumulated: concurrent sub-batches (api.cu) each add their images' share
-            atomicAdd(p.dbeta + c, (float)db);
+            if (p.dgamma) atomicAdd(p.dgamma + c, (float)dg);   // accumulated: concurrent sub-batches (api.cu) each add their images' share
+            if (p.dbeta) atomicAdd(p.dbeta + c, (float)db);
         }
     }
     __syncthreads();
@@ -391,7 +391,7 @@ struct HeadBwdArgs {
     const float* dOut;    // [N,OC,H,W]
     const float* w;       // [OC][C]
     float* G; double* P;  // [N,H,W,C], [N,C,2]
-    float* dW; float* dB; // [OC][C], [OC] accumulated atomically (zero on entry)
+    float* dW; float* dB; // [OC][C], [OC] accumulated atomically (zero on entry); either NULL = not computed (frozen)
     int N, H, W, C, OC, groups; float eps;
     // nn.L1Loss backward fused (optimized_train.py:439,210/226): when `target` is set, dOut is not read at all -- the seed
     // sign(y - target) * (*scale) * inv_numel is generated here from the forward output y (sign(0) = 0, as torch)
@@ -455,8 +455,8 @@ __global__ void __launch_bounds__(BW_THREADS) head_bwd_kernel(const HeadBwdArgs 
     }
     __syncthreads();
     for (int i = threadIdx.x; i < 2 * C; i += BW_THREADS) atomicAdd(p.P + (size_t)n * C * 2 + i, psm[i]);
-    for (int i = threadIdx.x; i < OC * C; i += BW_THREADS) atomicAdd(p.dW + i, (float)wacc[i]);
-    for (int i = threadIdx.x; i < OC; i += BW_THREADS) atomicAdd(p.dB + i, (float)wacc[OC * C + i]);
+    if (p.dW) for (int i = threadIdx.x; i < OC * C; i += BW_THREADS) atomicAdd(p.dW + i, (float)wacc[i]);
+    if (p.dB) for (int i = threadIdx.x; i < OC; i += BW_THREADS) atomicAdd(p.dB + i, (float)wacc[OC * C + i]);
 }
 
 // ---- ConvTranspose2d(k=2,s=2) backward ---------------------------------------------------------------------------------
@@ -741,8 +741,8 @@ __global__ void __launch_bounds__(BW_THREADS) head_bwd_fast_kernel(const HeadBwd
         for (int k = 0; k < BW_THREADS / 32; ++k) t += (double)slot[k][i];
         if (i < C) atomicAdd(p.P + ((size_t)n * C + i) * 2, t);
         else if (i < 2 * C) atomicAdd(p.P + ((size_t)n * C + (i - C)) * 2 + 1, t);
-        else if (i < 3 * C) atomicAdd(p.dW + (i - 2 * C), (float)t);
-        else atomicAdd(p.dB, (float)t);
+        else if (i < 3 * C) { if (p.dW) atomicAdd(p.dW + (i - 2 * C), (float)t); }
+        else if (p.dB) atomicAdd(p.dB, (float)t);
     }
 }
 
@@ -809,6 +809,91 @@ __global__ void __launch_bounds__(BW_THREADS) first_wgrad_kernel(const float* __
         for (int w = 0; w < BW_THREADS / 32; ++w) v += red[w][i];
         const int t = i / CO, k = i - t * CO;
         atomicAdd(dW + k * 9 + t, v);   // parameter layout [CO][1][3][3]
+    }
+}
+
+// ---- data gradient of the first conv w.r.t. the input image (enc1.0, src/model.py:93) ------------------------------------------
+// dX[n,ci,y,x] = sum_{ky,kx,co} dR[n, y+1-ky, x+1-kx, co] * W[ky][kx][ci][co], zero padding.  Memory-bound: dR fp32 read once,
+// dX fp32 written once, every output pixel its own sum (no atomics).  One CTA per output tile.
+// in_channels == 1: every dR pixel of the haloed tile is first contracted over co with all 9 taps (v[t] = sum_co dR[co] W[t][co],
+// dR read straight from global memory), then each output pixel adds its 9 shifted v[t] out of shared memory -- 72 B of shared
+// traffic per pixel instead of 9 * C * 4 for re-reading a staged dR tile per tap.
+template <int C>
+__global__ void __launch_bounds__(BW_THREADS, 4) first_dgrad_kernel(const float* __restrict__ dR, const float* __restrict__ w,
+                                                                     float* __restrict__ dx, int H, int W, int tiles_x, int tiles_y) {
+    constexpr int TH = 16, TW = 64, PH = TH + 2, PW = TW + 2;
+    __shared__ float wsm[9 * C];          // [tap][co]
+    __shared__ float v[9][PH * PW];       // per tap: the contracted haloed tile
+    for (int i = threadIdx.x; i < 9 * C; i += BW_THREADS) wsm[i] = __ldg(w + i);
+    const int tiles_per_img = tiles_x * tiles_y;
+    const int n = blockIdx.x / tiles_per_img, tr = blockIdx.x - n * tiles_per_img;
+    const int y0 = (tr / tiles_x) * TH, x0 = (tr % tiles_x) * TW;
+    __syncthreads();
+    for (int q = threadIdx.x; q < PH * PW; q += BW_THREADS) {
+        const int r = q / PW, c = q - r * PW;
+        const int gy = y0 + r - 1, gx = x0 + c - 1;
+        float d[C];
+        if ((unsigned)gy < (unsigned)H && (unsigned)gx < (unsigned)W) {
+            const float4* s = reinterpret_cast<const float4*>(dR + (((size_t)n * H + gy) * W + gx) * C);
+#pragma unroll
+            for (int k = 0; k < C / 4; ++k) {
+                const float4 f = __ldg(s + k);
+                d[4 * k] = f.x; d[4 * k + 1] = f.y; d[4 * k + 2] = f.z; d[4 * k + 3] = f.w;
+            }
+        } else {
+#pragma unroll
+            for (int k = 0; k < C; ++k) d[k] = 0.f;
+        }
+#pragma unroll
+        for (int t = 0; t < 9; ++t) {
+            float a = 0.f;
+#pragma unroll
+            for (int k = 0; k < C; ++k) a = fmaf(d[k], wsm[t * C + k], a);
+            v[t][q] = a;
+        }
+    }
+    __syncthreads();
+    for (int pix = threadIdx.x; pix < TH * TW; pix += BW_THREADS) {
+        const int r = pix / TW, c = pix - r * TW;
+        const int gy = y0 + r, gx = x0 + c;
+        if (gy >= H || gx >= W) continue;
+        float s = 0.f;
+#pragma unroll
+        for (int t = 0; t < 9; ++t) s += v[t][(r + 2 - t / 3) * PW + c + 2 - t % 3];
+        dx[((size_t)n * H + gy) * W + gx] = s;
+    }
+}
+
+// any in_channels and C (fs=12 with in=3, the wide fs=64 variant): the haloed dR tile staged in shared memory with an odd row
+// stride (conflict-free reads for every C), one output pixel per thread, all input channels
+__global__ void __launch_bounds__(BW_THREADS) first_dgrad_any_kernel(const float* __restrict__ dR, const float* __restrict__ w,
+                                                                     float* __restrict__ dx, int H, int W, int CI, int C, int tiles_x,
+                                                                     int tiles_y) {
+    constexpr int TH = 8, TW = 32, PW = TW + 2;
+    static_assert(TH * TW == BW_THREADS, "one output pixel per thread");
+    extern __shared__ float dsm[];        // [(TH + 2) * PW][SC]
+    const int SC = C | 1;
+    const int tiles_per_img = tiles_x * tiles_y;
+    const int n = blockIdx.x / tiles_per_img, tr = blockIdx.x - n * tiles_per_img;
+    const int y0 = (tr / tiles_x) * TH, x0 = (tr % tiles_x) * TW;
+    for (int i = threadIdx.x; i < (TH + 2) * PW * C; i += BW_THREADS) {
+        const int q = i / C, co = i - q * C;
+        const int r = q / PW, c = q - r * PW;
+        const int gy = y0 + r - 1, gx = x0 + c - 1;
+        dsm[q * SC + co] = ((unsigned)gy < (unsigned)H && (unsigned)gx < (unsigned)W) ? __ldg(dR + (((size_t)n * H + gy) * W + gx) * C + co) : 0.f;
+    }
+    __syncthreads();
+    const int r = threadIdx.x / TW, c = threadIdx.x % TW;
+    const int gy = y0 + r, gx = x0 + c;
+    if (gy >= H || gx >= W) return;
+    for (int ci = 0; ci < CI; ++ci) {
+        float s = 0.f;
+        for (int t = 0; t < 9; ++t) {
+            const float* d = dsm + ((r + 2 - t / 3) * PW + c + 2 - t % 3) * SC;
+            const float* wt = w + ((size_t)t * CI + ci) * C;
+            for (int co = 0; co < C; ++co) s = fmaf(d[co], __ldg(wt + co), s);
+        }
+        dx[(((size_t)n * CI + ci) * H + gy) * W + gx] = s;
     }
 }
 
@@ -882,6 +967,32 @@ int first_wgrad_launch(const float* x, const float* dR, float* dW, int N, int H,
     *handled = true;
     count_launch();
     return check_launch("first_wgrad");
+}
+
+// dX fp32 NCHW [N,CI,H,W] = first-layer input gradient; dR fp32 [N,H,W,C], w = the packed [3][3][CI][C] forward weights
+int first_dgrad_launch(const float* dR, const float* w, float* dx, int N, int H, int W, int CI, int C, cudaStream_t st) {
+    if (N < 1 || H < 1 || W < 1 || CI < 1 || C < 1) { set_error("first dgrad: bad shape %dx%dx%dx%d -> %d", N, C, H, W, CI); return 3; }
+    if (CI == 1 && (C == 8 || C == 16) && aligned16(dR)) {
+        const int tx = (W + 63) / 64, ty = (H + 15) / 16;
+        if ((size_t)tx * ty * N > 0x7fffffff) { set_error("first dgrad: too many tiles"); return 3; }
+        if (C == 8) first_dgrad_kernel<8><<<tx * ty * N, BW_THREADS, 0, st>>>(dR, w, dx, H, W, tx, ty);
+        else first_dgrad_kernel<16><<<tx * ty * N, BW_THREADS, 0, st>>>(dR, w, dx, H, W, tx, ty);
+        count_launch();
+        return check_launch("first_dgrad");
+    }
+    const int tx = (W + 31) / 32, ty = (H + 7) / 8;
+    if ((size_t)tx * ty * N > 0x7fffffff) { set_error("first dgrad: too many tiles"); return 3; }
+    const size_t smem = (size_t)10 * 34 * (C | 1) * sizeof(float);
+    if (smem > 227 * 1024) { set_error("first dgrad: %d channels need %zu B of shared memory", C, smem); return 3; }
+    static size_t smem_set = 48 * 1024;
+    if (smem > smem_set) {
+        cudaError_t e = cudaFuncSetAttribute(first_dgrad_any_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) { set_error("first dgrad: cudaFuncSetAttribute(%zu B): %s", smem, cudaGetErrorString(e)); return 4; }
+        smem_set = smem;
+    }
+    first_dgrad_any_kernel<<<tx * ty * N, BW_THREADS, smem, st>>>(dR, w, dx, H, W, CI, C, tx, ty);
+    count_launch();
+    return check_launch("first_dgrad_any");
 }
 
 // dRb (optional): ask for the bf16 copy instead of the in-place fp32 result; *wrote_bf16 reports whether that happened (only the
@@ -970,12 +1081,14 @@ int convt_bwd_launch(int dtype, const float* dCat, int stride, const float* wt, 
     if (act_fused) *act_fused = false;
     if (Cu % 4 || (stride % 4) || (reinterpret_cast<uintptr_t>(dCat) & 15)) { set_error("convT backward: unaligned gradient"); return 3; }
     ConvtBwdArgs a{dCat, stride, wt, wt_t, raw_low, stats, gamma, beta, dAlow, dWt, nullptr, coefbuf, N, H, W, Cl, Cu, groups, eps};
-    gn_mean_rstd_kernel<<<N, 128, 0, st>>>(stats, coefbuf, Cl, groups, (double)(H / 2) * (W / 2), eps);
-    count_launch();
+    if (dWt != nullptr) {
+        gn_mean_rstd_kernel<<<N, 128, 0, st>>>(stats, coefbuf, Cl, groups, (double)(H / 2) * (W / 2), eps);
+        count_launch();
+    }
     const size_t total = (size_t)N * (H / 2) * (W / 2) * Cl;
     int rc = 0;
-    bool data_done = false;
-    if (dtype != DG_F32 && wtc_bf16 != nullptr) {   // tensor cores where covered (dgrad_tc.cu)
+    bool data_done = dAlow == nullptr;   // NULL: nothing below the ConvTranspose wants a gradient
+    if (!data_done && dtype != DG_F32 && wtc_bf16 != nullptr) {   // tensor cores where covered (dgrad_tc.cu)
         if (act != nullptr && act_fused != nullptr) {   // dAlow is then G of the low-resolution producer, never the plain gradient
             rc = convt_dgrad_tc_launch(dCat, stride, wtc_bf16, dAlow, N, H, W, Cl, Cu, st, &data_done, act);
             if (rc) return rc;
@@ -998,25 +1111,36 @@ int convt_bwd_launch(int dtype, const float* dCat, int stride, const float* wt, 
         if (rc) return rc;
     }
     // weight + bias gradient on the tensor cores where the configuration is covered (wgrad_tc.cu: the bias sum rides on the
-    // gradient staging), else the two CUDA-core kernels below
-    {
+    // gradient staging), else the two CUDA-core kernels below.  dWt / dBias NULL = frozen: its kernel does not run (a frozen
+    // weight with a trained bias takes the bias kernel alone)
+    if (dWt != nullptr) {
         bool handled = false;
         rc = convt_wgrad_tc_launch(dtype, dCat, stride, raw_low, stats, gamma, beta, dWt, dBias, N, H, W, Cl, Cu, groups, eps, st, &handled);
         if (rc || handled) return rc;
     }
-    // bias gradient
-    ConvtBwdArgs ab = a;
-    ab.dBias = dBias;
-    int bb = (int)(((size_t)N * H * W * Cu + BW_THREADS * 16 - 1) / (BW_THREADS * 16));
-    if (bb > 1024) bb = 1024;
-    if (bb < 1) bb = 1;
-    convt_bwd_bias_kernel<<<bb, BW_THREADS, (size_t)Cu * sizeof(float), st>>>(ab);
-    count_launch();
+    if (dBias != nullptr) {
+        ConvtBwdArgs ab = a;
+        ab.dBias = dBias;
+        int bb = (int)(((size_t)N * H * W * Cu + BW_THREADS * 16 - 1) / (BW_THREADS * 16));
+        if (bb > 1024) bb = 1024;
+        if (bb < 1) bb = 1;
+        convt_bwd_bias_kernel<<<bb, BW_THREADS, (size_t)Cu * sizeof(float), st>>>(ab);
+        count_launch();
+    }
+    if (dWt == nullptr) return check_launch("convt_bwd_bias");
     // weight gradient: 256 combos per CTA
     // slab sized for ~32 KB of staged operands
     const int ncombo = 4 * Cl * Cu;
     const int per_cta_ci = (BW_THREADS / Cu) < 1 ? 1 : (BW_THREADS / Cu) + 1;
-    const int width = (Cl * Cu >= BW_THREADS) ? (per_cta_ci + Cu) : (Cl + 4 * Cu);  // floats staged per low pixel (upper bound)
+    int width = (Cl * Cu >= BW_THREADS) ? (per_cta_ci + Cu) : (Cl + 4 * Cu);  // floats staged per low pixel (upper bound)
+    // ... which the kernel's own (ci, position) ranges can exceed when Cl * Cu is not a multiple of BW_THREADS (a CTA whose combos
+    // cross a position stages every input channel and two positions): take the largest nci + nab * Cu over the CTAs
+    for (int c_first = 0; c_first < ncombo; c_first += BW_THREADS) {
+        const int c_last = min(c_first + BW_THREADS, ncombo) - 1;
+        const int ab_lo = c_first / (Cl * Cu), ab_hi = c_last / (Cl * Cu);
+        const int nci = ab_hi > ab_lo ? Cl : (c_last / Cu) % Cl - (c_first / Cu) % Cl + 1;
+        width = max(width, nci + (ab_hi - ab_lo + 1) * Cu);
+    }
     int slab = 8192 / width;
     if (slab > 128) slab = 128;
     if (slab < 8) slab = 8;

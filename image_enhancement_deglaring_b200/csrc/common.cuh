@@ -179,6 +179,7 @@ int convt_dgrad_t5_launch(const float* dCat, int stride, void* scratch_bf16, con
 int image_metrics_launch(const float* out, const float* tgt, int N, int H, int W, int clip01, double data_range, double* acc,
                          cudaStream_t st);
 int first_wgrad_launch(const float* x, const float* dR, float* dW, int N, int H, int W, int CO, cudaStream_t st, bool* handled);
+int first_dgrad_launch(const float* dR, const float* w, float* dx, int N, int H, int W, int CI, int C, cudaStream_t st);
 
 int convt_wgrad_tc_launch(int dtype, const float* dCat, int stride, const void* raw_low, const double* stats, const float* gamma,
                           const float* beta, float* dWt, float* dBias, int N, int H, int W, int Cl, int Cu, int groups, float eps,

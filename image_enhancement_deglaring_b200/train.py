@@ -3,8 +3,9 @@
 Reference call sequence (optimized_train.py:197-236, fp32 branch :220-233):
     optimizer.zero_grad(set_to_none=True); outputs = model(inputs); loss = criterion(outputs, targets)
     loss.backward(); clip_grad_norm_(model.parameters(), 1.0); optimizer.step()
-`model(inputs)` lands in `lightweight_forward_train` when autograd is recording; gradients of every parameter come back
-through `torch.autograd.Function.backward`, i.e. they land in `param.grad` the normal way (wandb.watch hooks keep working).
+`model(inputs)` lands in `lightweight_forward_train` when autograd is recording; the gradients autograd asks for (every parameter
+that requires one, and the input image when it does) come back through `torch.autograd.Function.backward`, i.e. they land in
+`param.grad` / `x.grad` the normal way (wandb.watch hooks keep working).  Frozen parameters cost no kernel work.
 `FusedAdamW` is a `torch.optim.Optimizer` with AdamW's constructor that keeps parameters, gradients and both moments in flat
 buffers and runs clip + update as two kernels (dg_adamw_step).
 
@@ -54,6 +55,7 @@ class _LightweightUNetFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, module, tctx, x, *params):
         lib = _lib.load()
+        x_dtype = x.dtype
         x = x.detach().float().contiguous()
         N, _, H, W = x.shape
         with torch.cuda.device(x.device):
@@ -63,6 +65,7 @@ class _LightweightUNetFn(torch.autograd.Function):
             _lib.check(lib.dg_lw_forward(C.byref(pc), x.data_ptr(), y.data_ptr(), N, H, W, ws.data_ptr(), ws.numel(),
                                          None, None, torch.cuda.current_stream().cuda_stream))
         ctx.module, ctx.ws, ctx.x, ctx.tctx = module, ws, x, tctx
+        ctx.x_dtype = x_dtype
         ctx.n_inputs = len(params)
         ctx.direct = getattr(module, "_dg_direct_grads", False)
         tctx.y = y
@@ -75,6 +78,14 @@ class _LightweightUNetFn(torch.autograd.Function):
         N, _, H, W = x.shape
         params = list(module.parameters())
         total = sum(p.numel() for p in params)
+        # Only what autograd asks for is computed: dL/dx when x needs it, the gradients of parameters that require one, and the
+        # backward stops below the lowest of them.  GraphedTrainStep's parameters are not autograd inputs: it always wants all.
+        want_x = ctx.needs_input_grad[2]
+        want_p = [True] * len(params) if ctx.direct else list(ctx.needs_input_grad[3:])
+        if len(want_p) != 64:
+            raise RuntimeError(f"gradient layout mismatch: {len(want_p)} parameter tensors, the library's backward has 64")
+        mask = sum(1 << k for k, w in enumerate(want_p) if w)
+        select = want_x or not all(want_p)
         with torch.cuda.device(x.device):
             pc = module._refresh(train=True)
             nb = C.c_size_t(0)
@@ -85,35 +96,52 @@ class _LightweightUNetFn(torch.autograd.Function):
             if cnt.value != total:
                 raise RuntimeError(f"gradient layout mismatch: library {cnt.value} vs module {total}")
             # gradients go straight into the optimizer's flat bucket when that is safe (fresh after zero_grad, no hooks): no
-            # per-parameter accumulate kernels, no temporary
-            sink = _flat_grad_sink(params) if total > 0 else None
+            # per-parameter accumulate kernels, no temporary.  A fully frozen net gets no flat buffer at all.
+            sink = _flat_grad_sink(params) if total > 0 and mask else None
             if ctx.direct and sink is None:
                 raise RuntimeError("GraphedTrainStep: the gradients must land in the optimizer's flat bucket (FusedAdamW.zero_grad "
                                    "inside the step, no per-parameter hooks)")
-            flat = sink if sink is not None else torch.empty(total, dtype=torch.float32, device=x.device)
+            flat = sink if sink is not None else (torch.empty(total, dtype=torch.float32, device=x.device) if mask else None)
+            grad_x = torch.empty_like(x) if want_x else None
             stream = torch.cuda.current_stream().cuda_stream
             fused_l1 = (tctx.l1_target is not None and tctx.l1_marker is not None and grad_y.data_ptr() == tctx.l1_marker.data_ptr()
                         and all(s == 0 for s in grad_y.stride()))
-            if fused_l1:   # loss = L1Loss (below): the seed sign(y - t) * dloss / numel is generated inside the head backward
+            if not fused_l1:
+                grad_y = grad_y.detach().float().contiguous()
+            if select:
+                req = _lib.DgLwBwdRequest()
+                if fused_l1:
+                    req.y, req.target, req.loss_grad = tctx.y.data_ptr(), tctx.l1_target.data_ptr(), tctx.l1_scale.data_ptr()
+                else:
+                    req.grad_y = grad_y.data_ptr()
+                req.grads = flat.data_ptr() if flat is not None else None
+                req.param_mask = mask
+                req.grad_x = grad_x.data_ptr() if grad_x is not None else None
+                _lib.check(lib.dg_lw_backward_select(C.byref(pc), x.data_ptr(), C.byref(req), N, H, W, ctx.ws.data_ptr(),
+                                                     ctx.ws.numel(), bws.data_ptr(), bws.numel(), stream))
+            elif fused_l1:   # loss = L1Loss (below): the seed sign(y - t) * dloss / numel is generated inside the head backward
                 _lib.check(lib.dg_lw_backward_l1(C.byref(pc), x.data_ptr(), tctx.y.data_ptr(), tctx.l1_target.data_ptr(),
                                                  tctx.l1_scale.data_ptr(), N, H, W, ctx.ws.data_ptr(), ctx.ws.numel(),
                                                  bws.data_ptr(), bws.numel(), flat.data_ptr(), stream))
             else:
-                grad_y = grad_y.detach().float().contiguous()
                 _lib.check(lib.dg_lw_backward(C.byref(pc), x.data_ptr(), grad_y.data_ptr(), N, H, W, ctx.ws.data_ptr(),
                                               ctx.ws.numel(), bws.data_ptr(), bws.numel(), flat.data_ptr(), stream))
         ctx.ws = None
         tctx.y = tctx.l1_target = tctx.l1_scale = tctx.l1_marker = None
-        sync_gradients(flat, getattr(module, "ddp_sync", True))
+        if grad_x is not None and grad_x.dtype != ctx.x_dtype:
+            grad_x = grad_x.to(ctx.x_dtype)
+        if flat is None:
+            return (None, None, grad_x) + (None,) * ctx.n_inputs
+        sync_gradients(flat, getattr(module, "ddp_sync", True))   # parameter gradients only: dL/dx is per rank's own batch
         if sink is not None:
             sink._dg_zero_version = None      # the bucket now holds a gradient: a second backward must accumulate the ordinary way
-            return (None, None, None) + (None,) * ctx.n_inputs
+            return (None, None, grad_x) + (None,) * ctx.n_inputs
         grads, off = [], 0
-        for p in params:
+        for p, want in zip(params, want_p):
             n = p.numel()
-            grads.append(flat[off:off + n].view_as(p) if p.requires_grad else None)
+            grads.append(flat[off:off + n].view_as(p) if want else None)   # a frozen range of `flat` is never written
             off += n
-        return (None, None, None, *grads)
+        return (None, None, grad_x, *grads)
 
 
 class _FusedL1(torch.autograd.Function):
@@ -172,10 +200,10 @@ def sync_gradients(flat, enabled=True, group=None):
 
 
 def lightweight_forward_train(module, x):
-    if x.requires_grad:
-        raise NotImplementedError("gradient w.r.t. the input image is not implemented (the reference never needs it)")
     tctx = _TrainCtx()
     if getattr(module, "_dg_direct_grads", False):
+        if x.requires_grad:
+            raise NotImplementedError("GraphedTrainStep computes parameter gradients only, not the input image's")
         # GraphedTrainStep: the parameters are NOT autograd inputs -- their AccumulateGrad nodes carry the stream they were created
         # on (the default stream if an eager step's graph is still alive), and the engine would synchronise the capturing stream
         # with it at the end of backward (cudaErrorStreamCaptureIsolation).  A fresh leaf anchors the node instead; the gradients

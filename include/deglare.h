@@ -276,7 +276,9 @@ int dg_lw_layout(const dg_lw_params* p, int32_t N, int32_t H, int32_t W, int32_t
  *   enc1.0.weight, enc1.1.weight, enc1.1.bias, enc1.3.weight, enc1.4.weight, enc1.4.bias, enc2..., bottleneck...,
  *   upconv4.weight, upconv4.bias, dec4..., upconv3..., dec3..., upconv2..., dec2..., upconv1..., dec1...,
  *   output_conv.weight, output_conv.bias.
- * grad_y is dL/d(output) fp32 [N,out,H,W] (nn.L1Loss backward = sign(o-t)/numel comes from the caller's autograd). */
+ * grad_y is dL/d(output) fp32 [N,out,H,W] (nn.L1Loss backward = sign(o-t)/numel comes from the caller's autograd).
+ * dg_lw_backward_l1 below takes the L1 loss's seed instead of grad_y; dg_lw_backward_select computes only a requested subset of
+ * the gradients, the input image's included. */
 int dg_lw_num_params(const dg_lw_params* p, size_t* count);
 int dg_lw_backward_workspace_bytes(const dg_lw_params* p, int32_t N, int32_t H, int32_t W, size_t* bytes);
 int dg_lw_backward(const dg_lw_params* p, const float* x, const float* grad_y, int32_t N, int32_t H, int32_t W,
@@ -292,6 +294,33 @@ int dg_l1_loss_sum(const float* y, const float* target, size_t count, double* su
 int dg_lw_backward_l1(const dg_lw_params* p, const float* x, const float* y, const float* target, const float* loss_grad,
                       int32_t N, int32_t H, int32_t W, void* fwd_workspace, size_t fwd_bytes, void* bwd_workspace, size_t bwd_bytes,
                       float* grads, dg_stream_t stream);
+
+/* dg_lw_backward_select: the backward of dg_lw_backward / dg_lw_backward_l1 restricted to the gradients a caller asks for -- the
+ * input-image gradient and any subset of the 64 parameter tensors (frozen layers, decoder-only fine-tuning).  The kernels of
+ * parameter tensors that are not requested do not run, and the backward stops below the lowest requested tensor in forward
+ * order (conv i and the GroupNorm after it at position i, an upconv just before the decoder conv that consumes it, the head
+ * last, x first).  With every bit of param_mask set and grad_x == NULL it launches exactly what dg_lw_backward launches.
+ * Returns 2 when both or neither gradient seed is given, when param_mask != 0 and grads == NULL, and when nothing is requested. */
+typedef struct {
+    const float* grad_y;      /* dL/dy fp32 [N,out,H,W]; or NULL and the fused-L1 seed below                               */
+    const float* y;           /* fused L1 seed (as dg_lw_backward_l1): forward output, target, device dL/dloss or NULL (= 1) */
+    const float* target;
+    const float* loss_grad;
+    float* grads;             /* flat buffer in parameters() order (dg_lw_num_params elements) or NULL                      */
+    uint64_t param_mask;      /* bit k = the k-th of the 64 parameter tensors in the order listed above dg_lw_num_params;
+                                 only those are written (zeroed, then set), the others are left untouched; 0 = none         */
+    float* grad_x;            /* dL/dx fp32 NCHW [N,in,H,W], overwritten; NULL = not wanted                                 */
+} dg_lw_bwd_request;
+
+int dg_lw_backward_select(const dg_lw_params* p, const float* x, const dg_lw_bwd_request* r, int32_t N, int32_t H, int32_t W,
+                          void* fwd_workspace, size_t fwd_bytes, void* bwd_workspace, size_t bwd_bytes, dg_stream_t stream);
+
+/* dg_conv_first_dgrad: data gradient of the first conv (enc1.0) w.r.t. the input image, the last step of dg_lw_backward_select
+ * when grad_x is requested:  dX[n,ci,y,x] = sum_{ky,kx,co} dR[n, y+1-ky, x+1-kx, co] * W[co][ci][ky][kx]  (zero padding).
+ * dR fp32 NHWC [N,H,W,cout]; w = the packed fp32 [3][3][cin][cout] weights (dg_lw_params.conv_w[0][0]); dX fp32 NCHW
+ * [N,cin,H,W], overwritten.  CUDA cores, fp32; exposed for per-op tests. */
+int dg_conv_first_dgrad(const float* dR, const float* w, float* dx, int32_t N, int32_t H, int32_t W, int32_t cin, int32_t cout,
+                        dg_stream_t stream);
 
 /* Fused optimizer tail over flat buffers: torch.nn.utils.clip_grad_norm_(max_norm) (skipped if max_norm <= 0) followed by
  * torch.optim.AdamW (optimized_train.py:215-218,230-233,440-446).  grads are first multiplied by grad_scale (1/world after a
