@@ -48,9 +48,9 @@ static const char* const kConvNames[18] = {"enc1.0", "enc1.3", "enc2.0", "enc2.3
                                            "bottleneck.3", "up4+dec4.0", "dec4.3", "up3+dec3.0", "dec3.3", "up2+dec2.0", "dec2.3",
                                            "up1+dec1.0", "dec1.3"};
 
-// Path bits 2-6 selected kernel variants that measured slower and were removed.  A caller that still sets one gets an error rather
-// than different kernels than it asked for.
-constexpr int32_t kRemovedPathBits = 0x7c;
+// Path bits 2-6 and 11 selected kernel variants that measured slower and were removed.  A caller that still sets one gets an error
+// rather than different kernels than it asked for.
+constexpr int32_t kRemovedPathBits = 0x87c;
 static int check_path(int32_t path, const char* who) {
     if (path & kRemovedPathBits) {
         set_error("%s: path %d sets bit %d, whose kernel variant was removed", who, path, __builtin_ctz(path & kRemovedPathBits));
@@ -192,10 +192,7 @@ static int lw_forward_range(const dg_lw_params* p, const LwPlan& pl, char* ws, c
             a.weight_comp = p->dec_comp[u];
             // deep levels (upconv4, upconv3): run the transposed conv as its own tensor-core GEMM and
             // feed its output as an identity source -- see convt_tc.cu for why this beats fusing there
-            // composite weights present for a level the tcgen05 decoder mode covers (C_up >= 16): ConvTranspose, concat and conv run
-            // as one low-resolution conv in conv3x3_t5.cu -- no stand-alone ConvTranspose, no `up` tensor
-            const bool dec_t5 = p->dec_comp[u] != nullptr && !(p->path & (128 | 1024)) && pl.f[lvl] >= 16;
-            const bool unfuse = p->dtype != DG_F32 && (p->path & 3) != 1 && lw_up_materialised(pl, u) && !dec_t5;
+            const bool unfuse = p->dtype != DG_F32 && (p->path & 3) != 1 && lw_up_materialised(pl, u);
             if (unfuse) {
                 bool handled = false;
                 void* up = ws + pl.up_off[u] + (size_t)n0 * a.H * a.W * pl.f[lvl] * esz;

@@ -454,64 +454,9 @@ int launch_dec(const DecArgs& a, cudaStream_t st) {
 
 }  // namespace
 
-// ---- composite weights for the tcgen05 decoder mode (conv3x3_t5.cu T5_DEC): the ConvTranspose + concat + conv as ONE 3x3 conv on the
-// low-resolution grid.  Wp fp32 [3][3][3 CL][4 CU]: input channel ci < CL = low channel, CL + (2a + b) CU + cs = skip channel cs of the
-// full-resolution pixel (2i + a, 2j + b); output column (2 py + px) CU + o = channel o of output pixel (2i + py, 2j + px).  For tap
-// (dy, dx) in {-1,0,1}^2 the conv taps (ky, kx) that contribute are those with floor((py + ky - 1) / 2) = dy (row parity a = (py + ky
-// - 1) - 2 dy), likewise for x.  bias9 [3][3][CU]: the ConvTranspose bias through the conv taps that stay inside the image, by border
-// kind (top, middle, bottom) x (left, middle, right) of the OUTPUT pixel.
-__global__ void dec_t5_fill_kernel(const float* __restrict__ ct_w, const float* __restrict__ ct_b, const float* __restrict__ w3,
-                                   float* __restrict__ Wp, float* __restrict__ bias9, int CL, int CU) {
-    const int K = 3 * CL, N = 4 * CU;
-    const long long total = 9LL * K * N;
-    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (idx < 9 * CU) {
-        const int o = (int)(idx % CU), kind = (int)(idx / CU), ry = kind / 3, rx = kind % 3;
-        float sacc = 0.f;
-        for (int ky = 0; ky < 3; ++ky) {
-            if ((ry == 0 && ky == 0) || (ry == 2 && ky == 2)) continue;
-            for (int kx = 0; kx < 3; ++kx) {
-                if ((rx == 0 && kx == 0) || (rx == 2 && kx == 2)) continue;
-                for (int co = 0; co < CU; ++co) sacc += w3[((ky * 3 + kx) * (2 * CU) + co) * CU + o] * ct_b[co];
-            }
-        }
-        bias9[idx] = sacc;
-    }
-    if (idx >= total) return;
-    const int n = (int)(idx % N), ci = (int)((idx / N) % K), tap = (int)(idx / ((long long)N * K));
-    const int dy = tap / 3 - 1, dx = tap % 3 - 1;
-    const int pos = n / CU, o = n - pos * CU, py = pos >> 1, px = pos & 1;
-    float v = 0.f;
-    for (int ky = 0; ky < 3; ++ky) {
-        const int ey = py + ky - 1, fy = ey < 0 ? -1 : ey >> 1, a = ey - 2 * fy;
-        if (fy != dy) continue;
-        for (int kx = 0; kx < 3; ++kx) {
-            const int ex = px + kx - 1, fx = ex < 0 ? -1 : ex >> 1, b = ex - 2 * fx;
-            if (fx != dx) continue;
-            if (ci < CL) {
-                for (int co = 0; co < CU; ++co)
-                    v += ct_w[((a * 2 + b) * CL + ci) * CU + co] * w3[((ky * 3 + kx) * (2 * CU) + co) * CU + o];
-            } else {
-                const int sc = ci - CL, par = sc / CU, cs = sc - par * CU;
-                if (par == a * 2 + b) v += w3[((ky * 3 + kx) * (2 * CU) + CU + cs) * CU + o];
-            }
-        }
-    }
-    Wp[idx] = v;
-}
-
-static bool dec_t5_covers(int cl, int cu) { return cl == 2 * cu && (cu == 16 || cu == 32 || cu == 64); }
-
 int dec_composite_bytes(int cl, int cu, size_t* bytes) {
     if (cl == DC_CL && cu == DC_CU) { *bytes = DC_BLOB_BYTES; return 0; }
-    if (dec_t5_covers(cl, cu)) {
-        size_t w = 0;
-        int rc = tc_conv3x3_bytes(3 * cl, 4 * cu, &w);
-        if (rc) return rc;
-        *bytes = (w + 15) / 16 * 16 + (size_t)9 * cu * 4;
-        return 0;
-    }
-    set_error("composite decoder packing: %d -> %d not covered ((16, 8), (32, 16), (64, 32), (128, 64))", cl, cu);
+    set_error("composite decoder packing: %d -> %d not covered (only (16, 8))", cl, cu);
     return 3;
 }
 
@@ -520,28 +465,9 @@ int pack_dec_composite(const float* ct_w, const float* ct_b, const float* conv_w
     int rc = dec_composite_bytes(cl, cu, &bytes);
     if (rc) return rc;
     if (dtype != DG_F16 && dtype != DG_BF16) { set_error("composite decoder packing needs a 16-bit dtype"); return 2; }
-    if (!(cl == DC_CL && cu == DC_CU)) {
-        // tcgen05 decoder mode: fp32 composite taps in a stream-ordered scratch, then the ordinary tensor-core weight packing
-        size_t wbytes = 0;
-        tc_conv3x3_bytes(3 * cl, 4 * cu, &wbytes);
-        const long long total = 9LL * 3 * cl * 4 * cu;
-        float* wp = nullptr;
-        if (cudaMallocAsync(reinterpret_cast<void**>(&wp), (size_t)total * 4, st) != cudaSuccess) {
-            set_error("composite decoder packing: scratch allocation failed");
-            return 4;
-        }
-        float* bias9 = reinterpret_cast<float*>(static_cast<unsigned char*>(out) + (wbytes + 15) / 16 * 16);
-        dec_t5_fill_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(ct_w, ct_b, conv_w, wp, bias9, cl, cu);
-        count_launch();
-        rc = check_launch("dec_t5_fill");
-        if (rc == 0) rc = pack_conv3x3_tc(wp, out, 3 * cl, 4 * cu, dtype, st);
-        cudaFreeAsync(wp, st);
-        return rc;
-    }
     const int threads = 16 * 2 * DC_CU * 8;
     if (dtype == DG_F16) pack_dec_composite_kernel<__half><<<(threads + 255) / 256, 256, 0, st>>>(ct_w, ct_b, conv_w, (unsigned char*)out);
-    else if (dtype == DG_BF16) pack_dec_composite_kernel<__nv_bfloat16><<<(threads + 255) / 256, 256, 0, st>>>(ct_w, ct_b, conv_w, (unsigned char*)out);
-    else { set_error("composite decoder packing needs a 16-bit dtype"); return 2; }
+    else pack_dec_composite_kernel<__nv_bfloat16><<<(threads + 255) / 256, 256, 0, st>>>(ct_w, ct_b, conv_w, (unsigned char*)out);
     count_launch();
     return check_launch("pack_dec_composite");
 }

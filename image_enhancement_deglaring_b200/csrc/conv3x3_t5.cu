@@ -31,21 +31,10 @@ namespace dg {
 
 namespace {
 
-enum { T5_SAME = 0, T5_POOL = 1, T5_CAT2 = 3, T5_CONVT = 4, T5_DEC = 5, T5_IDENT = 6 };   // T5_CONVT: ConvTranspose2d(2,2)+bias as a 1-tap GEMM with N = 4*C_up
+enum { T5_SAME = 0, T5_POOL = 1, T5_CAT2 = 3, T5_CONVT = 4, T5_IDENT = 6 };   // T5_CONVT: ConvTranspose2d(2,2)+bias as a 1-tap GEMM with N = 4*C_up
 // T5_IDENT: the conv DATA GRADIENT of the wide layers (dgrad = a 3x3 conv of dR with the taps-flipped, transposed weights): the one
 // source is an identity bf16 tensor (no GroupNorm, no SiLU: chunks are copied), the epilogue stores the fp32 accumulators as fp32
 // [N,H,W,cout] and keeps no statistics.
-// T5_DEC: ConvTranspose2d(2,2) + torch.cat + 3x3 conv (src/model.py:116-128 + :93) as ONE 3x3 conv on the LOW-resolution grid:
-//   input channels  = CL activated low channels + the activated skip tensor in space-to-depth form (4 parities x CU channels),
-//   output channels = 4 output-pixel parities x CU channels (scattered to the full-resolution tensor by the epilogue),
-//   weights         = the ConvTranspose folded into the conv taps (dec_t5 blob, conv3x3_dec.cu): per output parity 4 of the 9 low taps
-//                     and 9 of the 36 (tap, skip parity) pairs are non-zero.
-// 3.2x the useful MACs, but with N = 4 CU = 64..256 and K = 27 CL it is the shape the tensor pipe is good at: neither `up` nor the
-// concatenation exists anywhere, and the stand-alone ConvTranspose kernel and its HBM round trip disappear.
-// MEASURED (B200, batch 64, fp16; DESIGN.md section 3.1): correct everywhere, but not faster with this kernel's role split -- the
-// epilogue (bias + parity scatter + statistics, ~3.3k clk per 128 x 32 tile on 4 warps) and the stagers bound it, and at 128 -> 64
-// the 3.5 MB of composite weights are re-streamed from L2 for every 256 pixels: up2+dec2.0 0.229 -> 0.246-0.260 ms, up3+dec3.0
-// 0.170 -> 0.162-0.174 ms, up4+dec4.0 0.108 -> 0.222 ms.  Opt-in (path bit 11); the default keeps the un-fused / mma.sync decoders.
 constexpr int T5_STAGE_WARPS = 16;   // staging is dependent-chain bound per warp (measured ~0.1 IPC): it scales with warps, not with ILP
 constexpr int T5_STAGE_THREADS = 32 * T5_STAGE_WARPS;
 // Warp roles by warp id.  The warp scheduler prefers the HIGHEST warp id among eligible warps (B300_MICROARCH.md, "arbiter
@@ -78,12 +67,11 @@ struct T5Args {
     int na, nbs, ts;  // ring depths: A chunks, weight tiles, TMEM accumulator stages
     int a_stage_bytes, b_stage_bytes;
     int tmem_cols;
-    int off_b, off_coef, off_scr, off_bias, off_bar;
+    int off_b, off_coef, off_scr, off_bar;
     int ncoef;
     int ntaps;        // 9, or 1 (T5_CONVT: the centre tap only)
-    int cu;           // T5_CONVT / T5_DEC: channels of the full-resolution output (GEMM N = cout = 4 * cu)
-    int cl;           // T5_DEC: channels of the low-resolution source
-    const float* bias;   // T5_CONVT: [cu];  T5_DEC: [9 border kinds][cu] ConvTranspose bias seen through the valid conv taps
+    int cu;           // T5_CONVT: channels of the full-resolution output (GEMM N = cout = 4 * cu)
+    const float* bias;   // T5_CONVT: [cu]
     int items;
     long long* trace;   // DG_T5_TRACE=1: per-role clock64 timestamps of CTA 0 (debug aid, see t5_trace_dump)
 };
@@ -360,13 +348,6 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
         for (int c = 0; c < 4; ++c) s1[c][0] = s1[c][1] = s2[c][0] = s2[c][1] = 0.0;
         int stats_n = -1, stats_nbk = 0;
         const int ncc = p.nb >> 5;
-        const int cu_shift = MODE == T5_DEC ? __ffs(p.cu) - 1 : 0;
-        const float* sbias = reinterpret_cast<const float*>(smem + p.off_bias);
-        if constexpr (MODE == T5_DEC) {   // the 9 bias vectors live in shared memory: a global load would sit in every tile's chain
-            float* sb = reinterpret_cast<float*>(smem + p.off_bias);
-            for (int i = tid - 32 * T5_EPI_WARP0; i < 9 * p.cu; i += 128) sb[i] = __ldg(p.bias + i);
-            asm volatile("bar.sync 2, 128;" ::: "memory");
-        }
         auto flush = [&]() {
             if (stats_n < 0 || p.out_stats == nullptr) return;
 #pragma unroll
@@ -378,9 +359,7 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
                         const double b = s2[c][e] + __shfl_xor_sync(0xffffffffu, s2[c][e], 16);
                         if (half == 0) {
                             const int col = stats_nbk * p.nb + c * 32 + 2 * pr + e;
-                            // T5_DEC: column = parity * cu + channel -- the four parities of a channel land on the same sums
-                            double* d = MODE == T5_DEC ? p.out_stats + ((size_t)stats_n * p.cu + (col & (p.cu - 1))) * 2
-                                                       : p.out_stats + ((size_t)stats_n * p.cout + col) * 2;
+                            double* d = p.out_stats + ((size_t)stats_n * p.cout + col) * 2;
                             atomicAdd(d, a);
                             atomicAdd(d + 1, b);
                         }
@@ -431,9 +410,7 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
                                     of[j] = make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]),
                                                         __uint_as_float(r[4 * j + 3]));
                             }
-                            continue;
-                        }
-                        if constexpr (MODE == T5_CONVT) {
+                        } else if constexpr (MODE == T5_CONVT) {
                             // ConvTranspose2d(2,2): column n = pos * cu + co of low pixel (y, x) is channel co of output pixel
                             // (2y + pos/2, 2x + pos%2); + bias, no statistics (the consumer treats `up` as an identity source)
                             const int n0 = it.nbk * p.nb + c * 32;
@@ -452,34 +429,8 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
                                         pack2<T>(__uint_as_float(r[8 * j + 6]) + b1.z, __uint_as_float(r[8 * j + 7]) + b1.w));
                                 }
                             }
-                            continue;
-                        }
-                        uint32_t pk[16];
-                        if constexpr (MODE == T5_DEC) {
-                            // column n = parity * cu + co of low pixel (y, x) is channel co of output pixel (2y + parity / 2,
-                            // 2x + parity % 2); the ConvTranspose bias reaches it through the conv taps that lie inside the image:
-                            // one of 9 pre-summed bias vectors by border kind (top / middle / bottom) x (left / middle / right)
-                            const int n0 = it.nbk * p.nb + c * 32;
-#pragma unroll
-                            for (int j = 0; j < 4; ++j) {
-                                const int nn = n0 + 8 * j, pos = nn >> cu_shift, co = nn & (p.cu - 1);
-                                const int gy = 2 * y + (pos >> 1), gx = 2 * x + (pos & 1);
-                                const int kind = (gy == 0 ? 0 : (gy == 2 * p.H - 1 ? 2 : 1)) * 3 + (gx == 0 ? 0 : (gx == 2 * p.W - 1 ? 2 : 1));
-                                float4 b0 = make_float4(0.f, 0.f, 0.f, 0.f), b1 = b0;
-                                if (valid) {
-                                    const float4* bp = reinterpret_cast<const float4*>(sbias + kind * p.cu + co);
-                                    b0 = bp[0]; b1 = bp[1];
-                                }
-                                pk[4 * j] = valid ? pack2<T>(__uint_as_float(r[8 * j]) + b0.x, __uint_as_float(r[8 * j + 1]) + b0.y) : 0u;
-                                pk[4 * j + 1] = valid ? pack2<T>(__uint_as_float(r[8 * j + 2]) + b0.z, __uint_as_float(r[8 * j + 3]) + b0.w) : 0u;
-                                pk[4 * j + 2] = valid ? pack2<T>(__uint_as_float(r[8 * j + 4]) + b1.x, __uint_as_float(r[8 * j + 5]) + b1.y) : 0u;
-                                pk[4 * j + 3] = valid ? pack2<T>(__uint_as_float(r[8 * j + 6]) + b1.z, __uint_as_float(r[8 * j + 7]) + b1.w) : 0u;
-                                if (valid)
-                                    *reinterpret_cast<uint4*>(reinterpret_cast<T*>(p.out) +
-                                                              ((size_t)(it.n * 2 * p.H + gy) * (2 * p.W) + gx) * p.cu + co) =
-                                        make_uint4(pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
-                            }
                         } else {
+                            uint32_t pk[16];
 #pragma unroll
                             for (int j = 0; j < 16; ++j)
                                 pk[j] = valid ? pack2<T>(__uint_as_float(r[2 * j]), __uint_as_float(r[2 * j + 1])) : 0u;
@@ -488,23 +439,23 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
                                 for (int j = 0; j < 4; ++j)
                                     *reinterpret_cast<uint4*>(o + c * 32 + j * 8) = make_uint4(pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
                             }
-                        }
-                        // statistics of the STORED values: transpose through shared memory, lane = (pixel half, channel pair)
-                        __syncwarp();
+                            // statistics of the STORED values: transpose through shared memory, lane = (pixel half, channel pair)
+                            __syncwarp();
 #pragma unroll
-                        for (int j = 0; j < 4; ++j)
-                            *reinterpret_cast<uint4*>(scr + lane * T5_SCR_PITCH + j * 16) = make_uint4(pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
-                        __syncwarp();
-                        float a0 = 0.f, a1 = 0.f, q0 = 0.f, q1 = 0.f;
+                            for (int j = 0; j < 4; ++j)
+                                *reinterpret_cast<uint4*>(scr + lane * T5_SCR_PITCH + j * 16) = make_uint4(pk[4 * j], pk[4 * j + 1], pk[4 * j + 2], pk[4 * j + 3]);
+                            __syncwarp();
+                            float a0 = 0.f, a1 = 0.f, q0 = 0.f, q1 = 0.f;
 #pragma unroll
-                        for (int i = 0; i < 16; ++i) {
-                            const int row = half * 16 + ((i + 4 * half) & 15);   // the two halves hit disjoint banks
-                            const float2 v = unpack2<T>(*reinterpret_cast<const uint32_t*>(scr + row * T5_SCR_PITCH + pr * 4));
-                            a0 += v.x; q0 = fmaf(v.x, v.x, q0);
-                            a1 += v.y; q1 = fmaf(v.y, v.y, q1);
+                            for (int i = 0; i < 16; ++i) {
+                                const int row = half * 16 + ((i + 4 * half) & 15);   // the two halves hit disjoint banks
+                                const float2 v = unpack2<T>(*reinterpret_cast<const uint32_t*>(scr + row * T5_SCR_PITCH + pr * 4));
+                                a0 += v.x; q0 = fmaf(v.x, v.x, q0);
+                                a1 += v.y; q1 = fmaf(v.y, v.y, q1);
+                            }
+                            s1[c][0] += (double)a0; s2[c][0] += (double)q0;
+                            s1[c][1] += (double)a1; s2[c][1] += (double)q1;
                         }
-                        s1[c][0] += (double)a0; s2[c][0] += (double)q0;
-                        s1[c][1] += (double)a1; s2[c][1] += (double)q1;
                     }
                 }
             }
@@ -534,7 +485,7 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
         const uint32_t rowb = (uint32_t)Ws * Cs * 2;
         const int njobs = (it1 - it0) * p.nchunk;
 
-        struct Job { int n, apix, r0, c0, cs, xs; bool ident; const unsigned char* src; uint32_t rowb, pxb; };
+        struct Job { int n, apix, r0, c0, cs, xs; bool ident; const unsigned char* src; };
         auto job_of = [&](int j) {
             Job jb;
             const int item = it0 + j / p.nchunk, ch = j - (j / p.nchunk) * p.nchunk;
@@ -546,24 +497,6 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
             jb.r0 = q0 / p.pitch;
             jb.c0 = q0 - jb.r0 * p.pitch;
             const int cg = ch * p.kc + c8 * 8;                         // first of this thread's 8 input channels
-            jb.rowb = 0; jb.pxb = 0;
-            if constexpr (MODE == T5_DEC) {
-                jb.ident = false;
-                if (cg < p.cl) {                                       // low-resolution source, pixel (gy, gx)
-                    jb.cs = cg;                                        // coefficient index
-                    jb.pxb = (uint32_t)p.cl * 2;
-                    jb.rowb = (uint32_t)W * jb.pxb;
-                    jb.src = reinterpret_cast<const unsigned char*>(p.src0) + (size_t)it.n * H * jb.rowb + (size_t)cg * 2;
-                } else {                                               // skip source, pixel (2 gy + a, 2 gx + b) of parity (a, b)
-                    const int sc = cg - p.cl, par = sc / p.cu, cs = sc - par * p.cu;
-                    jb.cs = p.cl + cs;
-                    jb.pxb = (uint32_t)p.cu * 4;                       // two full-resolution pixels
-                    jb.rowb = (uint32_t)W * 2 * jb.pxb;                // two full-resolution rows
-                    jb.src = reinterpret_cast<const unsigned char*>(p.src1) + (size_t)it.n * H * jb.rowb +
-                             (size_t)((par >> 1) * (jb.rowb >> 1)) + (size_t)((par & 1) * (jb.pxb >> 1)) + (size_t)cs * 2;
-                }
-                return jb;
-            }
             jb.ident = (MODE == T5_CAT2 && cg < p.cout) || MODE == T5_IDENT;   // `up` half of the concat / a gradient tensor: plain copy
             jb.cs = (MODE == T5_CAT2 && !jb.ident) ? cg - p.cout : cg;
             jb.src = reinterpret_cast<const unsigned char*>((MODE == T5_CAT2 && !jb.ident) ? p.src1 : p.src0) +
@@ -593,8 +526,6 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
                         q.v[b][1] = __ldg(reinterpret_cast<const uint4*>(base + Cs * 2));
                         q.v[b][2] = __ldg(reinterpret_cast<const uint4*>(base + rowb));
                         q.v[b][3] = __ldg(reinterpret_cast<const uint4*>(base + rowb + Cs * 2));
-                    } else if constexpr (MODE == T5_DEC) {
-                        q.v[b][0] = __ldg(reinterpret_cast<const uint4*>(jb.src + ((size_t)gy * jb.rowb + (size_t)gx * jb.pxb)));
                     } else {
                         q.v[b][0] = __ldg(reinterpret_cast<const uint4*>(jb.src + ((size_t)gy * rowb + (size_t)gx * (Cs * 2))));
                     }
@@ -644,10 +575,7 @@ __global__ void __launch_bounds__(T5_THREADS, 1) conv3x3_t5_kernel(const __grid_
             const double plane = (double)Hs * Ws;
             for (int c = ts_; c < p.ncoef; c += T5_STAGE_THREADS) {
                 float a, b;
-                if (MODE == T5_DEC) {
-                    if (c < p.cl) gn_coef(p.st0, p.g0, p.b0, n, p.cl, p.groups0, c, plane, p.eps, a, b);
-                    else gn_coef(p.st1, p.g1, p.b1, n, p.cu, p.groups1, c - p.cl, 4.0 * plane, p.eps, a, b);
-                } else if (MODE == T5_CAT2) {
+                if (MODE == T5_CAT2) {
                     if (p.cf1) { a = __ldg(p.cf1 + (size_t)(n * p.ncoef + c) * 2); b = __ldg(p.cf1 + (size_t)(n * p.ncoef + c) * 2 + 1); }
                     else gn_coef(p.st1, p.g1, p.b1, n, p.ncoef, p.groups1, c, plane, p.eps, a, b);
                 } else {
@@ -719,13 +647,13 @@ bool t5_plan(T5Args& t, int mode, int ntaps = 0) {
     if (cout % t.nb || (t.nb != 32 && t.nb != 64 && t.nb != 128 && t.nb != 96)) return false;
     if (t.nb == 96) return false;   // keep N a power of two (TMEM stage arithmetic)
     t.nnb = cout / t.nb;
-    const int csrc = mode == T5_CAT2 ? cout : (mode == T5_DEC ? t.cl : cin);   // channels of one source tensor
+    const int csrc = mode == T5_CAT2 ? cout : cin;   // channels of one source tensor
     t.ntaps = ntaps ? ntaps : (mode == T5_CONVT ? 1 : 9);   // ntaps = 1 with T5_IDENT: a plain GEMM over pixels (centre tap)
     t.kc = csrc >= 64 ? 64 : csrc;
     if (t.kc != 16 && t.kc != 32 && t.kc != 64) return false;
     if (csrc % t.kc || cin % t.kc) return false;
     t.nchunk = cin / t.kc;
-    t.ncoef = mode == T5_DEC ? t.cl + t.cu : csrc;
+    t.ncoef = csrc;
     t.tw = t.W <= 128 ? t.W : 126;                 // pitch 128 for wide images; one strip = the whole width up to 128 columns
     t.nstrips = (t.W + t.tw - 1) / t.tw;
     t.pitch = t.tw + 2;
@@ -749,7 +677,7 @@ bool t5_plan(T5Args& t, int mode, int ntaps = 0) {
         t.plane_px = px;
         t.a_stage_bytes = nc8 * px * 16;
         t.b_stage_bytes = (t.kc / 16) * t.nb * 32;
-        const int fixed = t.ncoef * 8 + 4 * 32 * T5_SCR_PITCH + (mode == T5_DEC ? 9 * t.cu * 4 : 0) + 8 * (4 * T5_MAX_RING + 4) + 16 + 1024;
+        const int fixed = t.ncoef * 8 + 4 * 32 * T5_SCR_PITCH + 8 * (4 * T5_MAX_RING + 4) + 16 + 1024;
         // ring depths: at least 2 A chunks and 3 weight tiles, more while shared memory lasts
         int budget = 227 * 1024 - fixed;
         t.na = 2; t.nbs = 3;
@@ -772,8 +700,7 @@ bool t5_plan(T5Args& t, int mode, int ntaps = 0) {
     t.off_b = (t.na * t.a_stage_bytes + 127) / 128 * 128;
     t.off_coef = t.off_b + t.nbs * t.b_stage_bytes;
     t.off_scr = (t.off_coef + t.ncoef * 8 + 15) / 16 * 16;
-    t.off_bias = t.off_scr + 4 * 32 * T5_SCR_PITCH;
-    t.off_bar = t.off_bias + (mode == T5_DEC ? 9 * t.cu * 4 : 0);
+    t.off_bar = t.off_scr + 4 * 32 * T5_SCR_PITCH;
     const long long items = (long long)t.N * t.nstrips * t.bands_img * t.nnb;
     if (items > 0x7fffffffLL) return false;
     t.items = (int)items;
@@ -828,7 +755,6 @@ int dispatch_t5(const T5Args& t, int mode, cudaStream_t st) {
     if (mode == T5_SAME) return launch_t5<T, T5_SAME>(t, st);
     if (mode == T5_POOL) return launch_t5<T, T5_POOL>(t, st);
     if (mode == T5_CONVT) return launch_t5<T, T5_CONVT>(t, st);
-    if (mode == T5_DEC) return launch_t5<T, T5_DEC>(t, st);
     return launch_t5<T, T5_CAT2>(t, st);
 }
 }  // namespace
@@ -844,29 +770,11 @@ int conv3x3_t5_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* handl
     if (a.path & 128) return 0;
     if (a.dtype != DG_F16 && a.dtype != DG_BF16) return decline("needs 16-bit storage");
     const dg_src& s0 = a.src[0];
-    const bool dec = a.nsrc == 2 && s0.xform == DG_X_CONVT2 && a.src[1].xform == DG_X_SAME;
-    if ((!dec && a.weight_tc == nullptr) || a.act_sum != nullptr) return decline("needs the tensor-core weight packing and no act_sum");
+    if (a.weight_tc == nullptr || a.act_sum != nullptr) return decline("needs the tensor-core weight packing and no act_sum");
     T5Args t;
     memset(&t, 0, sizeof(t));
     int mode;
-    const void* wgt = a.weight_tc;
-    if (dec) {
-        // ConvTranspose + concat + conv as one low-resolution conv (T5_DEC); (16, 8) belongs to conv3x3_dec.cu's kernel
-        const dg_src& s1 = a.src[1];
-        const int cl = s0.channels, cu = a.cout;
-        if (a.weight_comp == nullptr || (a.path & 1024)) return decline("composite decoder weights missing / disabled");
-        if (cl != 2 * cu || s0.ct_cout != cu || s1.channels != cu || (cu != 16 && cu != 32 && cu != 64)) return decline("decoder channel set not covered");
-        if (s0.stats == nullptr || !s0.silu || s0.scale || s1.stats == nullptr || !s1.silu || s1.scale || s0.coef || s1.coef)
-            return decline("decoder sources must be GroupNorm + SiLU");
-        if ((a.H | a.W) & 1) return decline("odd output size");
-        size_t wbytes = 0;
-        if (tc_conv3x3_bytes(3 * cl, 4 * cu, &wbytes)) return decline("weight packing");
-        mode = T5_DEC;
-        t.cin = 3 * cl; t.cl = cl; t.cu = cu;
-        t.src1 = s1.raw; t.st1 = s1.stats; t.g1 = s1.gamma; t.b1 = s1.beta; t.groups1 = s1.groups;
-        wgt = a.weight_comp;
-        t.bias = reinterpret_cast<const float*>(static_cast<const unsigned char*>(a.weight_comp) + ((wbytes + 15) / 16) * 16);
-    } else if (a.nsrc == 1 && (s0.xform == DG_X_SAME || s0.xform == DG_X_POOL2)) {
+    if (a.nsrc == 1 && (s0.xform == DG_X_SAME || s0.xform == DG_X_POOL2)) {
         if (s0.stats == nullptr || !s0.silu || s0.scale != nullptr) return decline("source must be GroupNorm + SiLU");
         mode = s0.xform == DG_X_SAME ? T5_SAME : T5_POOL;
         t.cin = s0.channels;
@@ -881,18 +789,17 @@ int conv3x3_t5_launch(const dg_conv3x3_args& a, cudaStream_t stream, bool* handl
     } else {
         return decline("source combination not covered");
     }
-    if ((reinterpret_cast<uintptr_t>(s0.raw) | reinterpret_cast<uintptr_t>(a.out) | reinterpret_cast<uintptr_t>(wgt) |
+    if ((reinterpret_cast<uintptr_t>(s0.raw) | reinterpret_cast<uintptr_t>(a.out) | reinterpret_cast<uintptr_t>(a.weight_tc) |
          reinterpret_cast<uintptr_t>(t.src1)) & 15)
         return decline("pointers must be 16-byte aligned");
     t.src0 = s0.raw; t.st0 = s0.stats; t.g0 = s0.gamma; t.b0 = s0.beta; t.cf0 = s0.coef; t.groups0 = s0.groups;
-    t.wgt = wgt;
+    t.wgt = a.weight_tc;
     t.out = a.out; t.out_stats = a.out_stats;
     t.N = a.N; t.H = a.H; t.W = a.W; t.eps = a.eps;
     t.cout = a.cout;
-    if (mode == T5_DEC) { t.H = a.H / 2; t.W = a.W / 2; t.cout = 4 * a.cout; }   // the GEMM runs on the low-resolution grid
     // N = 32 with a single-source prologue: a UMMA re-reads its 4 KB A tile for only 32 output channels, and the mma.sync kernel
     // measured on par or faster (enc3.0 0.071 vs 0.100 ms, enc3.3 0.079 vs 0.083 ms at batch 64); the concat conv (K = 576) wins here
-    if (!forced && a.cout == 32 && mode != T5_CAT2 && mode != T5_DEC) return 0;
+    if (!forced && a.cout == 32 && mode != T5_CAT2) return 0;
     if (!t5_plan(t, mode)) return decline("shape does not fit the tcgen05 plan");
     *handled = true;
     return a.dtype == DG_F16 ? dispatch_t5<__half>(t, mode, stream) : dispatch_t5<__nv_bfloat16>(t, mode, stream);

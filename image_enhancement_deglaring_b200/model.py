@@ -153,13 +153,11 @@ class LightweightUNet(nn.Module):
                 w2t = ops.pack_convt2x2_tc(w2, ops.DG_BF16)
             pc.up_w_dgrad_tc_bf16[u] = None if w2t is None else w2t.data_ptr()
             keep.append(w2t)
-            # composite decoder taps (ConvTranspose folded into the consuming conv, conv3x3_dec.cu) where that kernel has coverage
-            # level 1 (16 -> 8): conv3x3_dec.cu's kernel, forward of both modes.  Levels 2-4 (32 -> 16, 64 -> 32, 128 -> 64) have the
-            # tcgen05 decoder mode of conv3x3_t5.cu (ConvTranspose + cat + conv as one low-resolution conv): correct but measured
-            # slower than the default kernels (DESIGN.md 3.1), so it is opt-in with path bit 11 (2048), inference only
+            # composite decoder taps (ConvTranspose folded into the consuming conv, conv3x3_dec.cu) where that kernel has coverage:
+            # level 1 (16 -> 8), forward of both modes
             comp = None
             cu_ = int(w.shape[3])
-            if self.path != 1 and pc.dtype != ops.DG_F32 and (cu_ == 8 or ((self.path & 2048) and not train)):
+            if self.path != 1 and pc.dtype != ops.DG_F32 and cu_ == 8:
                 dblk = getattr(self, _BLOCKS[5 + u])
                 comp = ops.pack_dec_composite(w, bt, ops.pack_conv3x3(dblk[0].weight), pc.dtype)
             pc.dec_comp[u] = None if comp is None else comp.data_ptr()

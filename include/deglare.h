@@ -95,9 +95,8 @@ typedef struct {
     int32_t path;         /* bits 0-1: 0 = auto, 1 = force generic CUDA-core path, 2 = force tensor-core path;
                              bit 7: do not use the tcgen05 kernel (conv3x3_t5.cu); bit 8: insist on it (tests);
                              bit 9 / bit 10: do not use the persistent TMA-fed 8 -> 8 kernel (conv3x3_ring.cu) / the composite
-                             decoder kernels (conv3x3_dec.cu, conv3x3_t5.cu decoder mode);
-                             bit 11 (module level): also pack the composite blobs of the 32 -> 16 ... 128 -> 64 decoders.
-                             Bits 2-6 are unused: a call that sets one fails with 2.                                        */
+                             decoder kernel (conv3x3_dec.cu).
+                             Bits 2-6 and 11 are unused: a call that sets one fails with 2.                                 */
     const void* weight_comp;  /* optional, decoder conv over (DG_X_CONVT2 low, DG_X_SAME skip) only: dg_pack_dec_composite blob --
                                  the ConvTranspose folded into the conv's taps (conv3x3_dec.cu); NULL = stage `up` in the CTA  */
 } dg_conv3x3_args;
@@ -243,8 +242,8 @@ typedef struct {
     int32_t path;                           /* dg_conv3x3_args.path: 0 auto, 1 generic, 2 tensor-core, ... */
     int32_t reserved;
     const void* dec_comp[4];                /* optional: dg_pack_dec_composite blobs of (upconv4..1, dec4..1 `.0`) for the
-                                               levels the composite decoder kernel covers (upconv1 + dec1.0 of the shipped
-                                               model); NULL elsewhere                                                  */
+                                               levels with (cl, cu) = (16, 8), the only pair it covers: of the shipped model
+                                               only the upconv1 slot [3] is used; NULL elsewhere                       */
     const void* conv_w_flip_tc_bf16[DG_MAX_BLOCKS][2]; /* backward only, optional: dg_pack_conv3x3_tc(conv_w_flip, DG_BF16) -- the
                                                taps-flipped weights in the tensor-core packing: the data gradient of the layers the
                                                mma.sync dgrad does not cover (wider variants, configs[4]) runs as a tcgen05 conv  */
@@ -403,10 +402,8 @@ int dg_pack_convt2x2_tc(const float* w, void* out, int32_t cin, int32_t cout, in
 
 /* Composite decoder taps (conv3x3_dec.cu): ConvTranspose2d(k=2, s=2)+bias folded into the 3x3 conv that consumes cat((up, skip)).
  * ct_w fp32 [2][2][cl][cu], ct_b [cu], conv_w fp32 [3][3][2 cu][cu] (the packings dg_conv3x3_fused takes); out = blob of
- * *bytes bytes in `dtype`.  Covers (cl, cu) = (16, 8) -- upconv1 + dec1.0 of LightweightUNet(features_start=8), src/model.py:53,54 --
- * for the kernel of conv3x3_dec.cu, and (32, 16), (64, 32), (128, 64) for the tcgen05 decoder mode of conv3x3_t5.cu (the three
- * layers as ONE 3x3 conv on the low-resolution grid: fp32 [3][3][3 cl][4 cu] composite taps in the tensor-core packing followed by
- * the 9 border-kind bias vectors [9][cu]); dg_conv3x3_fused uses whichever blob `weight_comp` holds for the channel set. */
+ * *bytes bytes in `dtype` (16-bit only).  Covers only (cl, cu) = (16, 8) -- upconv1 + dec1.0 of LightweightUNet(features_start=8),
+ * src/model.py:53,54; any other pair fails with 3. */
 int dg_dec_composite_bytes(int32_t cl, int32_t cu, size_t* bytes);
 int dg_pack_dec_composite(const float* ct_w, const float* ct_b, const float* conv_w, void* out, int32_t cl, int32_t cu,
                           int32_t dtype, dg_stream_t stream);

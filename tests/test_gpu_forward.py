@@ -58,24 +58,6 @@ def test_png_golden_16bit(best_sd, golden, storage, tol, min_psnr):
         assert p >= min_psnr
 
 
-def test_png_golden_fp16_with_the_tcgen05_decoder_mode(best_sd, golden):
-    """path bit 11: upconv + cat + dec*.0 of levels 2-4 as one low-resolution tcgen05 conv each (conv3x3_t5.cu T5_DEC, opt-in): the
-    whole network stays inside the 16-bit tier's bound and within rounding of the default kernels."""
-    g = golden("lw_png.npz")
-    net = _net(best_sd, storage="fp16", path=2048)
-    ref = _net(best_sd, storage="fp16")
-    for i in (1, 2):
-        x = torch.from_numpy(g[f"x{i}_u8"].astype(np.float32) / 255.0)[None, None].cuda()
-        with torch.no_grad():
-            y = net(x)[0, 0].cpu().numpy()
-            y0 = ref(x)[0, 0].cpu().numpy()
-        assert np.abs(y - g[f"y{i}"]).max() <= 5e-3 and psnr(y, g[f"y{i}"]) >= 50.0
-        assert np.abs(y - y0).max() <= 3e-3 and not np.array_equal(y, y0)      # a different kernel chain, same function
-    x = _rand((5, 1, 64, 96), 3).cuda()                                          # batch, non-square, two-stream split off
-    with torch.no_grad():
-        assert float((net(x) - ref(x)).abs().max()) <= 3e-3
-
-
 def test_random_golden_and_layer_taps(best_sd, golden):
     g = golden("lw_rand.npz")
     net = _net(best_sd)

@@ -535,48 +535,6 @@ def test_composite_decoder_kernel(dtype, N, H, W):
     assert not torch.equal(o_c, o_h) or H * W <= 4      # really two different kernels
 
 
-@pytest.mark.parametrize("dtype", TC_DTYPES)
-@pytest.mark.parametrize("c,N,H,W", [(16, 2, 64, 128), (16, 3, 48, 80), (16, 1, 256, 256), (16, 2, 16, 16), (32, 2, 64, 64), (32, 3, 34, 66),
-                                      (32, 1, 128, 128), (64, 2, 32, 32), (64, 3, 16, 48), (64, 1, 64, 64), (16, 1, 2, 2), (16, 1, 32, 520)])
-def test_t5_decoder_mode(dtype, c, N, H, W):
-    """ConvTranspose2d(2,2) + cat + 3x3 conv as ONE low-resolution tcgen05 conv (conv3x3_t5.cu T5_DEC: low channels + the skip tensor
-    in space-to-depth form -> 4 output parities x C channels, composite weights from dg_pack_dec_composite) vs the oracle's
-    ConvTranspose -> cat -> conv (src/model.py:116-128, :93) and vs the un-fused kernels (path bit 10)."""
-    rs = _rs(31 + c)
-    low = torch.from_numpy((rs.standard_normal((N, 2 * c, H // 2, W // 2)) * 2).astype(np.float32))
-    skip = torch.from_numpy((rs.standard_normal((N, c, H, W)) * 2 + 0.3).astype(np.float32))
-    ql, seen_l = _nhwc(low, dtype)
-    qs, seen_s = _nhwc(skip, dtype)
-    g1, b1 = _gn_params(rs, 2 * c)
-    g2, b2 = _gn_params(rs, c)
-    ctw = torch.from_numpy((rs.standard_normal((2 * c, c, 2, 2)) * (1.0 / np.sqrt(2 * c))).astype(np.float32))
-    ctb = torch.from_numpy((rs.standard_normal(c) * 0.5).astype(np.float32))     # a bias large enough to expose border mistakes
-    w = torch.from_numpy((rs.standard_normal((c, 2 * c, 3, 3)) * (1.0 / np.sqrt(18 * c))).astype(np.float32))
-    wp = ops.pack_conv3x3(w.cuda())
-    ctp = ops.pack_convt2x2(ctw.cuda())
-    s0 = ops.make_src(ql, 2 * c, xform=ops.DG_X_CONVT2, stats=_stats(seen_l), gamma=g1.cuda(), beta=b1.cuda(),
-                      groups=8, ct_w=ctp, ct_b=ctb.cuda(), ct_cout=c, ct_w_tc=ops.pack_convt2x2_tc(ctp, dtype))
-    s1 = ops.make_src(qs, c, stats=_stats(seen_s), gamma=g2.cuda(), beta=b2.cuda(), groups=8)
-    comp = ops.pack_dec_composite(ctp, ctb.cuda(), wp, dtype)
-    assert comp is not None
-    wtc = ops.pack_conv3x3_tc(wp, dtype)
-    o_c, s_c = ops.conv3x3_fused([s0, s1], wp, c, N, H, W, dtype, path=2 | 256, weight_tc=wtc, weight_comp=comp)   # 256: must be t5
-    torch.cuda.synchronize()
-    up = F.conv_transpose2d(tpo.gn_silu(seen_l, 8, g1, b1), ctw, ctb, stride=2)
-    ref = F.conv2d(torch.cat((up, tpo.gn_silu(seen_s, 8, g2, b2)), 1), w, None, 1, 1)
-    scale = max(1.0, float(ref.abs().max()))
-    tol = (6e-3 if dtype == ops.DG_F16 else 4e-2) * scale
-    got = o_c.float().cpu().permute(0, 3, 1, 2)
-    err = (got - ref).abs()
-    assert float(err.max()) <= tol, f"t5 decoder vs oracle {float(err.max()):.3e} at {np.unravel_index(int(err.argmax()), err.shape)} (scale {scale:.2f})"
-    want = torch.stack((got.double().sum(dim=(2, 3)), (got.double() ** 2).sum(dim=(2, 3))), dim=2)
-    assert float((s_c.cpu() - want).abs().max() / max(1.0, float(want.abs().max()))) <= (6e-4 if H * W >= 1024 else 5e-3)
-    if c == 16 and H * W >= 256:   # the round-1 fused mma.sync kernel on the same operands
-        o_h, _ = ops.conv3x3_fused([s0, s1], wp, c, N, H, W, dtype, path=2 | 1024, weight_tc=wtc, weight_comp=comp)
-        assert float((o_c.float() - o_h.float()).abs().max()) <= tol
-        assert not torch.equal(o_c, o_h)
-
-
 DGRAD_CASES = [(8, 8), (8, 16), (16, 16), (16, 32), (32, 32), (32, 64), (64, 64), (64, 128), (128, 128), (128, 64), (64, 32), (32, 16), (16, 8)]
 
 

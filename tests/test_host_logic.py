@@ -53,35 +53,46 @@ from image_enhancement_deglaring_b200 import _lib
 lib = _lib.load()
 buf = (C.c_float * 4096)()   # placeholder for every pointer: none may be dereferenced
 res = {}
-for path in (4, 8, 16, 32, 64, 0, 2 | 128):
+for path in (4, 8, 16, 32, 64, 2048, 0, 2 | 128):
     p = _lib.DgLwParams()
     p.in_channels, p.out_channels, p.features_start, p.dtype, p.path = 1, 1, 8, _lib.DG_F16, path
     rc = lib.dg_lw_workspace_bytes(C.byref(p), 1, 16, 16, C.byref(C.c_size_t(0)))
     res[path] = [rc, lib.dg_last_error_string().decode()]
-    if path & 0x7c:
+    if path & 0x87c:
         a = _lib.DgConv3x3Args()
         a.nsrc, a.dtype, a.N, a.H, a.W, a.cout, a.eps, a.path = 1, _lib.DG_F16, 1, 16, 16, 8, 1e-5, path
         a.weight = a.out = a.out_stats = C.addressof(buf)
         a.src[0].raw, a.src[0].channels, a.src[0].groups, a.src[0].xform = C.addressof(buf), 8, 1, _lib.DG_X_SAME
         res[path] += [lib.dg_conv3x3_fused(C.byref(a), None), lib.dg_last_error_string().decode()]
-print(json.dumps(res))
+comp = {}
+for cl, cu in ((16, 8), (32, 16), (64, 32), (128, 64)):
+    n = C.c_size_t(0)
+    rc = lib.dg_dec_composite_bytes(cl, cu, C.byref(n))
+    comp[f"{cl},{cu}"] = [rc, n.value, lib.dg_last_error_string().decode() if rc else ""]
+print(json.dumps({"path": res, "comp": comp}))
 """
 
 
 def test_removed_path_bits_are_rejected():
-    """Path bits 2-6 no longer select anything: dg_conv3x3_fused and the dg_lw_* planner return 2 and name the bit, before any
-    CUDA call -- run in a process that sees no CUDA device, where a call that reached the runtime would fail differently."""
+    """Path bits 2-6 and 11 no longer select anything: dg_conv3x3_fused and the dg_lw_* planner return 2 and name the bit, before
+    any CUDA call -- run in a process that sees no CUDA device, where a call that reached the runtime would fail differently.  With
+    bit 11 went the tcgen05 decoder mode's composite packing: dg_dec_composite_bytes covers (16, 8) only."""
     import json
     import subprocess
     out = subprocess.run([sys.executable, "-c", _REMOVED_PATH_BITS_PROBE], cwd=ROOT, env={**os.environ, "CUDA_VISIBLE_DEVICES": ""},
                          capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr[-500:]
-    res = {int(k): v for k, v in json.loads(out.stdout.splitlines()[-1]).items()}
-    for bit in range(2, 7):
+    probe = json.loads(out.stdout.splitlines()[-1])
+    res = {int(k): v for k, v in probe["path"].items()}
+    for bit in (2, 3, 4, 5, 6, 11):
         ws_rc, ws_err, conv_rc, conv_err = res[1 << bit]
         assert conv_rc == 2 and f"path {1 << bit} sets bit {bit}," in conv_err, (bit, conv_rc, conv_err)
         assert ws_rc == 2 and f"path {1 << bit} sets bit {bit}," in ws_err, (bit, ws_rc, ws_err)
     assert res[0][0] == 0 and res[2 | 128][0] == 0, res   # the surviving bits still plan a workspace
+    comp = probe["comp"]
+    assert comp["16,8"][0] == 0 and comp["16,8"][1] > 0, comp
+    for pair in ("32,16", "64,32", "128,64"):
+        assert comp[pair][0] == 3 and "(16, 8)" in comp[pair][2], (pair, comp[pair])
 
 
 def test_module_surface_matches_reference_contract(best_sd, golden):
