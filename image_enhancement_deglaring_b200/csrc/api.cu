@@ -78,12 +78,30 @@ static int validate_src(const dg_src& s, const char* who) {
 }
 
 // ---- LightweightUNet plan -----------------------------------------------------------------
+constexpr float kGnEps = 1e-5f;   // every GroupNorm of the reference module (nn.GroupNorm's default)
+
+// Kernel tiers of the orchestrator: path & 3 == 1 keeps every op on the CUDA-core kernels; the tensor-core choices made here
+// (materialised ConvTranspose, bf16 backward) also need 16-bit storage.
+static inline bool generic_only(const dg_lw_params* p) { return (p->path & 3) == 1; }
+static inline bool tc16(const dg_lw_params* p) { return p->dtype != DG_F32 && !generic_only(p); }
+
 struct LwPlan {
     int f[5];
     int conv_c[18], conv_h[18], conv_w[18];
+    int conv_cin[18];   // input channels: the image, the previous conv, the level above (pooled) or cat(up, skip)
+    size_t esz;         // bytes per stored activation element
     size_t raw_off[18], stats_off[18];
     size_t up_off[4];  // scratch for a materialised upconvK output (deep decoder levels, 16-bit storage)
     size_t stats_bytes, total_bytes;  // stats_bytes = the zero-initialised prefix (statistics)
+
+    // workspace slices from image n0 on (every per-image tensor is contiguous over the batch): conv i's output before its
+    // GroupNorm, that GroupNorm's statistics, and upconv u's materialised output
+    char* raw(char* ws, int i, int n0) const { return ws + raw_off[i] + (size_t)n0 * conv_h[i] * conv_w[i] * conv_c[i] * esz; }
+    double* stats(char* ws, int i, int n0) const { return reinterpret_cast<double*>(ws + stats_off[i]) + (size_t)n0 * conv_c[i] * 2; }
+    char* up(char* ws, int u, int n0) const {
+        const int i = 2 * (u + 5);   // the decoder conv consuming it
+        return ws + up_off[u] + (size_t)n0 * conv_h[i] * conv_w[i] * f[3 - u] * esz;
+    }
 };
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
@@ -101,10 +119,12 @@ static int make_plan(const dg_lw_params* p, int N, int H, int W, LwPlan* pl) {
     if (p->dtype < DG_F32 || p->dtype > DG_BF16) { set_error("bad dtype %d", p->dtype); return 2; }
     if (p->features_start < 1 || p->in_channels < 1 || p->out_channels < 1) { set_error("bad channel configuration"); return 2; }
     for (int l = 0; l < 5; ++l) pl->f[l] = p->features_start << l;
+    pl->esz = dtype_size(p->dtype);
     size_t off = 0;
     for (int i = 0; i < 18; ++i) {
-        const int lvl = block_level(i / 2);
+        const int b = i / 2, lvl = block_level(b);
         pl->conv_c[i] = pl->f[lvl];
+        pl->conv_cin[i] = i == 0 ? p->in_channels : (i % 2 ? pl->f[lvl] : (b < 5 ? pl->f[lvl - 1] : 2 * pl->f[lvl]));
         pl->conv_h[i] = H >> lvl;
         pl->conv_w[i] = W >> lvl;
         pl->stats_off[i] = off;
@@ -114,13 +134,13 @@ static int make_plan(const dg_lw_params* p, int N, int H, int W, LwPlan* pl) {
     off = align_up(off, 256);
     for (int i = 0; i < 18; ++i) {
         pl->raw_off[i] = off;
-        off += align_up((size_t)N * pl->conv_h[i] * pl->conv_w[i] * pl->conv_c[i] * dtype_size(p->dtype), 256);
+        off += align_up((size_t)N * pl->conv_h[i] * pl->conv_w[i] * pl->conv_c[i] * pl->esz, 256);
     }
     for (int u = 0; u < 4; ++u) {
         const int lvl = 3 - u;
         pl->up_off[u] = off;
         if (p->dtype != DG_F32)   // all four: inference materialises the deep ones, the tensor-core wgrad wants every `up`
-            off += align_up((size_t)N * (H >> lvl) * (W >> lvl) * pl->f[lvl] * dtype_size(p->dtype), 256);
+            off += align_up((size_t)N * (H >> lvl) * (W >> lvl) * pl->f[lvl] * pl->esz, 256);
     }
     pl->total_bytes = off;
     return 0;
@@ -131,14 +151,13 @@ static int make_plan(const dg_lw_params* p, int N, int H, int W, LwPlan* pl) {
 // wide variant (features_start = 64).  The concat itself is never stored.
 static inline bool lw_up_materialised(const LwPlan& pl, int u) { return pl.f[3 - u] >= 32; }
 
-// n0: first image of the sub-batch the descriptor is for (every per-image tensor is contiguous over the batch)
-static dg_src gn_src(const dg_lw_params* p, const LwPlan& pl, char* ws, int conv_idx, int xform, int n0 = 0) {
+// conv conv_idx's output through its GroupNorm + SiLU, images from n0 on
+static dg_src gn_src(const dg_lw_params* p, const LwPlan& pl, char* ws, int conv_idx, int xform, int n0) {
     dg_src s;
     memset(&s, 0, sizeof(s));
     const int b = conv_idx / 2, j = conv_idx % 2;
-    const size_t img = (size_t)pl.conv_h[conv_idx] * pl.conv_w[conv_idx] * pl.conv_c[conv_idx] * dtype_size(p->dtype);
-    s.raw = ws + pl.raw_off[conv_idx] + (size_t)n0 * img;
-    s.stats = reinterpret_cast<const double*>(ws + pl.stats_off[conv_idx]) + (size_t)n0 * pl.conv_c[conv_idx] * 2;
+    s.raw = pl.raw(ws, conv_idx, n0);
+    s.stats = pl.stats(ws, conv_idx, n0);
     s.gamma = p->gn_w[b][j];
     s.beta = p->gn_b[b][j];
     s.channels = pl.conv_c[conv_idx];
@@ -148,64 +167,75 @@ static dg_src gn_src(const dg_lw_params* p, const LwPlan& pl, char* ws, int conv
     return s;
 }
 
+// a tensor read as it is stored: no GroupNorm, no SiLU
+static dg_src ident_src(const void* raw, int channels, int xform = DG_X_SAME) {
+    dg_src s;
+    memset(&s, 0, sizeof(s));
+    s.raw = raw;
+    s.channels = channels;
+    s.groups = 1;
+    s.xform = xform;
+    return s;
+}
+
+// upconv u's output, materialised in the workspace by the stand-alone tensor-core kernel (convt_tc.cu), as the first source of
+// the decoder conv consuming it in place of the fused DG_X_CONVT2 source
+static dg_src up_src(const LwPlan& pl, char* ws, int u, int n0) { return ident_src(pl.up(ws, u, n0), pl.f[3 - u]); }
+
+// Conv i's arguments for images [n0, n0 + nn).  The forward launches them; the backward computes the weight gradient from the
+// same sources.  x = the whole batch's input image, uint8 when x_u8.
+static dg_conv3x3_args conv_args(const dg_lw_params* p, const LwPlan& pl, char* ws, const void* x, bool x_u8, int n0, int nn, int i) {
+    const int b = i / 2;
+    dg_conv3x3_args a;
+    memset(&a, 0, sizeof(a));
+    a.dtype = p->dtype;
+    a.N = nn; a.H = pl.conv_h[i]; a.W = pl.conv_w[i];
+    a.cout = pl.conv_c[i];
+    a.weight = p->conv_w[b][i % 2];
+    a.weight_tc = p->conv_w_tc[b][i % 2];
+    a.out = pl.raw(ws, i, n0);
+    a.out_stats = pl.stats(ws, i, n0);
+    a.eps = kGnEps;
+    a.path = p->path;
+    a.nsrc = 1;
+    if (i == 0) {
+        const size_t img = (size_t)p->in_channels * a.H * a.W * (x_u8 ? 1 : sizeof(float));
+        a.src[0] = ident_src(static_cast<const char*>(x) + n0 * img, p->in_channels, x_u8 ? DG_X_IMAGE_U8 : DG_X_IMAGE);
+    } else if (i % 2 == 1) {
+        a.src[0] = gn_src(p, pl, ws, i - 1, DG_X_SAME, n0);
+    } else if (b < 5) {
+        a.src[0] = gn_src(p, pl, ws, i - 1, DG_X_POOL2, n0);        // pool1..4, src/model.py:107-112
+    } else {
+        const int lvl = block_level(b), u = b - 5;
+        a.src[0] = gn_src(p, pl, ws, i - 1, DG_X_CONVT2, n0);      // upconv4..1, src/model.py:115-127
+        a.src[0].ct_w = p->up_w[u];
+        a.src[0].ct_b = p->up_b[u];
+        a.src[0].ct_w_tc = p->up_w_tc[u];
+        a.src[0].ct_cout = pl.f[lvl];
+        a.src[1] = gn_src(p, pl, ws, 2 * lvl + 1, DG_X_SAME, n0);  // skip: torch.cat((up, skip), 1)
+        a.nsrc = 2;
+        a.weight_comp = p->dec_comp[u];   // read by the forward's composite-tap kernel only (conv3x3_dec.cu)
+    }
+    return a;
+}
+
 // One forward over images [n0, n0 + nn) of a batch whose workspace was laid out for the whole batch (make_plan), on `stream`.
 // io: bit 0 = x is uint8 (normalised by 1/255 on load), bit 1 = y is uint8 (clip + quantise in the head)
 static int lw_forward_range(const dg_lw_params* p, const LwPlan& pl, char* ws, const void* x, void* y, int n0, int nn, int H, int W,
                             const float* target, double* l1_sum, cudaStream_t stream, cudaEvent_t* evs, int io) {
     int rc = 0;
-    const size_t esz = dtype_size(p->dtype);
     if (evs) cudaEventRecord(evs[0], stream);
     for (int i = 0; i < 18; ++i) {
-        const int b = i / 2;
         NvtxRange range(kConvNames[i]);
-        dg_conv3x3_args a;
-        memset(&a, 0, sizeof(a));
-        a.dtype = p->dtype;
-        a.N = nn; a.H = pl.conv_h[i]; a.W = pl.conv_w[i];
-        a.cout = pl.conv_c[i];
-        a.weight = p->conv_w[b][i % 2];
-        a.weight_tc = p->conv_w_tc[b][i % 2];
-        a.out = ws + pl.raw_off[i] + (size_t)n0 * a.H * a.W * a.cout * esz;
-        a.out_stats = reinterpret_cast<double*>(ws + pl.stats_off[i]) + (size_t)n0 * a.cout * 2;
-        a.eps = 1e-5f;
-        a.path = p->path;
-        a.nsrc = 1;
-        if (i == 0) {
-            memset(&a.src[0], 0, sizeof(dg_src));
-            a.src[0].raw = static_cast<const char*>(x) + (size_t)n0 * p->in_channels * H * W * ((io & 1) ? 1 : sizeof(float));
-            a.src[0].channels = p->in_channels;
-            a.src[0].groups = 1;
-            a.src[0].xform = (io & 1) ? DG_X_IMAGE_U8 : DG_X_IMAGE;
-        } else if (i % 2 == 1) {
-            a.src[0] = gn_src(p, pl, ws, i - 1, DG_X_SAME, n0);
-        } else if (b < 5) {
-            a.src[0] = gn_src(p, pl, ws, i - 1, DG_X_POOL2, n0);        // pool1..4, src/model.py:107-112
-        } else {
-            const int lvl = block_level(b), u = b - 5;
-            a.src[0] = gn_src(p, pl, ws, i - 1, DG_X_CONVT2, n0);      // upconv4..1, src/model.py:115-127
-            a.src[0].ct_w = p->up_w[u];
-            a.src[0].ct_b = p->up_b[u];
-            a.src[0].ct_w_tc = p->up_w_tc[u];
-            a.src[0].ct_cout = pl.f[lvl];
-            a.src[1] = gn_src(p, pl, ws, 2 * lvl + 1, DG_X_SAME, n0);  // skip: torch.cat((up, skip), 1)
-            a.nsrc = 2;
-            a.weight_comp = p->dec_comp[u];
-            // deep levels (upconv4, upconv3): run the transposed conv as its own tensor-core GEMM and
-            // feed its output as an identity source -- see convt_tc.cu for why this beats fusing there
-            const bool unfuse = p->dtype != DG_F32 && (p->path & 3) != 1 && lw_up_materialised(pl, u);
-            if (unfuse) {
-                bool handled = false;
-                void* up = ws + pl.up_off[u] + (size_t)n0 * a.H * a.W * pl.f[lvl] * esz;
-                rc = convt_tc_launch(a.src[0], p->dtype, nn, a.H, a.W, up, 1e-5f, p->path, stream, &handled);
-                if (rc) return rc;
-                if (handled) {
-                    memset(&a.src[0], 0, sizeof(dg_src));
-                    a.src[0].raw = up;
-                    a.src[0].channels = pl.f[lvl];
-                    a.src[0].groups = 1;
-                    a.src[0].xform = DG_X_SAME;
-                }
-            }
+        dg_conv3x3_args a = conv_args(p, pl, ws, x, io & 1, n0, nn, i);
+        const int u = i / 2 - 5;
+        // deep levels (upconv4, upconv3): run the transposed conv as its own tensor-core GEMM and
+        // feed its output as an identity source -- see convt_tc.cu for why this beats fusing there
+        if (a.nsrc == 2 && tc16(p) && lw_up_materialised(pl, u)) {
+            bool handled = false;
+            rc = convt_tc_launch(a.src[0], p->dtype, nn, a.H, a.W, pl.up(ws, u, n0), kGnEps, p->path, stream, &handled);
+            if (rc) return rc;
+            if (handled) a.src[0] = up_src(pl, ws, u, n0);
         }
         rc = dg_conv3x3_fused(&a, reinterpret_cast<dg_stream_t>(stream));
         if (rc) return rc;
@@ -224,7 +254,7 @@ static int lw_forward_range(const dg_lw_params* p, const LwPlan& pl, char* ws, c
     h.out = static_cast<char*>(y) + (size_t)n0 * out_img * ((io & 2) ? 1 : sizeof(float));
     h.target = target ? target + (size_t)n0 * out_img : nullptr;
     h.l1_sum = l1_sum;
-    h.eps = 1e-5f;
+    h.eps = kGnEps;
     h.out_kind = (io & 2) ? 1 : 0;
     rc = dg_head1x1(&h, reinterpret_cast<dg_stream_t>(stream));
     if (evs) cudaEventRecord(evs[19], stream);
@@ -248,7 +278,7 @@ struct FwdFork {
 static FwdFork g_forks[5];
 static std::atomic<int> g_split{16};   // minimum batch for the two-stream split; 0 disables (dg_set_batch_split)
 
-static int fork_init(int slot = 0) {
+static int fork_init(int slot) {
     FwdFork& g_fork = g_forks[slot];
     int dev = 0;
     cudaGetDevice(&dev);
@@ -260,6 +290,25 @@ static int fork_init(int slot = 0) {
     if (e != cudaSuccess) { set_error("forward fork streams: %s", cudaGetErrorString(e)); return 10; }
     g_fork.ready = true;
     g_fork.device = dev;
+    return 0;
+}
+
+// range(n0, nn, stream) over the whole batch on st or, from g_split images on, over its two halves on the fork streams of `slot`
+template <class Range>
+static int run_halves(cudaStream_t st, int slot, int N, Range&& range) {
+    const int split = g_split.load();
+    if (split <= 0 || N < split || N < 2) return range(0, N, st);
+    if (int rc = fork_init(slot)) return rc;
+    FwdFork& F = g_forks[slot];
+    cudaEventRecord(F.fork, st);
+    const int half = N / 2;
+    for (int k = 0; k < 2; ++k) {
+        cudaStreamWaitEvent(F.s[k], F.fork, 0);
+        const int rc = range(k ? half : 0, k ? N - half : half, F.s[k]);
+        cudaEventRecord(F.join[k], F.s[k]);
+        cudaStreamWaitEvent(st, F.join[k], 0);   // joined even on error, so the caller's stream stays ordered
+        if (rc) return rc;
+    }
     return 0;
 }
 
@@ -277,22 +326,10 @@ static int lw_forward(const dg_lw_params* p, const void* x, void* y, int N, int 
     char* ws = static_cast<char*>(workspace);
     cudaError_t e = cudaMemsetAsync(ws, 0, pl.stats_bytes, stream);
     if (e != cudaSuccess) { set_error("memset: %s", cudaGetErrorString(e)); return 10; }
-    const int split = g_split.load();
-    if (evs == nullptr && split > 0 && N >= split && N >= 2) {
-        if ((rc = fork_init(fork_slot))) return rc;
-        FwdFork& F = g_forks[fork_slot];
-        cudaEventRecord(F.fork, stream);
-        const int half = N / 2;
-        for (int k = 0; k < 2; ++k) {
-            cudaStreamWaitEvent(F.s[k], F.fork, 0);
-            rc = lw_forward_range(p, pl, ws, x, y, k ? half : 0, k ? N - half : half, H, W, target, l1_sum, F.s[k], nullptr, io);
-            cudaEventRecord(F.join[k], F.s[k]);
-            cudaStreamWaitEvent(stream, F.join[k], 0);   // joined even on error, so the caller's stream stays ordered
-            if (rc) return rc;
-        }
-        return 0;
-    }
-    return lw_forward_range(p, pl, ws, x, y, 0, N, H, W, target, l1_sum, stream, evs, io);
+    auto range = [&](int n0, int nn, cudaStream_t s) {
+        return lw_forward_range(p, pl, ws, x, y, n0, nn, H, W, target, l1_sum, s, evs, io);
+    };
+    return evs ? range(0, N, stream) : run_halves(stream, fork_slot, N, range);   // per-conv events time one stream
 }
 
 // ---- LightweightUNet backward ------------------------------------------------------------------
@@ -313,10 +350,8 @@ static void make_grad_layout(const dg_lw_params* p, const LwPlan& pl, GradLayout
     int k = 0;
     auto add = [&](size_t count, int pos) { g->off[k] = off; g->pos[k] = pos; off += count; return k++; };
     auto block = [&](int b) {
-        const int lvl = block_level(b);
-        const int c = pl.f[lvl];
-        const int cin0 = b == 0 ? p->in_channels : (b < 5 ? pl.f[lvl - 1] : 2 * c);
-        g->conv_w[b][0] = add((size_t)c * cin0 * 9, 4 * b);
+        const int c = pl.f[block_level(b)];
+        g->conv_w[b][0] = add((size_t)c * pl.conv_cin[2 * b] * 9, 4 * b);
         g->gn_w[b][0] = add(c, 4 * b);
         g->gn_b[b][0] = add(c, 4 * b);
         g->conv_w[b][1] = add((size_t)c * c * 9, 4 * b + 2);
@@ -346,7 +381,7 @@ struct BwdRequest {
 
 struct BwdPlan {
     size_t p_off[18], g_off[18], t_off[18], gb_off[18], low_off[4], coef_off, p_bytes, total;   // gb: dR as bf16 (16-bit tiers)
-    int cin_tot[18], maxc;
+    int maxc;
 };
 
 static void make_bwd_plan(const dg_lw_params* p, const LwPlan& pl, int N, BwdPlan* bp) {
@@ -356,12 +391,10 @@ static void make_bwd_plan(const dg_lw_params* p, const LwPlan& pl, int N, BwdPla
     off = align_up(off, 256);
     int maxc = 0;
     for (int i = 0; i < 18; ++i) {
-        const int b = i / 2, lvl = block_level(b);
-        bp->cin_tot[i] = i == 0 ? p->in_channels : (i % 2 ? pl.conv_c[i] : (b < 5 ? pl.f[lvl - 1] : 2 * pl.f[lvl]));
         bp->g_off[i] = off;
         off += align_up((size_t)N * pl.conv_h[i] * pl.conv_w[i] * pl.conv_c[i] * sizeof(float), 256);
         bp->t_off[i] = off;
-        if (i > 0) off += align_up((size_t)N * pl.conv_h[i] * pl.conv_w[i] * bp->cin_tot[i] * sizeof(float), 256);
+        if (i > 0) off += align_up((size_t)N * pl.conv_h[i] * pl.conv_w[i] * pl.conv_cin[i] * sizeof(float), 256);
         if (pl.conv_c[i] > maxc) maxc = pl.conv_c[i];
     }
     for (int u = 0; u < 4; ++u) {
@@ -379,48 +412,176 @@ static void make_bwd_plan(const dg_lw_params* p, const LwPlan& pl, int N, BwdPla
     bp->total = off;
 }
 
-// the forward conv i's argument block for images [n0, n0 + nn) (x = the WHOLE batch's input)
-static void fwd_conv_args(const dg_lw_params* p, const LwPlan& pl, char* ws, const float* x, int nn, int i, dg_conv3x3_args* a,
-                          int n0 = 0) {
-    const int b = i / 2;
-    memset(a, 0, sizeof(*a));
-    a->dtype = p->dtype;
-    a->N = nn; a->H = pl.conv_h[i]; a->W = pl.conv_w[i];
-    a->cout = pl.conv_c[i];
-    a->weight = p->conv_w[b][i % 2];
-    a->weight_tc = p->conv_w_tc[b][i % 2];
-    a->out = ws + pl.raw_off[i] + (size_t)n0 * a->H * a->W * a->cout * dtype_size(p->dtype);
-    a->out_stats = reinterpret_cast<double*>(ws + pl.stats_off[i]) + (size_t)n0 * a->cout * 2;
-    a->eps = 1e-5f;
-    a->path = p->path;
-    a->nsrc = 1;
-    if (i == 0) {
-        a->src[0].raw = x + (size_t)n0 * p->in_channels * pl.conv_h[0] * pl.conv_w[0];
-        a->src[0].channels = p->in_channels;
-        a->src[0].groups = 1;
-        a->src[0].xform = DG_X_IMAGE;
-    } else if (i % 2 == 1) {
-        a->src[0] = gn_src(p, pl, ws, i - 1, DG_X_SAME, n0);
-    } else if (b < 5) {
-        a->src[0] = gn_src(p, pl, ws, i - 1, DG_X_POOL2, n0);       // pool1..4, src/model.py:107-112
-    } else {
-        const int lvl = block_level(b), u = b - 5;
-        a->src[0] = gn_src(p, pl, ws, i - 1, DG_X_CONVT2, n0);     // upconv4..1, src/model.py:115-127
-        a->src[0].ct_w = p->up_w[u];
-        a->src[0].ct_b = p->up_b[u];
-        a->src[0].ct_w_tc = p->up_w_tc[u];
-        a->src[0].ct_cout = pl.f[lvl];
-        a->src[1] = gn_src(p, pl, ws, 2 * lvl + 1, DG_X_SAME, n0); // skip: torch.cat((up, skip), 1)
-        a->nsrc = 2;
-    }
-}
-
 // nn.L1Loss backward fused into the head backward: forward output, target, device scalar dLoss (NULL = 1) and 1 / numel
 struct L1Seed { const float* y; const float* target; const float* scale; float inv_numel; };
 
-static int lw_backward_range(const dg_lw_params* p, const struct LwPlan& pl, const struct BwdPlan& bp, const struct GradLayout& gl,
-                             const float* x, const float* grad_y, int n0, int N, int H, int W, char* fw, char* bw,
-                             const BwdRequest& rq, cudaStream_t st, const L1Seed* l1);
+// Backward over images [n0, n0 + N) of a batch of N_total; every buffer was laid out for the whole batch (`N` below is the
+// sub-batch size).  Parameter gradients are accumulated atomically, so concurrent sub-batches add up; the input gradient is per
+// image.  Tensors outside rq.mask get no kernel work, and the loop ends below the lowest requested position.
+static int lw_backward_range(const dg_lw_params* p, const LwPlan& pl, const BwdPlan& bp, const GradLayout& gl, const float* x,
+                             const float* grad_y, int n0, int N, int H, int W, char* fw, char* bw, const BwdRequest& rq,
+                             cudaStream_t st, const L1Seed* l1) {
+    int rc = 0;
+    auto gp = [&](int k) { return ((rq.mask >> k) & 1) ? rq.grads + gl.off[k] : nullptr; };
+    bool t_split[18] = {};   // decoder conv i: T(i) holds the two halves of the concat gradient as two compact tensors
+    auto hwc = [&](int i, int c) { return (size_t)pl.conv_h[i] * pl.conv_w[i] * c; };
+    auto G = [&](int i) { return reinterpret_cast<float*>(bw + bp.g_off[i]) + (size_t)n0 * hwc(i, pl.conv_c[i]); };
+    auto T = [&](int i) { return reinterpret_cast<float*>(bw + bp.t_off[i]) + (size_t)n0 * hwc(i, pl.conv_cin[i]); };
+    auto P = [&](int i) { return reinterpret_cast<double*>(bw + bp.p_off[i]) + (size_t)n0 * pl.conv_c[i] * 2; };
+    auto Rb = [&](int i) { return bw + bp.gb_off[i] + (size_t)n0 * hwc(i, pl.conv_c[i]) * 2; };   // dR_i as bf16 (16-bit tiers)
+    auto raw = [&](int i) { return pl.raw(fw, i, n0); };
+    auto stats = [&](int i) { return pl.stats(fw, i, n0); };
+    auto act_bwd = [&](int j, const float* da, int sa, int oa, const float* db, int sb, int ob) {
+        return act_bwd_launch(p->dtype, raw(j), stats(j), p->gn_w[j / 2][j % 2], p->gn_b[j / 2][j % 2], da, sa, oa, db, sb, ob, G(j),
+                              P(j), N, pl.conv_h[j], pl.conv_w[j], pl.conv_c[j], p->groups[j / 2], kGnEps, st);
+    };
+    // head: src/model.py:131 backward
+    const size_t o0 = (size_t)n0 * p->out_channels * H * W;
+    rc = head_bwd_launch(p->dtype, raw(17), stats(17), p->gn_w[8][1], p->gn_b[8][1],
+                         grad_y ? grad_y + o0 : nullptr, p->head_w, G(17), P(17),
+                         gp(gl.head_w), gp(gl.head_b), N, H, W, pl.conv_c[17], p->out_channels, p->groups[8], kGnEps, st,
+                         l1 ? l1->y + o0 : nullptr, l1 ? l1->target + o0 : nullptr, l1 ? l1->scale : nullptr, l1 ? l1->inv_numel : 0.f);
+    if (rc) return rc;
+    for (int i = 17; i >= 0 && rq.low <= 2 * i; --i) {
+        const int b = i / 2, j = i % 2, C = pl.conv_c[i], Cin = pl.conv_cin[i], Hi = pl.conv_h[i], Wi = pl.conv_w[i];
+        float* const dW = gp(gl.conv_w[b][j]);   // NULL: frozen, no weight-gradient kernel
+        const bool dgrad = rq.low < 2 * i;       // something below conv i wants a gradient (i = 0: the input image)
+        char rname[32];
+        snprintf(rname, sizeof(rname), "bwd %s", kConvNames[i]);
+        NvtxRange range(rname);
+        // dW_i: same sources as the forward conv, correlated with dR_i; written in the parameter's [Co][Ci][3][3] layout.  The
+        // tensor-core wgrad (wa) reads a decoder conv's ConvTranspose output materialised, the CUDA-core one (a) fuses it.
+        const dg_conv3x3_args a = conv_args(p, pl, fw, x, false, n0, N, i);
+        dg_conv3x3_args wa = a;
+        if (a.nsrc == 2) wa.src[0] = up_src(pl, fw, b - 5, n0);
+        // G_i -> dR_i, dgamma / dbeta.  Where BOTH consumers of dR_i are tensor-core kernels (they round it to bf16 anyway) it is
+        // written once as bf16 instead of fp32 in place: they read half the bytes and copy the tile instead of converting it.  A
+        // skipped weight gradient leaves the data gradient to decide alone.
+        void* dRb = nullptr;
+        if (i > 0 && (dW != nullptr || dgrad) && tc16(p) && p->conv_w_tc_bf16[b][j] != nullptr) {
+            bool wg_ok = dW == nullptr, dgr_ok = false;
+            if (dW != nullptr) conv3x3_wgrad_tc_launch(wa, G(i), dW, 1, 9, 9 * Cin, st, &wg_ok, nullptr, /*dry*/ true);
+            conv3x3_dgrad_tc_launch(G(i), p->conv_w_tc_bf16[b][j], G(i), N, Hi, Wi, C, Cin, st, &dgr_ok, nullptr, nullptr, true);
+            if (wg_ok && dgr_ok) dRb = Rb(i);
+        }
+        bool dr_bf16 = false;
+        rc = gn_bwd_apply_launch(p->dtype, raw(i), stats(i), p->gn_w[b][j], P(i), G(i), gp(gl.gn_w[b][j]), gp(gl.gn_b[b][j]),
+                                 N, Hi, Wi, C, p->groups[b], kGnEps, st, dRb, &dr_bf16);
+        if (rc) return rc;
+        const void* dRb_in = dr_bf16 ? dRb : nullptr;   // when set, G(i) still holds G, NOT dR: only the bf16 copy is valid
+        bool wg_done = dW == nullptr;
+        if (dW != nullptr && tc16(p) && i > 0) {
+            // tensor-core wgrad (wgrad_tc.cu): the forward left the deep levels' ConvTranspose output in the workspace, for the
+            // fused levels it is rebuilt here by the same stand-alone kernel
+            bool ok = true;
+            if (a.nsrc == 2 && !lw_up_materialised(pl, b - 5)) {
+                rc = convt_tc_launch(a.src[0], p->dtype, N, Hi, Wi, pl.up(fw, b - 5, n0), kGnEps, p->path, st, &ok);
+                if (rc) return rc;
+            }
+            if (ok) {
+                rc = conv3x3_wgrad_tc_launch(wa, G(i), dW, 1, 9, 9 * Cin, st, &wg_done, dRb_in);
+                if (rc) return rc;
+            }
+        }
+        if (dW != nullptr && i == 0 && !generic_only(p) && p->in_channels == 1) {   // first conv: dedicated streaming kernel (backward.cu)
+            rc = first_wgrad_launch(x + (size_t)n0 * p->in_channels * H * W, G(0), dW, N, Hi, Wi, C, st, &wg_done);
+            if (rc) return rc;
+        }
+        if (!wg_done && dRb_in != nullptr) { set_error("backward: conv %d wgrad probe / launch mismatch", i); return 11; }
+        if (!wg_done) {
+            rc = conv3x3_wgrad_launch(a, G(i), dW, /*tap*/ 1, /*ci*/ 9, /*co*/ 9 * Cin, st);
+            if (rc) return rc;
+        }
+        if (!dgrad) break;
+        if (i == 0)   // dL/dx: dR_0 is fp32 in G(0) in every tier (conv 0 never gets the bf16 copy)
+            return first_dgrad_launch(G(0), p->conv_w[0][0], rq.grad_x + (size_t)n0 * p->in_channels * H * W, N, H, W, p->in_channels, C, st);
+        // dA_in = conv3x3(dR_i, flipped weights): tensor cores where covered (dgrad_tc.cu) ...
+        bool dg_done = false;
+        bool act_fused = false;
+        if (tc16(p) && p->conv_w_tc_bf16[b][j] != nullptr) {
+            if (j == 1) {
+                // the second conv of a block: its input is the activated output of the first and nothing else consumes that, so
+                // the data gradient goes straight through the producer's SiLU' / statistics sums into G(i-1), P(i-1)
+                DgradAct act{raw(i - 1), stats(i - 1), p->gn_w[b][0], p->gn_b[b][0], P(i - 1), p->groups[b], p->dtype, kGnEps};
+                rc = conv3x3_dgrad_tc_launch(G(i), p->conv_w_tc_bf16[b][j], G(i - 1), N, Hi, Wi, C, Cin, st, &dg_done, &act, dRb_in);
+                if (rc) return rc;
+                act_fused = dg_done;
+            }
+            if (!dg_done && j == 0 && b >= 5) {
+                // decoder conv: its input gradient is a concat gradient whose halves go to different consumers -- written as two
+                // compact tensors (up half at T(i), skip half right behind it) instead of one interleaved [.., 2C]
+                rc = conv3x3_dgrad_tc_launch(G(i), p->conv_w_tc_bf16[b][j], T(i), N, Hi, Wi, C, Cin, st, &dg_done, nullptr, dRb_in,
+                                             false, T(i) + (size_t)N * hwc(i, C));
+                if (rc) return rc;
+                t_split[i] = dg_done;
+            }
+            if (!dg_done) {
+                rc = conv3x3_dgrad_tc_launch(G(i), p->conv_w_tc_bf16[b][j], T(i), N, Hi, Wi, C, Cin, st, &dg_done, nullptr, dRb_in);
+                if (rc) return rc;
+            }
+        }
+        // ... the tcgen05 kernel where the mma.sync data gradient has no instance (wider variants): dR rounded to bf16, the
+        // taps-flipped weights in the tensor-core packing, fp32 result (conv3x3_t5.cu, T5_IDENT) ...
+        if (!dg_done && dRb_in == nullptr && tc16(p) && p->conv_w_flip_tc_bf16[b][j] != nullptr) {
+            rc = conv3x3_dgrad_t5_launch(G(i), nullptr, Rb(i), p->conv_w_flip_tc_bf16[b][j], T(i), N, Hi, Wi, C, Cin, st, &dg_done);
+            if (rc) return rc;
+        }
+        // ... else the forward generic kernel on an identity fp32 source
+        if (!dg_done && dRb_in != nullptr) { set_error("backward: conv %d dgrad probe / launch mismatch", i); return 11; }
+        if (!dg_done) {
+            if (p->conv_w_flip[b][j] == nullptr) { set_error("backward: conv %d needs the CUDA-core dgrad but conv_w_flip is NULL", i); return 2; }
+            dg_conv3x3_args d;
+            memset(&d, 0, sizeof(d));
+            d.dtype = DG_F32;
+            d.N = N; d.H = Hi; d.W = Wi;
+            d.cout = Cin;
+            d.weight = p->conv_w_flip[b][j];
+            d.out = T(i);
+            d.eps = kGnEps;
+            d.path = 1;
+            d.nsrc = 1;
+            d.src[0] = ident_src(G(i), C);
+            rc = conv3x3_generic_launch(d, st);
+            if (rc) return rc;
+        }
+        if (j == 1) {
+            if (!act_fused) rc = act_bwd(i - 1, T(i), C, 0, nullptr, 0, 0);
+        } else if (b < 5) {
+            // producer = skip tensor of level b-1: gradient from the decoder's concat (skip half) + this pooled path
+            const int lvl = b - 1, dconv = 2 * (8 - lvl);
+            if (t_split[dconv]) rc = act_bwd(i - 1, T(dconv) + (size_t)N * hwc(dconv, pl.f[lvl]), pl.f[lvl], 0, T(i), pl.f[lvl], 0);
+            else rc = act_bwd(i - 1, T(dconv), 2 * pl.f[lvl], pl.f[lvl], T(i), pl.f[lvl], 0);
+        } else {
+            const int lvl = block_level(b), u = b - 5;
+            float* dlow = reinterpret_cast<float*>(bw + bp.low_off[u]) + (size_t)n0 * (Hi / 2) * (Wi / 2) * pl.f[lvl + 1];
+            // the low-resolution producer feeds nothing but this ConvTranspose: with the tensor-core data gradient its activation
+            // backward is fused into that kernel's epilogue, which then writes G(i-1) / P(i-1) directly
+            // (the ConvTranspose's own data gradient only when something below it, at conv i-1 or lower, is requested)
+            const bool low_wanted = rq.low < 2 * i - 1;
+            const bool try_fuse = low_wanted && tc16(p) && p->up_w_tc_bf16[u] != nullptr;
+            DgradAct lact{raw(i - 1), stats(i - 1), p->gn_w[b - 1][1], p->gn_b[b - 1][1], P(i - 1), p->groups[b - 1], p->dtype, kGnEps};
+            bool low_fused = false;
+            rc = convt_bwd_launch(p->dtype, T(i), t_split[i] ? pl.f[lvl] : 2 * pl.f[lvl], p->up_w[u], p->up_w_t[u], raw(i - 1), stats(i - 1), p->gn_w[b - 1][1],
+                                  p->gn_b[b - 1][1], !low_wanted ? nullptr : try_fuse ? G(i - 1) : dlow, gp(gl.up_w[u]), gp(gl.up_b[u]),
+                                  reinterpret_cast<float*>(bw + bp.coef_off) + (size_t)n0 * bp.maxc * 2, N, Hi, Wi, pl.f[lvl + 1], pl.f[lvl],
+                                  p->groups[b - 1], kGnEps, st, !generic_only(p) ? p->up_w_tc_bf16[u] : nullptr,
+                                  try_fuse ? &lact : nullptr, try_fuse ? &low_fused : nullptr,
+                                  !generic_only(p) ? p->up_w_dgrad_tc_bf16[u] : nullptr,
+                                  p->dtype != DG_F32 ? Rb(i) : nullptr);   // conv i's bf16 dR scratch is free again
+            if (rc) return rc;
+            if (!low_wanted) break;
+            if (low_fused) continue;   // G(i-1), P(i-1) are done
+            if (try_fuse) {            // the kernel declined: G(i-1) holds the plain gradient; act_bwd works in place on it
+                rc = act_bwd(i - 1, G(i - 1), pl.f[lvl + 1], 0, nullptr, 0, 0);
+                if (rc) return rc;
+                continue;
+            }
+            rc = act_bwd(i - 1, dlow, pl.f[lvl + 1], 0, nullptr, 0, 0);
+        }
+        if (rc) return rc;
+    }
+    return 0;
+}
 
 // grads / mask / grad_x as in dg_lw_bwd_request; dg_lw_backward and dg_lw_backward_l1 are mask = every tensor, grad_x = NULL
 static int lw_backward(const dg_lw_params* p, const float* x, const float* grad_y, int N, int H, int W, void* fwd_ws,
@@ -461,213 +622,9 @@ static int lw_backward(const dg_lw_params* p, const float* x, const float* grad_
         k = k1;
     }
     if (e != cudaSuccess) { set_error("memset: %s", cudaGetErrorString(e)); return 10; }
-    const int split = g_split.load();
-    if (split > 0 && N >= split && N >= 2) {   // two concurrent sub-batches, as in lw_forward
-        if ((rc = fork_init())) return rc;
-        FwdFork& F = g_forks[0];
-        cudaEventRecord(F.fork, st);
-        const int half = N / 2;
-        for (int k = 0; k < 2; ++k) {
-            cudaStreamWaitEvent(F.s[k], F.fork, 0);
-            rc = lw_backward_range(p, pl, bp, gl, x, grad_y, k ? half : 0, k ? N - half : half, H, W, fw, bw, rq, F.s[k], l1);
-            cudaEventRecord(F.join[k], F.s[k]);
-            cudaStreamWaitEvent(st, F.join[k], 0);
-            if (rc) return rc;
-        }
-        return 0;
-    }
-    return lw_backward_range(p, pl, bp, gl, x, grad_y, 0, N, H, W, fw, bw, rq, st, l1);
-}
-
-// Backward over images [n0, n0 + N) of a batch of N_total; every buffer was laid out for the whole batch (`N` below is the
-// sub-batch size).  Parameter gradients are accumulated atomically, so concurrent sub-batches add up; the input gradient is per
-// image.  Tensors outside rq.mask get no kernel work, and the loop ends below the lowest requested position.
-static int lw_backward_range(const dg_lw_params* p, const LwPlan& pl, const BwdPlan& bp, const GradLayout& gl, const float* x,
-                             const float* grad_y, int n0, int N, int H, int W, char* fw, char* bw, const BwdRequest& rq,
-                             cudaStream_t st, const L1Seed* l1) {
-    int rc = 0;
-    auto gp = [&](int k) { return ((rq.mask >> k) & 1) ? rq.grads + gl.off[k] : nullptr; };
-    const size_t esz = dtype_size(p->dtype);
-    bool t_split[18] = {};   // decoder conv i: T(i) holds the two halves of the concat gradient as two compact tensors
-    auto hwc = [&](int i, int c) { return (size_t)pl.conv_h[i] * pl.conv_w[i] * c; };
-    auto G = [&](int i) { return reinterpret_cast<float*>(bw + bp.g_off[i]) + (size_t)n0 * hwc(i, pl.conv_c[i]); };
-    auto T = [&](int i) { return reinterpret_cast<float*>(bw + bp.t_off[i]) + (size_t)n0 * hwc(i, bp.cin_tot[i]); };
-    auto P = [&](int i) { return reinterpret_cast<double*>(bw + bp.p_off[i]) + (size_t)n0 * pl.conv_c[i] * 2; };
-    auto raw = [&](int i) { return static_cast<const void*>(fw + pl.raw_off[i] + (size_t)n0 * hwc(i, pl.conv_c[i]) * esz); };
-    auto stats = [&](int i) { return reinterpret_cast<const double*>(fw + pl.stats_off[i]) + (size_t)n0 * pl.conv_c[i] * 2; };
-    auto act_bwd = [&](int j, const float* da, int sa, int oa, const float* db, int sb, int ob) {
-        return act_bwd_launch(p->dtype, raw(j), stats(j), p->gn_w[j / 2][j % 2], p->gn_b[j / 2][j % 2], da, sa, oa, db, sb, ob, G(j),
-                              P(j), N, pl.conv_h[j], pl.conv_w[j], pl.conv_c[j], p->groups[j / 2], 1e-5f, st);
-    };
-    // head: src/model.py:131 backward
-    const size_t o0 = (size_t)n0 * p->out_channels * H * W;
-    rc = head_bwd_launch(p->dtype, raw(17), stats(17), p->gn_w[8][1], p->gn_b[8][1],
-                         grad_y ? grad_y + o0 : nullptr, p->head_w, G(17), P(17),
-                         gp(gl.head_w), gp(gl.head_b), N, H, W, pl.conv_c[17], p->out_channels, p->groups[8], 1e-5f, st,
-                         l1 ? l1->y + o0 : nullptr, l1 ? l1->target + o0 : nullptr, l1 ? l1->scale : nullptr, l1 ? l1->inv_numel : 0.f);
-    if (rc) return rc;
-    for (int i = 17; i >= 0 && rq.low <= 2 * i; --i) {
-        const int b = i / 2, j = i % 2, C = pl.conv_c[i], Hi = pl.conv_h[i], Wi = pl.conv_w[i];
-        float* const dW = gp(gl.conv_w[b][j]);   // NULL: frozen, no weight-gradient kernel
-        const bool dgrad = rq.low < 2 * i;       // something below conv i wants a gradient (i = 0: the input image)
-        char rname[32];
-        snprintf(rname, sizeof(rname), "bwd %s", kConvNames[i]);
-        NvtxRange range(rname);
-        // dW_i: same sources as the forward conv, correlated with dR_i; written in the parameter's [Co][Ci][3][3] layout
-        dg_conv3x3_args a;
-        fwd_conv_args(p, pl, fw, x, N, i, &a, n0);
-        // G_i -> dR_i, dgamma / dbeta.  Where BOTH consumers of dR_i are tensor-core kernels (they round it to bf16 anyway) it is
-        // written once as bf16 instead of fp32 in place: they read half the bytes and copy the tile instead of converting it.  A
-        // skipped weight gradient leaves the data gradient to decide alone.
-        void* dRb = nullptr;
-        if (i > 0 && (dW != nullptr || dgrad) && p->dtype != DG_F32 && (p->path & 3) != 1 && p->conv_w_tc_bf16[b][j] != nullptr) {
-            dg_conv3x3_args probe = a;
-            if (probe.nsrc == 2) {   // the wgrad kernel sees a decoder conv with its ConvTranspose source materialised
-                memset(&probe.src[0], 0, sizeof(dg_src));
-                probe.src[0].raw = fw + pl.up_off[b - 5];
-                probe.src[0].channels = pl.f[block_level(b)];
-                probe.src[0].groups = 1;
-                probe.src[0].xform = DG_X_SAME;
-            }
-            bool wg_ok = dW == nullptr, dgr_ok = false;
-            if (dW != nullptr) conv3x3_wgrad_tc_launch(probe, G(i), dW, 1, 9, 9 * bp.cin_tot[i], st, &wg_ok, nullptr, /*dry*/ true);
-            conv3x3_dgrad_tc_launch(G(i), p->conv_w_tc_bf16[b][j], G(i), N, Hi, Wi, C, bp.cin_tot[i], st, &dgr_ok, nullptr, nullptr, true);
-            if (wg_ok && dgr_ok) dRb = bw + bp.gb_off[i] + (size_t)n0 * hwc(i, C) * 2;
-        }
-        bool dr_bf16 = false;
-        rc = gn_bwd_apply_launch(p->dtype, raw(i), stats(i), p->gn_w[b][j], P(i), G(i), gp(gl.gn_w[b][j]), gp(gl.gn_b[b][j]),
-                                 N, Hi, Wi, C, p->groups[b], 1e-5f, st, dRb, &dr_bf16);
-        if (rc) return rc;
-        const void* dRb_in = dr_bf16 ? dRb : nullptr;   // when set, G(i) still holds G, NOT dR: only the bf16 copy is valid
-        bool wg_done = dW == nullptr;
-        if (dW != nullptr && p->dtype != DG_F32 && (p->path & 3) != 1 && i > 0) {
-            // tensor-core wgrad (wgrad_tc.cu); a decoder conv reads the MATERIALISED ConvTranspose output: the forward left it
-            // in the workspace for the deep levels, for the fused levels it is rebuilt here by the same stand-alone kernel
-            bool ok = true;
-            if (a.nsrc == 2) {
-                const int lvl = block_level(b), u = b - 5;
-                void* up = fw + pl.up_off[u] + (size_t)n0 * Hi * Wi * pl.f[lvl] * esz;
-                const bool have_up = lw_up_materialised(pl, u);
-                if (!have_up) {
-                    rc = convt_tc_launch(a.src[0], p->dtype, N, Hi, Wi, up, 1e-5f, p->path, st, &ok);
-                    if (rc) return rc;
-                }
-                if (ok) {
-                    memset(&a.src[0], 0, sizeof(dg_src));
-                    a.src[0].raw = up;
-                    a.src[0].channels = pl.f[lvl];
-                    a.src[0].groups = 1;
-                    a.src[0].xform = DG_X_SAME;
-                }
-            }
-            if (ok) {
-                rc = conv3x3_wgrad_tc_launch(a, G(i), dW, 1, 9, 9 * bp.cin_tot[i], st, &wg_done, dRb_in);
-                if (rc) return rc;
-            }
-            if (!wg_done) fwd_conv_args(p, pl, fw, x, N, i, &a, n0);  // restore the fused description for the generic kernel
-        }
-        if (dW != nullptr && i == 0 && (p->path & 3) != 1 && p->in_channels == 1) {   // first conv: dedicated streaming kernel (backward.cu)
-            rc = first_wgrad_launch(x + (size_t)n0 * p->in_channels * H * W, G(0), dW, N, Hi, Wi, C, st, &wg_done);
-            if (rc) return rc;
-        }
-        if (!wg_done && dRb_in != nullptr) { set_error("backward: conv %d wgrad probe / launch mismatch", i); return 11; }
-        if (!wg_done) {
-            rc = conv3x3_wgrad_launch(a, G(i), dW, /*tap*/ 1, /*ci*/ 9, /*co*/ 9 * bp.cin_tot[i], st);
-            if (rc) return rc;
-        }
-        if (!dgrad) break;
-        if (i == 0)   // dL/dx: dR_0 is fp32 in G(0) in every tier (conv 0 never gets the bf16 copy)
-            return first_dgrad_launch(G(0), p->conv_w[0][0], rq.grad_x + (size_t)n0 * p->in_channels * H * W, N, H, W, p->in_channels, C, st);
-        // dA_in = conv3x3(dR_i, flipped weights): tensor cores where covered (dgrad_tc.cu) ...
-        bool dg_done = false;
-        bool act_fused = false;
-        if (p->dtype != DG_F32 && (p->path & 3) != 1 && p->conv_w_tc_bf16[b][j] != nullptr) {
-            if (j == 1) {
-                // the second conv of a block: its input is the activated output of the first and nothing else consumes that, so
-                // the data gradient goes straight through the producer's SiLU' / statistics sums into G(i-1), P(i-1)
-                DgradAct act{raw(i - 1), stats(i - 1), p->gn_w[b][0], p->gn_b[b][0], P(i - 1), p->groups[b], p->dtype, 1e-5f};
-                rc = conv3x3_dgrad_tc_launch(G(i), p->conv_w_tc_bf16[b][j], G(i - 1), N, Hi, Wi, C, bp.cin_tot[i], st, &dg_done, &act, dRb_in);
-                if (rc) return rc;
-                act_fused = dg_done;
-            }
-            if (!dg_done && j == 0 && b >= 5) {
-                // decoder conv: its input gradient is a concat gradient whose halves go to different consumers -- written as two
-                // compact tensors (up half at T(i), skip half right behind it) instead of one interleaved [.., 2C]
-                rc = conv3x3_dgrad_tc_launch(G(i), p->conv_w_tc_bf16[b][j], T(i), N, Hi, Wi, C, bp.cin_tot[i], st, &dg_done, nullptr, dRb_in,
-                                             false, T(i) + (size_t)N * hwc(i, C));
-                if (rc) return rc;
-                t_split[i] = dg_done;
-            }
-            if (!dg_done) {
-                rc = conv3x3_dgrad_tc_launch(G(i), p->conv_w_tc_bf16[b][j], T(i), N, Hi, Wi, C, bp.cin_tot[i], st, &dg_done, nullptr, dRb_in);
-                if (rc) return rc;
-            }
-        }
-        // ... the tcgen05 kernel where the mma.sync data gradient has no instance (wider variants): dR rounded to bf16, the
-        // taps-flipped weights in the tensor-core packing, fp32 result (conv3x3_t5.cu, T5_IDENT) ...
-        if (!dg_done && dRb_in == nullptr && p->dtype != DG_F32 && (p->path & 3) != 1 && p->conv_w_flip_tc_bf16[b][j] != nullptr) {
-            rc = conv3x3_dgrad_t5_launch(G(i), nullptr, bw + bp.gb_off[i] + (size_t)n0 * hwc(i, C) * 2, p->conv_w_flip_tc_bf16[b][j], T(i),
-                                         N, Hi, Wi, C, bp.cin_tot[i], st, &dg_done);
-            if (rc) return rc;
-        }
-        // ... else the forward generic kernel on an identity fp32 source
-        dg_conv3x3_args d;
-        memset(&d, 0, sizeof(d));
-        d.dtype = DG_F32;
-        d.N = N; d.H = Hi; d.W = Wi;
-        d.cout = bp.cin_tot[i];
-        d.weight = p->conv_w_flip[b][j];
-        d.out = T(i);
-        d.eps = 1e-5f;
-        d.path = 1;
-        d.nsrc = 1;
-        d.src[0].raw = G(i);
-        d.src[0].channels = C;
-        d.src[0].groups = 1;
-        d.src[0].xform = DG_X_SAME;
-        if (!dg_done && dRb_in != nullptr) { set_error("backward: conv %d dgrad probe / launch mismatch", i); return 11; }
-        if (!dg_done) {
-            if (d.weight == nullptr) { set_error("backward: conv %d needs the CUDA-core dgrad but conv_w_flip is NULL", i); return 2; }
-            rc = conv3x3_generic_launch(d, st);
-            if (rc) return rc;
-        }
-        if (j == 1) {
-            if (!act_fused) rc = act_bwd(i - 1, T(i), C, 0, nullptr, 0, 0);
-        } else if (b < 5) {
-            // producer = skip tensor of level b-1: gradient from the decoder's concat (skip half) + this pooled path
-            const int lvl = b - 1, dconv = 2 * (8 - lvl);
-            if (t_split[dconv]) rc = act_bwd(i - 1, T(dconv) + (size_t)N * hwc(dconv, pl.f[lvl]), pl.f[lvl], 0, T(i), pl.f[lvl], 0);
-            else rc = act_bwd(i - 1, T(dconv), 2 * pl.f[lvl], pl.f[lvl], T(i), pl.f[lvl], 0);
-        } else {
-            const int lvl = block_level(b), u = b - 5;
-            float* dlow = reinterpret_cast<float*>(bw + bp.low_off[u]) + (size_t)n0 * (Hi / 2) * (Wi / 2) * pl.f[lvl + 1];
-            // the low-resolution producer feeds nothing but this ConvTranspose: with the tensor-core data gradient its activation
-            // backward is fused into that kernel's epilogue, which then writes G(i-1) / P(i-1) directly
-            // (the ConvTranspose's own data gradient only when something below it, at conv i-1 or lower, is requested)
-            const bool low_wanted = rq.low < 2 * i - 1;
-            const bool try_fuse = low_wanted && p->dtype != DG_F32 && (p->path & 3) != 1 && p->up_w_tc_bf16[u] != nullptr;
-            DgradAct lact{raw(i - 1), stats(i - 1), p->gn_w[b - 1][1], p->gn_b[b - 1][1], P(i - 1), p->groups[b - 1], p->dtype, 1e-5f};
-            bool low_fused = false;
-            rc = convt_bwd_launch(p->dtype, T(i), t_split[i] ? pl.f[lvl] : 2 * pl.f[lvl], p->up_w[u], p->up_w_t[u], raw(i - 1), stats(i - 1), p->gn_w[b - 1][1],
-                                  p->gn_b[b - 1][1], !low_wanted ? nullptr : try_fuse ? G(i - 1) : dlow, gp(gl.up_w[u]), gp(gl.up_b[u]),
-                                  reinterpret_cast<float*>(bw + bp.coef_off) + (size_t)n0 * bp.maxc * 2, N, Hi, Wi, pl.f[lvl + 1], pl.f[lvl],
-                                  p->groups[b - 1], 1e-5f, st, (p->path & 3) != 1 ? p->up_w_tc_bf16[u] : nullptr,
-                                  try_fuse ? &lact : nullptr, try_fuse ? &low_fused : nullptr,
-                                  (p->path & 3) != 1 ? p->up_w_dgrad_tc_bf16[u] : nullptr,
-                                  p->dtype != DG_F32 ? bw + bp.gb_off[i] + (size_t)n0 * hwc(i, C) * 2 : nullptr);   // conv i's bf16 dR scratch is free again
-            if (rc) return rc;
-            if (!low_wanted) break;
-            if (low_fused) continue;   // G(i-1), P(i-1) are done
-            if (try_fuse) {            // the kernel declined: G(i-1) holds the plain gradient; act_bwd works in place on it
-                rc = act_bwd(i - 1, G(i - 1), pl.f[lvl + 1], 0, nullptr, 0, 0);
-                if (rc) return rc;
-                continue;
-            }
-            rc = act_bwd(i - 1, dlow, pl.f[lvl + 1], 0, nullptr, 0, 0);
-        }
-        if (rc) return rc;
-    }
-    return 0;
+    return run_halves(st, 0, N, [&](int n0, int nn, cudaStream_t s) {   // two concurrent sub-batches, as in lw_forward
+        return lw_backward_range(p, pl, bp, gl, x, grad_y, n0, nn, H, W, fw, bw, rq, s, l1);
+    });
 }
 
 // ---- host-buffer pipeline state --------------------------------------------------------------
