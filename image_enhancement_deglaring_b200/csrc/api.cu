@@ -907,7 +907,7 @@ static int check_gn(const char* who, const void* raw, const double* stats, const
 }
 
 int dg_head1x1_bwd(const dg_head_args* a, const float* grad_y, float* G, double* P, float* dW, float* dB, dg_stream_t stream) {
-    if (a == nullptr || grad_y == nullptr || G == nullptr || P == nullptr || dW == nullptr || dB == nullptr) {
+    if (a == nullptr || grad_y == nullptr || G == nullptr || P == nullptr) {   // dW / dB NULL: that gradient is not computed
         set_error("head backward: null pointer");
         return 2;
     }
@@ -975,8 +975,12 @@ int dg_scale_bwd_sum(int32_t dtype, const void* raw, const double* stats, const 
 
 int dg_channel_attention_bwd(const double* act_sum, double plane, const float* w1, const float* w2, const double* dscale, int32_t N,
                              int32_t C, int32_t hidden, float* add, float* dw1, float* dw2, dg_stream_t stream) {
-    if (act_sum == nullptr || w1 == nullptr || w2 == nullptr || dscale == nullptr || add == nullptr || dw1 == nullptr || dw2 == nullptr) {
+    if (act_sum == nullptr || w1 == nullptr || w2 == nullptr || dscale == nullptr) {
         set_error("attention backward: null pointer");
+        return 2;
+    }
+    if ((dw1 == nullptr) != (dw2 == nullptr) || (dw1 == nullptr && add == nullptr)) {
+        set_error("attention backward: request dw1 and dw2 together, and at least one of them or add");
         return 2;
     }
     if (N < 1 || C < 1 || hidden < 1 || plane <= 0.0 || (size_t)(2 * C + 3 * hidden) * sizeof(float) > 48 * 1024) {

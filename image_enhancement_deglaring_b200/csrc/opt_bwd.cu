@@ -142,6 +142,9 @@ __global__ void __launch_bounds__(OB_THREADS) scale_bwd_sum_kernel(const ScaleBw
 // forward (se.cu): m = act_sum / plane; a = W1 m; h = silu(a); z = W2 h; att = sigmoid(z)
 // backward: dz = datt * att (1 - att); dW2 += dz h^T; dh = W2^T dz; da = dh * silu'(a); dW1 += da m^T; dm = W1^T da;
 //           every pixel of the activated tensor receives dm[c] / plane (the mean's gradient)
+// WANT_W: accumulate dW1 / dW2 (a frozen ChannelAttention skips them); WANT_ADD: write dm / plane (nothing upstream of the
+// attended tensor needs a gradient: skip it).  The launcher never instantiates <false, false>.
+template <bool WANT_W, bool WANT_ADD>
 __global__ void se_bwd_kernel(const double* __restrict__ act_sum, double inv_plane, const float* __restrict__ w1,
                               const float* __restrict__ w2, const double* __restrict__ dscale, int C, int hidden,
                               float* __restrict__ add, float* __restrict__ dw1, float* __restrict__ dw2) {
@@ -174,13 +177,19 @@ __global__ void se_bwd_kernel(const double* __restrict__ act_sum, double inv_pla
         const float s = 1.f / (1.f + __expf(-pre[j]));
         da[j] = d * s * (1.f + pre[j] * (1.f - s));
     }
-    for (int i = threadIdx.x; i < C * hidden; i += blockDim.x) atomicAdd(dw2 + i, dz[i / hidden] * h[i % hidden]);
+    if constexpr (WANT_W) {
+        for (int i = threadIdx.x; i < C * hidden; i += blockDim.x) atomicAdd(dw2 + i, dz[i / hidden] * h[i % hidden]);
+    }
     __syncthreads();
-    for (int i = threadIdx.x; i < hidden * C; i += blockDim.x) atomicAdd(dw1 + i, da[i / C] * mean[i % C]);
-    for (int c = threadIdx.x; c < C; c += blockDim.x) {
-        float d = 0.f;
-        for (int j = 0; j < hidden; ++j) d = fmaf(w1[j * C + c], da[j], d);
-        add[(size_t)n * C + c] = (float)((double)d * inv_plane);
+    if constexpr (WANT_W) {
+        for (int i = threadIdx.x; i < hidden * C; i += blockDim.x) atomicAdd(dw1 + i, da[i / C] * mean[i % C]);
+    }
+    if constexpr (WANT_ADD) {
+        for (int c = threadIdx.x; c < C; c += blockDim.x) {
+            float d = 0.f;
+            for (int j = 0; j < hidden; ++j) d = fmaf(w1[j * C + c], da[j], d);
+            add[(size_t)n * C + c] = (float)((double)d * inv_plane);
+        }
     }
 }
 
@@ -224,7 +233,12 @@ int scale_bwd_sum_launch(int dtype, const void* raw, const double* stats, const 
 int se_bwd_launch(const double* act_sum, double plane, const float* w1, const float* w2, const double* dscale, int N, int C,
                   int hidden, float* add, float* dw1, float* dw2, cudaStream_t st) {
     const size_t smem = (size_t)(2 * C + 3 * hidden) * sizeof(float);
-    se_bwd_kernel<<<N, 128, smem, st>>>(act_sum, 1.0 / plane, w1, w2, dscale, C, hidden, add, dw1, dw2);
+    if (dw1 != nullptr && add != nullptr)
+        se_bwd_kernel<true, true><<<N, 128, smem, st>>>(act_sum, 1.0 / plane, w1, w2, dscale, C, hidden, add, dw1, dw2);
+    else if (dw1 != nullptr)
+        se_bwd_kernel<true, false><<<N, 128, smem, st>>>(act_sum, 1.0 / plane, w1, w2, dscale, C, hidden, add, dw1, dw2);
+    else
+        se_bwd_kernel<false, true><<<N, 128, smem, st>>>(act_sum, 1.0 / plane, w1, w2, dscale, C, hidden, add, dw1, dw2);
     count_launch();
     return check_launch("se_bwd");
 }

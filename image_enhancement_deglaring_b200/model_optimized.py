@@ -22,6 +22,52 @@ from . import _lib, ops
 from ._lib import DTYPE_CODES
 
 
+def _producers():
+    """Which units' outputs each unit reads in `_run`: a unit is a 3x3 conv with its GroupNorm, a ChannelAttention, or the head."""
+    enc = ["enc1", "enc2", "enc3", "enc4", "bottleneck"]
+    t = {"enc1.0": (), "enc1.3": ("enc1.0",), "head": ("dec1.3",)}
+    for lvl in range(1, 5):
+        t[enc[lvl] + ".0"] = (enc[lvl - 1] + ".3",)
+        t[enc[lvl] + ".3"] = (enc[lvl] + ".0",)
+        t[f"attention{lvl}"] = (f"enc{lvl}.3",)
+    for k in (4, 3, 2, 1):
+        t[f"upconv{k}.1"] = (f"dec{k + 1}.3" if k < 4 else "bottleneck.3",)
+        t[f"dec{k}.0"] = (f"upconv{k}.1", f"enc{k}.3", f"attention{k}")
+        t[f"dec{k}.3"] = (f"dec{k}.0",)
+    return t
+
+
+def _unit_params(unit):
+    if unit == "head":
+        return ("output.weight", "output.bias")
+    if unit.startswith("attention"):
+        return (unit + ".fc.0.weight", unit + ".fc.2.weight")
+    blk, idx = unit.rsplit(".", 1)
+    return (unit + ".weight", f"{blk}.{int(idx) + 1}.weight", f"{blk}.{int(idx) + 1}.bias")
+
+
+_PRODUCERS = _producers()
+_UNIT_PARAMS = {u: _unit_params(u) for u in _PRODUCERS}
+
+
+def _upstream():
+    """unit -> every unit whose output reaches its inputs (transitively)."""
+    up = {}
+
+    def walk(u):
+        if u not in up:
+            up[u] = set()
+            for p in _PRODUCERS[u]:
+                up[u] |= {p} | walk(p)
+        return up[u]
+    for u in _PRODUCERS:
+        walk(u)
+    return up
+
+
+_UPSTREAM = _upstream()
+
+
 def _on_device_of(t):
     """Make t's GPU the current one for the launches below (the public forward has already refused CPU tensors)."""
     return torch.cuda.device(t.device) if t.is_cuda else contextlib.nullcontext()
@@ -225,17 +271,39 @@ class OptimizedUNet(nn.Module):
     _tc_dgrad_ok = {}   # (cin, cout) -> does the mma.sync data gradient cover the pair (probed once per process)
     _t5_dgrad_ok = {}   # (cin, cout, h, w) -> does the tcgen05 data gradient have a plan
 
-    def _backward(self, keep, grad_y, flat):
-        """All 76 parameter gradients into `flat` (zero on entry; parameters() order, the parameters' own layouts)."""
+    def _backward(self, keep, grad_y, flat, want=None):
+        """The parameter gradients named in `want` (None: all 76) into `flat`, zero on entry, in parameters() order and the
+        parameters' own layouts; `flat` holds either every parameter (unrequested ranges are never written) or only the requested
+        ones.  Nothing no request reads is computed: a conv's weight gradient runs only if its weight is requested, its data
+        gradient only if a requested tensor lies upstream of its inputs, so the walk stops below the lowest request."""
         pk, bk = self._packs(), self._packs_bwd()
         dt = DTYPE_CODES[self.storage]
         N, _, H, W = grad_y.shape
         dev = grad_y.device
+        sizes = {name: p.numel() for name, p in self.named_parameters()}
+        want = set(sizes) if want is None else set(want)
+        if want - set(sizes):
+            raise ValueError(f"OptimizedUNet has no parameters {sorted(want - set(sizes))}")
+        req = {u for u, ps in _UNIT_PARAMS.items() if want.intersection(ps)}
+        reach = {u for u, up in _UPSTREAM.items() if up & req}     # a gradient at the unit's inputs is needed
+        need = reach | req                                            # a gradient at the unit's output is needed
+        layout = list(sizes) if flat.numel() == sum(sizes.values()) else [k for k in sizes if k in want]
         views, off = {}, 0
-        for name, p in self.named_parameters():
-            views[name] = flat[off:off + p.numel()]
-            off += p.numel()
+        for name in layout:
+            views[name] = flat[off:off + sizes[name]]
+            off += sizes[name]
+        if off != flat.numel():
+            raise ValueError(f"flat gradient of {flat.numel()} elements: expected {sum(sizes.values())} or {off}")
+        if not want:
+            return
         T = {}   # conv name -> gradient at the conv's input grid, fp32 NHWC [N,h,w,cin_total]
+
+        def outs(*names):
+            """Views of the requested tensors of a pair a kernel computes together: None for an unrequested pair, a scratch
+            buffer for the unrequested half of a requested one."""
+            if not want.intersection(names):
+                return (None,) * len(names)
+            return tuple(views[k] if k in want else torch.zeros(sizes[k], dtype=torch.float32, device=dev) for k in names)
 
         def gn_of(name):
             blk, idx = name.rsplit(".", 1)
@@ -267,11 +335,12 @@ class OptimizedUNet(nn.Module):
             L = keep[name]
             gn = gn_of(name)
             g, _, groups = pk[gn]
-            ops.gn_bwd_apply(L["raw"], L["stats"], g, groups, dt, N, L["h"], L["w"], L["c"], P, G, views[gn + ".weight"],
-                             views[gn + ".bias"])
-            ops.conv3x3_wgrad(L["srcs"], G, L["cin"], L["c"], N, L["h"], L["w"], dt, path=self.path & 3,
-                              out=views[name + ".weight"])
-            if name != "enc1.0":
+            ops.gn_bwd_apply(L["raw"], L["stats"], g, groups, dt, N, L["h"], L["w"], L["c"], P, G,
+                             *outs(gn + ".weight", gn + ".bias"))
+            if name + ".weight" in want:
+                ops.conv3x3_wgrad(L["srcs"], G, L["cin"], L["c"], N, L["h"], L["w"], dt, path=self.path & 3,
+                                  out=views[name + ".weight"])
+            if name in reach:
                 T[name] = dgrad(name, G)
 
         def act(name, dA, off_a=0):
@@ -286,19 +355,28 @@ class OptimizedUNet(nn.Module):
         L = keep["dec1.3"]
         G = torch.empty((N, H, W, L["c"]), dtype=torch.float32, device=dev)
         P = torch.zeros((N, L["c"], 2), dtype=torch.float64, device=dev)
-        ops.head1x1_bwd(keep["head"], pk["head"][0], grad_y, N, H, W, dt, G, P, views["output.weight"], views["output.bias"])
-        finish("dec1.3", G, P)
+        dW, dB = (views[k] if k in want else None for k in ("output.weight", "output.bias"))
+        ops.head1x1_bwd(keep["head"], pk["head"][0], grad_y, N, H, W, dt, G, P, dW, dB)
+        if "dec1.3" in need:
+            finish("dec1.3", G, P)
         # decoder, top level first (:138-156 backwards)
         for k in (1, 2, 3, 4):
-            act(f"dec{k}.0", T.pop(f"dec{k}.3"))
-            act(f"upconv{k}.1", T[f"dec{k}.0"], 0)                    # first half of torch.cat((dec, enc * att))
-            prod = f"dec{k + 1}.3" if k < 4 else "bottleneck.3"       # nn.Upsample(x2, nearest) backward: 2x2 sums
-            Lp = keep[prod]
-            act(prod, ops.grad_gather(N, Lp["h"], Lp["w"], Lp["c"], u=T.pop(f"upconv{k}.1")))
-        act("bottleneck.0", T.pop("bottleneck.3"))
+            if f"dec{k}.0" in need:
+                act(f"dec{k}.0", T.pop(f"dec{k}.3"))
+            if f"upconv{k}.1" in need:
+                act(f"upconv{k}.1", T[f"dec{k}.0"], 0)                    # first half of torch.cat((dec, enc * att))
+            prod = f"dec{k + 1}.3" if k < 4 else "bottleneck.3"           # nn.Upsample(x2, nearest) backward: 2x2 sums
+            if prod in need:
+                Lp = keep[prod]
+                act(prod, ops.grad_gather(N, Lp["h"], Lp["w"], Lp["c"], u=T.pop(f"upconv{k}.1")))
+        if "bottleneck.0" in need:
+            act("bottleneck.0", T.pop("bottleneck.3"))
         # encoder: each skip tensor feeds the decoder concat (x att), the next level's pool and the attention squeeze
         for lvl in (4, 3, 2, 1):
             name = f"enc{lvl}.3"
+            if f"attention{lvl}" not in need:
+                T.pop(f"dec{lvl}.0", None)     # the concat gradient, the level's largest tensor: nothing below reads it
+                continue
             nxt = "bottleneck.0" if lvl == 4 else f"enc{lvl + 1}.0"
             L = keep[name]
             g, b, groups = pk[gn_of(name)]
@@ -306,19 +384,24 @@ class OptimizedUNet(nn.Module):
             w1, w2 = pk[f"attention{lvl}"]
             tdec = T.pop(f"dec{lvl}.0")
             dscale = ops.scale_bwd_sum(L["raw"], L["stats"], g, b, groups, dt, N, L["h"], L["w"], L["c"], tdec, L["c"])
-            add = ops.channel_attention_bwd(att["act_sum"], att["plane"], w1, w2, dscale, views[f"attention{lvl}.fc.0.weight"],
-                                            views[f"attention{lvl}.fc.2.weight"])
+            dw1, dw2 = outs(f"attention{lvl}.fc.0.weight", f"attention{lvl}.fc.2.weight")
+            if name not in need:   # only the attention's own weights are requested
+                ops.channel_attention_bwd(att["act_sum"], att["plane"], w1, w2, dscale, dw1, dw2, want_add=False)
+                continue
+            add = ops.channel_attention_bwd(att["act_sum"], att["plane"], w1, w2, dscale, dw1, dw2)
             dA = ops.grad_gather(N, L["h"], L["w"], L["c"], a=tdec, off_a=L["c"], a_scale=att["scale"], b=T.pop(nxt), add=add)
             del tdec
             act(name, dA)
             del dA
-            act(f"enc{lvl}.0", T.pop(name))
+            if f"enc{lvl}.0" in need:
+                act(f"enc{lvl}.0", T.pop(name))
 
 
 class _OptimizedUNetFn(torch.autograd.Function):
-    """Autograd bridge of OptimizedUNet: forward keeps the raw activations, backward writes every parameter gradient into one
-    flat buffer (the optimizer's own bucket when FusedAdamW / FlatGradBucket own `.grad` and it is fresh after zero_grad) and
-    ends with the data-parallel mean all-reduce, exactly like the LightweightUNet bridge (train._LightweightUNetFn)."""
+    """Autograd bridge of OptimizedUNet: forward keeps the raw activations, backward writes the gradients of the parameters that
+    need one into one flat buffer (the optimizer's own bucket when FusedAdamW / FlatGradBucket own `.grad` and it is fresh after
+    zero_grad) and ends with the data-parallel mean all-reduce, exactly like the LightweightUNet bridge (train._LightweightUNetFn).
+    Frozen parameters cost no kernel work."""
 
     @staticmethod
     def forward(ctx, module, x, *params):
@@ -335,24 +418,27 @@ class _OptimizedUNetFn(torch.autograd.Function):
         module, keep = ctx.module, ctx.keep
         if keep is None:
             raise RuntimeError("OptimizedUNet: backward through the same forward twice (the saved activations were released)")
-        params = list(module.parameters())
-        total = sum(p.numel() for p in params)
+        named = list(module.named_parameters())
+        # GraphedTrainStep's parameters are not autograd inputs: there the trainable ones are requested
+        want_p = [p.requires_grad for _, p in named] if ctx.direct else list(ctx.needs_input_grad[2:])
+        want = [k for (k, _), w in zip(named, want_p) if w]
         grad_y = grad_y.detach().float().contiguous()
         with _on_device_of(grad_y):
-            sink = _flat_grad_sink(params)
+            sink = _flat_grad_sink([p for _, p in named], want_p)
             if ctx.direct and sink is None:
                 raise RuntimeError("GraphedTrainStep: the gradients must land in the optimizer's flat bucket (FusedAdamW.zero_grad "
                                    "inside the step, no per-parameter hooks)")
-            flat = sink if sink is not None else torch.zeros(total, dtype=torch.float32, device=grad_y.device)
-            module._backward(keep, grad_y, flat)
+            # the requested gradients only, in parameters() order
+            flat = sink if sink is not None else torch.zeros(sum(p.numel() for (_, p), w in zip(named, want_p) if w),
+                                                              dtype=torch.float32, device=grad_y.device)
+            module._backward(keep, grad_y, flat, want)
         ctx.keep = None
         sync_gradients(flat, getattr(module, "ddp_sync", True))
         if sink is not None:
             sink._dg_zero_version = None      # the bucket now holds a gradient: a second backward accumulates the ordinary way
             return (None, None) + (None,) * ctx.n_inputs
         grads, off = [], 0
-        for p in params:
-            n = p.numel()
-            grads.append(flat[off:off + n].view_as(p) if p.requires_grad else None)
-            off += n
+        for (_, p), w in zip(named, want_p):
+            grads.append(flat[off:off + p.numel()].view_as(p) if w else None)
+            off += p.numel() if w else 0
         return (None, None, *grads)

@@ -234,6 +234,7 @@ def flip_conv3x3(w):
 
 
 def head1x1_bwd(src, weight, grad_y, N, H, W, dtype, G, P, dW, dB, stream=None, eps=1e-5):
+    """G / P of the head's source conv; dW / dB accumulated (None: that gradient is not computed)."""
     a = DgHeadArgs()
     a.src = src
     a.dtype = dtype
@@ -282,11 +283,12 @@ def scale_bwd_sum(raw, stats, gamma, beta, groups, dtype, N, H, W, channels, d, 
     return out
 
 
-def channel_attention_bwd(act_sum, plane, w1, w2, dscale, dw1, dw2, stream=None):
-    """ChannelAttention backward (dg_channel_attention_bwd): accumulates dw1 / dw2, returns add [N,C] fp32."""
+def channel_attention_bwd(act_sum, plane, w1, w2, dscale, dw1, dw2, want_add=True, stream=None):
+    """ChannelAttention backward (dg_channel_attention_bwd): accumulates dw1 / dw2 (both None: skipped), returns add [N,C] fp32
+    (None with want_add=False)."""
     _require_cuda(act_sum, w1, w2, dscale, dw1, dw2)
     N, channels = act_sum.shape
-    add = torch.empty((N, channels), dtype=torch.float32, device=act_sum.device)
+    add = torch.empty((N, channels), dtype=torch.float32, device=act_sum.device) if want_add else None
     _lib.check(_lib.load().dg_channel_attention_bwd(_ptr(act_sum), float(plane), _ptr(w1), _ptr(w2), _ptr(dscale), N, channels,
                                                     int(w1.shape[0]), _ptr(add), _ptr(dw1), _ptr(dw2), _stream(stream)))
     return add

@@ -31,24 +31,49 @@ class _TrainCtx:
         self.y = self.l1_target = self.l1_scale = self.l1_marker = None
 
 
-def _flat_grad_sink(params):
-    """The flat fp32 buffer all `.grad`s are views of (FusedAdamW / FlatGradBucket layout, parameters() order) if it is known to be
-    all-zero since its last zero_grad and nothing else would observe the per-parameter accumulation; else None."""
-    g0 = params[0].grad
-    if g0 is None:
+def _flat_grad_sink(params, want=None):
+    """The flat fp32 buffer whose consecutive views are the `.grad`s of the parameters flagged in `want` (default: those that
+    require a gradient), in parameters() order -- the FusedAdamW / FlatGradBucket layout over the trainable parameters -- if it is
+    known to be all-zero since its last zero_grad and nothing else would observe the per-parameter accumulation; else None.
+    No other parameter's `.grad` may live in it."""
+    if want is None:
+        want = [p.requires_grad for p in params]
+    sel = [p for p, w in zip(params, want) if w]
+    if not sel or sel[0].grad is None:
         return None
+    g0 = sel[0].grad
     base = g0._base if g0._base is not None else g0
     if getattr(base, "_dg_zero_version", None) != base._version or base.dtype != torch.float32 or not base.is_contiguous():
         return None
     off = 0
-    for p in params:
+    for p in sel:
         g = p.grad
         if g is None or not p.requires_grad or g.data_ptr() != base.data_ptr() + 4 * off or g.numel() != p.numel():
             return None
         if p._backward_hooks or getattr(p, "_post_accumulate_grad_hooks", None):
             return None     # wandb.watch and friends hook the per-parameter accumulation: keep the ordinary autograd path
         off += p.numel()
-    return base if off == base.numel() else None
+    if off != base.numel():
+        return None
+    storage = base.untyped_storage().data_ptr()
+    if any(not w and p.grad is not None and p.grad.untyped_storage().data_ptr() == storage for p, w in zip(params, want)):
+        return None
+    return base
+
+
+def _gather_index(module, params, want, device):
+    """Positions of the flagged parameters' elements in the full parameters() layout, built once per request and kept on the
+    module for its lifetime: a captured step reads the index by address, so no later request may release it."""
+    cache = module.__dict__.setdefault("_dg_gather_index", {})
+    key = (tuple(want), device)
+    if key not in cache:
+        idx, off = [], 0
+        for p, w in zip(params, want):
+            if w:
+                idx.append(torch.arange(off, off + p.numel()))
+            off += p.numel()
+        cache[key] = torch.cat(idx).to(device)
+    return cache[key]
 
 
 class _LightweightUNetFn(torch.autograd.Function):
@@ -79,9 +104,9 @@ class _LightweightUNetFn(torch.autograd.Function):
         params = list(module.parameters())
         total = sum(p.numel() for p in params)
         # Only what autograd asks for is computed: dL/dx when x needs it, the gradients of parameters that require one, and the
-        # backward stops below the lowest of them.  GraphedTrainStep's parameters are not autograd inputs: it always wants all.
+        # backward stops below the lowest of them.  GraphedTrainStep's parameters are not autograd inputs: it wants the trainable ones.
         want_x = ctx.needs_input_grad[2]
-        want_p = [True] * len(params) if ctx.direct else list(ctx.needs_input_grad[3:])
+        want_p = [p.requires_grad for p in params] if ctx.direct else list(ctx.needs_input_grad[3:])
         if len(want_p) != 64:
             raise RuntimeError(f"gradient layout mismatch: {len(want_p)} parameter tensors, the library's backward has 64")
         mask = sum(1 << k for k, w in enumerate(want_p) if w)
@@ -96,12 +121,16 @@ class _LightweightUNetFn(torch.autograd.Function):
             if cnt.value != total:
                 raise RuntimeError(f"gradient layout mismatch: library {cnt.value} vs module {total}")
             # gradients go straight into the optimizer's flat bucket when that is safe (fresh after zero_grad, no hooks): no
-            # per-parameter accumulate kernels, no temporary.  A fully frozen net gets no flat buffer at all.
-            sink = _flat_grad_sink(params) if total > 0 and mask else None
+            # per-parameter accumulate kernels.  A bucket over a subset of the parameters is filled by one gather from the
+            # native full layout.  A fully frozen net gets no flat buffer at all.
+            sink = _flat_grad_sink(params, want_p) if total > 0 and mask else None
             if ctx.direct and sink is None:
                 raise RuntimeError("GraphedTrainStep: the gradients must land in the optimizer's flat bucket (FusedAdamW.zero_grad "
                                    "inside the step, no per-parameter hooks)")
-            flat = sink if sink is not None else (torch.empty(total, dtype=torch.float32, device=x.device) if mask else None)
+            if sink is not None and sink.numel() == total:
+                flat = sink
+            else:
+                flat = torch.empty(total, dtype=torch.float32, device=x.device) if mask else None
             grad_x = torch.empty_like(x) if want_x else None
             stream = torch.cuda.current_stream().cuda_stream
             fused_l1 = (tctx.l1_target is not None and tctx.l1_marker is not None and grad_y.data_ptr() == tctx.l1_marker.data_ptr()
@@ -132,6 +161,9 @@ class _LightweightUNetFn(torch.autograd.Function):
             grad_x = grad_x.to(ctx.x_dtype)
         if flat is None:
             return (None, None, grad_x) + (None,) * ctx.n_inputs
+        if sink is not None and sink is not flat:
+            torch.index_select(flat, 0, _gather_index(module, params, want_p, flat.device), out=sink)
+            flat = sink
         sync_gradients(flat, getattr(module, "ddp_sync", True))   # parameter gradients only: dL/dx is per rank's own batch
         if sink is not None:
             sink._dg_zero_version = None      # the bucket now holds a gradient: a second backward must accumulate the ordinary way
@@ -375,6 +407,28 @@ class FusedAdamW(torch.optim.Optimizer):
         return float(self._scratch.sqrt().item())
 
 
+def _check_trainable(module, opt_params):
+    """The optimizer's parameters must be the module's trainable ones, in parameters() order: the gradients land in its flat
+    bucket in that layout."""
+    names = {id(p): k for k, p in module.named_parameters()}
+    trainable = [p for p in module.parameters() if p.requires_grad]
+    if not trainable:
+        raise ValueError("GraphedTrainStep: the module has no trainable parameter (requires_grad)")
+
+    def what(p):
+        if p is None:
+            return "nothing"
+        if id(p) not in names:
+            return "a tensor that is not a parameter of the module"
+        return names[id(p)] + ("" if p.requires_grad else " (frozen)")
+    for i in range(max(len(trainable), len(opt_params))):
+        a = opt_params[i] if i < len(opt_params) else None
+        b = trainable[i] if i < len(trainable) else None
+        if a is not b:
+            raise ValueError(f"GraphedTrainStep: the optimizer must hold exactly the module's trainable parameters in parameters() "
+                             f"order; at position {i} it has {what(a)} where the module's trainable parameters have {what(b)}")
+
+
 class GraphedTrainStep:
     """One training step of the reference loop (optimized_train.py:201-233: zero_grad, forward, L1, backward -- with the data-parallel
     all-reduce at its end -- clip, AdamW) captured ONCE in a CUDA graph and replayed per batch.
@@ -382,6 +436,8 @@ class GraphedTrainStep:
     Why: at the reference's own configuration (global batch 32 = 4 images per GPU on 8 GPUs) a step is ~75 kernels of 10-50 us
     plus the packing kernels of the updated weights; issued from Python the host launch rate bounds it, not the GPU.
     Needs a `FusedAdamW(..., capturable=True)` (step count and learning rate in device memory) and fixed batch shapes.
+    Trainable means `requires_grad`: the optimizer must hold exactly the module's trainable parameters, in parameters() order,
+    and only their gradients are computed (fine-tuning with frozen layers; the frozen ones cost no kernel work).
 
         step = GraphedTrainStep(net, opt, criterion, inputs.shape)
         for inputs, targets in loader: loss = step(inputs, targets)      # loss: 0-d device tensor, valid until the next call
@@ -390,6 +446,7 @@ class GraphedTrainStep:
     def __init__(self, module, optimizer, criterion, shape, warmup=3, clip_grad_norm=None):
         if not getattr(optimizer, "capturable", False):
             raise RuntimeError("GraphedTrainStep needs FusedAdamW(..., capturable=True)")
+        _check_trainable(module, optimizer._ps)
         dev = next(module.parameters()).device
         self.module, self.optimizer, self.criterion, self.clip = module, optimizer, criterion, clip_grad_norm
         # The warm-up steps run with lr = 0 and weight decay 0 against saved moments: they must not train.  Their input is uniform

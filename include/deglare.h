@@ -178,8 +178,9 @@ int dg_channel_attention(const double* act_sum, double plane, const float* w1, c
  *
  * dg_head1x1_bwd: backward of dg_head1x1 (src/optimized_model.py:74,158) for grad_y = dL/d(out) fp32 [N,cout,H,W] (cout <= 4):
  *   G [N,H,W,C] = dL/dy of the head's source conv, P [N,C,2] += per-(n, c) (sum G, sum G*xhat) (zero on entry),
- *   dW [cout][C] and dB [cout] += the 1x1 conv's parameter gradients (zero on entry, or a running sum).  `a` is the forward
- *   call's argument block (out / target / l1_sum ignored).
+ *   dW [cout][C] and dB [cout] += the 1x1 conv's parameter gradients (zero on entry, or a running sum); either may be NULL, and
+ *   that gradient is then not computed (G and P are the same).  `a` is the forward call's argument block (out / target / l1_sum
+ *   ignored).
  * dg_act_bwd: G = (dA_a + 0.25 * replicate2x2(dA_b)) * SiLU'(y) and P += (sum G, sum G*xhat).  dA_a = same-resolution gradient
  *   [N,H,W,stride_a], channels off_a .. off_a+C (one half of a concat gradient is a window of it); dA_b = optional gradient
  *   of the 2x2 average pool of A, [N,H/2,W/2,stride_b] (nn.AvgPool2d backward).  Either may be NULL, not both.
@@ -207,7 +208,9 @@ int dg_grad_gather(const float* a, int32_t stride_a, int32_t off_a, const float*
  *   as the forward does; d = the consumer's input gradient [N,H,W,stride_d]; dscale [N,C] double, zero on entry.
  * dg_channel_attention_bwd: from the forward's act_sum / plane / w1 / w2 (dg_channel_attention) and dscale:
  *   dw1 [hidden][C], dw2 [C][hidden] += the two nn.Linear weight gradients summed over the batch (zero on entry or a running
- *   sum); add[n][c] = dL/dmean[n][c] / plane, the constant every pixel of A receives through the global average. */
+ *   sum); add[n][c] = dL/dmean[n][c] / plane, the constant every pixel of A receives through the global average.
+ *   dw1 = dw2 = NULL (both or neither) skips the weight gradients, add = NULL skips the mean's gradient; at least one of the
+ *   two must be requested (else 2). */
 int dg_scale_bwd_sum(int32_t dtype, const void* raw, const double* stats, const float* gamma, const float* beta, int32_t groups,
                      const float* d, int32_t stride_d, int32_t off_d, double* dscale, int32_t N, int32_t H, int32_t W, int32_t C,
                      float eps, dg_stream_t stream);
