@@ -16,6 +16,7 @@ import torch.nn as nn
 
 from . import _lib, ops
 from ._lib import DTYPE_CODES, DgLwParams
+from .train import _gather_index, train_forward
 
 _BLOCKS = ("enc1", "enc2", "enc3", "enc4", "bottleneck", "dec4", "dec3", "dec2", "dec1")
 
@@ -198,8 +199,7 @@ class LightweightUNet(nn.Module):
         if x.dim() != 4 or x.shape[1] != self.in_channels:
             raise RuntimeError(f"expected input [N,{self.in_channels},H,W], got {tuple(x.shape)}")
         if torch.is_grad_enabled() and (x.requires_grad or any(p.requires_grad for p in self.parameters())):
-            from .train import lightweight_forward_train
-            return lightweight_forward_train(self, x)
+            return train_forward(self, x)
         x = x.detach().float().contiguous()
         N, _, H, W = x.shape
         with torch.cuda.device(x.device):   # the library launches on the CURRENT device's stream: make it the tensors' device
@@ -209,6 +209,62 @@ class LightweightUNet(nn.Module):
             _lib.check(lib.dg_lw_forward(C.byref(pc), x.data_ptr(), y.data_ptr(), N, H, W, ws.data_ptr(), ws.numel(),
                                          None, None, torch.cuda.current_stream().cuda_stream))
         return y
+
+    # ---- training: the model half of train._TrainFn ------------------------------------------------------------------------
+    _fused_l1 = True   # the backward generates train.L1Loss's gradient seed inside the head backward
+
+    def _train_forward(self, x):
+        """y, and what the backward re-reads: a workspace of its own (raw activations, statistics) and x as fp32."""
+        x = x.detach().float().contiguous()
+        N, _, H, W = x.shape
+        pc = self._refresh(train=True)
+        ws = torch.empty(self.workspace_bytes(N, H, W), dtype=torch.uint8, device=x.device)
+        y = torch.empty((N, self.out_channels, H, W), dtype=torch.float32, device=x.device)
+        _lib.check(_lib.load().dg_lw_forward(C.byref(pc), x.data_ptr(), y.data_ptr(), N, H, W, ws.data_ptr(), ws.numel(),
+                                             None, None, torch.cuda.current_stream().cuda_stream))
+        return y, (ws, x)
+
+    def _train_backward(self, saved, grad_y, tctx, want_p, grad_x, sink):
+        """One dg_lw_backward_select for every request: any subset of the parameters, dL/dx or not, grad_y or the fused-L1 seed.
+        The native layout is the full one; a sink over a subset of the parameters is filled by one gather from a scratch buffer."""
+        lib = _lib.load()
+        ws, x = saved
+        N, _, H, W = x.shape
+        params = list(self.parameters())
+        total = sum(p.numel() for p in params)
+        if len(want_p) != 64:
+            raise RuntimeError(f"gradient layout mismatch: {len(want_p)} parameter tensors, the library's backward has 64")
+        mask = sum(1 << k for k, w in enumerate(want_p) if w)
+        pc = self._refresh(train=True)
+        nb = C.c_size_t(0)
+        _lib.check(lib.dg_lw_backward_workspace_bytes(C.byref(pc), N, H, W, C.byref(nb)))
+        bws = torch.empty(nb.value, dtype=torch.uint8, device=x.device)
+        cnt = C.c_size_t(0)
+        _lib.check(lib.dg_lw_num_params(C.byref(pc), C.byref(cnt)))
+        if cnt.value != total:
+            raise RuntimeError(f"gradient layout mismatch: library {cnt.value} vs module {total}")
+        # the backward zeroes the requested ranges itself; a frozen range is never written
+        if sink is not None and sink.numel() == total:
+            flat = sink
+        else:
+            flat = torch.empty(total, dtype=torch.float32, device=x.device) if mask else None
+        req = _lib.DgLwBwdRequest()
+        if (tctx.l1_target is not None and tctx.l1_marker is not None and grad_y.data_ptr() == tctx.l1_marker.data_ptr()
+                and all(s == 0 for s in grad_y.stride())):
+            # loss = train.L1Loss: the seed sign(y - t) * dloss / numel is generated inside the head backward
+            req.y, req.target, req.loss_grad = tctx.y.data_ptr(), tctx.l1_target.data_ptr(), tctx.l1_scale.data_ptr()
+        else:
+            grad_y = grad_y.detach().float().contiguous()
+            req.grad_y = grad_y.data_ptr()
+        req.grads = flat.data_ptr() if flat is not None else None
+        req.param_mask = mask
+        req.grad_x = grad_x.data_ptr() if grad_x is not None else None
+        _lib.check(lib.dg_lw_backward_select(C.byref(pc), x.data_ptr(), C.byref(req), N, H, W, ws.data_ptr(), ws.numel(),
+                                             bws.data_ptr(), bws.numel(), torch.cuda.current_stream().cuda_stream))
+        if sink is not None and sink is not flat:
+            torch.index_select(flat, 0, _gather_index(self, params, want_p, flat.device), out=sink)
+            return sink
+        return flat
 
     def forward_u8(self, x):
         """uint8 in, uint8 out: the /infer pre/post-processing of api/app.py:153,190-193 folded into the first and last

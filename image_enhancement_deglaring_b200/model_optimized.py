@@ -13,13 +13,12 @@ Mapping onto the fused 3x3 conv (include/deglare.h):
                                   two tiny mat-vecs (dg_channel_attention), scale applied on load (dg_src.scale) :185-202
   torch.cat((up, skip*att))    -> two-source conv, never materialised                                    :140-156
 """
-import contextlib
-
 import torch
 import torch.nn as nn
 
 from . import _lib, ops
 from ._lib import DTYPE_CODES
+from .train import _on_device_of, train_forward
 
 
 def _producers():
@@ -66,11 +65,6 @@ def _upstream():
 
 
 _UPSTREAM = _upstream()
-
-
-def _on_device_of(t):
-    """Make t's GPU the current one for the launches below (the public forward has already refused CPU tensors)."""
-    return torch.cuda.device(t.device) if t.is_cuda else contextlib.nullcontext()
 
 
 class ChannelAttention(nn.Module):
@@ -199,12 +193,7 @@ class OptimizedUNet(nn.Module):
         if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             if x.requires_grad:
                 raise NotImplementedError("gradient w.r.t. the input image is not implemented (the reference never needs it)")
-            if getattr(self, "_dg_direct_grads", False):
-                # train.GraphedTrainStep: inside a captured step the parameters are not autograd inputs (their AccumulateGrad nodes
-                # would join the stream they were created on into the capture); a fresh leaf anchors the node and the gradients go
-                # straight into the optimizer's flat bucket
-                return _OptimizedUNetFn.apply(self, x, torch.zeros((), device=x.device, requires_grad=True))
-            return _OptimizedUNetFn.apply(self, x, *self.parameters())
+            return train_forward(self, x)
         with _on_device_of(x):
             return self._run(x)
 
@@ -270,6 +259,22 @@ class OptimizedUNet(nn.Module):
     # ---- training: autograd of the forward above (optimized_train.py:210/226 drives it through loss.backward()) ----------------
     _tc_dgrad_ok = {}   # (cin, cout) -> does the mma.sync data gradient cover the pair (probed once per process)
     _t5_dgrad_ok = {}   # (cin, cout, h, w) -> does the tcgen05 data gradient have a plan
+
+    def _train_forward(self, x):
+        """The model half of train._TrainFn: y, and the raw activations the backward re-reads."""
+        keep = {}
+        return self._run(x, keep), keep
+
+    def _train_backward(self, keep, grad_y, tctx, want_p, grad_x, sink):
+        """The gradients of the parameters flagged in `want_p` into `sink`, or into a zeroed buffer in the compact layout over
+        them.  No input gradient (the forward refuses an input that requires one) and no fused L1 seed (`tctx` is None)."""
+        named = list(self.named_parameters())
+        want = [k for (k, _), w in zip(named, want_p) if w]
+        grad_y = grad_y.detach().float().contiguous()
+        flat = sink if sink is not None else torch.zeros(sum(p.numel() for (_, p), w in zip(named, want_p) if w),
+                                                          dtype=torch.float32, device=grad_y.device)
+        self._backward(keep, grad_y, flat, want)
+        return flat
 
     def _backward(self, keep, grad_y, flat, want=None):
         """The parameter gradients named in `want` (None: all 76) into `flat`, zero on entry, in parameters() order and the
@@ -395,50 +400,3 @@ class OptimizedUNet(nn.Module):
             del dA
             if f"enc{lvl}.0" in need:
                 act(f"enc{lvl}.0", T.pop(name))
-
-
-class _OptimizedUNetFn(torch.autograd.Function):
-    """Autograd bridge of OptimizedUNet: forward keeps the raw activations, backward writes the gradients of the parameters that
-    need one into one flat buffer (the optimizer's own bucket when FusedAdamW / FlatGradBucket own `.grad` and it is fresh after
-    zero_grad) and ends with the data-parallel mean all-reduce, exactly like the LightweightUNet bridge (train._LightweightUNetFn).
-    Frozen parameters cost no kernel work."""
-
-    @staticmethod
-    def forward(ctx, module, x, *params):
-        keep = {}
-        with _on_device_of(x):
-            y = module._run(x, keep)
-        ctx.module, ctx.keep, ctx.n_inputs = module, keep, len(params)
-        ctx.direct = getattr(module, "_dg_direct_grads", False)
-        return y
-
-    @staticmethod
-    def backward(ctx, grad_y):
-        from .train import _flat_grad_sink, sync_gradients
-        module, keep = ctx.module, ctx.keep
-        if keep is None:
-            raise RuntimeError("OptimizedUNet: backward through the same forward twice (the saved activations were released)")
-        named = list(module.named_parameters())
-        # GraphedTrainStep's parameters are not autograd inputs: there the trainable ones are requested
-        want_p = [p.requires_grad for _, p in named] if ctx.direct else list(ctx.needs_input_grad[2:])
-        want = [k for (k, _), w in zip(named, want_p) if w]
-        grad_y = grad_y.detach().float().contiguous()
-        with _on_device_of(grad_y):
-            sink = _flat_grad_sink([p for _, p in named], want_p)
-            if ctx.direct and sink is None:
-                raise RuntimeError("GraphedTrainStep: the gradients must land in the optimizer's flat bucket (FusedAdamW.zero_grad "
-                                   "inside the step, no per-parameter hooks)")
-            # the requested gradients only, in parameters() order
-            flat = sink if sink is not None else torch.zeros(sum(p.numel() for (_, p), w in zip(named, want_p) if w),
-                                                              dtype=torch.float32, device=grad_y.device)
-            module._backward(keep, grad_y, flat, want)
-        ctx.keep = None
-        sync_gradients(flat, getattr(module, "ddp_sync", True))
-        if sink is not None:
-            sink._dg_zero_version = None      # the bucket now holds a gradient: a second backward accumulates the ordinary way
-            return (None, None) + (None,) * ctx.n_inputs
-        grads, off = [], 0
-        for (_, p), w in zip(named, want_p):
-            grads.append(flat[off:off + p.numel()].view_as(p) if w else None)
-            off += p.numel() if w else 0
-        return (None, None, *grads)

@@ -9,6 +9,8 @@ The reference has no distributed code at all (optimized_train.py:383 is single-d
 import torch
 import torch.distributed as dist
 
+from .train import _alias_grads, _zero_grads
+
 
 def shard_range(n_items, rank, world):
     """Contiguous [start, stop) slice of `n_items` independent units (images / tiles) owned by `rank`.
@@ -65,16 +67,10 @@ class FlatGradBucket:
         self.attach()
 
     def attach(self):
-        off = 0
-        for p in self.params:
-            n = p.numel()
-            p.grad = self.flat[off:off + n].view_as(p)
-            off += n
+        _alias_grads(self.flat, self.params)
 
     def zero_(self):
-        self.flat.zero_()
-        self.flat._dg_zero_version = self.flat._version   # lets the fused backward write straight into the bucket (train._flat_grad_sink)
-        self.attach()
+        _zero_grads(self.flat, self.params)   # lets the fused backward write straight into the bucket
 
     def allreduce_mean(self, group=None):
         if dist.is_available() and dist.is_initialized():

@@ -1,21 +1,22 @@
-"""Training path of the drop-in module: autograd bridge to dg_lw_forward / dg_lw_backward and the fused optimizer tail.
+"""Training path of the drop-in modules: one autograd bridge for LightweightUNet and OptimizedUNet, and the fused optimizer tail.
 
 Reference call sequence (optimized_train.py:197-236, fp32 branch :220-233):
     optimizer.zero_grad(set_to_none=True); outputs = model(inputs); loss = criterion(outputs, targets)
     loss.backward(); clip_grad_norm_(model.parameters(), 1.0); optimizer.step()
-`model(inputs)` lands in `lightweight_forward_train` when autograd is recording; the gradients autograd asks for (every parameter
-that requires one, and the input image when it does) come back through `torch.autograd.Function.backward`, i.e. they land in
-`param.grad` / `x.grad` the normal way (wandb.watch hooks keep working).  Frozen parameters cost no kernel work.
+`model(inputs)` lands in `train_forward` when autograd is recording; the gradients autograd asks for (every parameter that
+requires one, and the input image when it does) come back through `torch.autograd.Function.backward`, i.e. they land in
+`param.grad` / `x.grad` the normal way (wandb.watch hooks keep working).  Frozen parameters cost no kernel work.  The bridge owns
+the gradient-delivery policy; each model supplies only its own forward and backward (`_train_forward`, `_train_backward`).
 `FusedAdamW` is a `torch.optim.Optimizer` with AdamW's constructor that keeps parameters, gradients and both moments in flat
 buffers and runs clip + update as two kernels (dg_adamw_step).
 
 Data parallel (one process per GPU, SURVEY.md section 8e): the ONE collective of a training step -- the mean all-reduce of the
-flat 486,409-float gradient -- is issued at the END OF BACKWARD (`_LightweightUNetFn.backward`), i.e. between `loss.backward()`
-and everything the reference does next (optimized_train.py:210-219 / :226-233): `scaler.unscale_` + its inf check,
-`clip_grad_norm_`, `optimizer.step()` all see the already-averaged gradient, every rank takes the same skip / clip decision,
-and no rank can miss the collective.  `module.ddp_sync = False` turns it off (gradient accumulation over micro-batches).
+flat gradient (486,409 floats for the shipped LightweightUNet) -- is issued at the END OF BACKWARD (`_TrainFn.backward`), i.e.
+between `loss.backward()` and everything the reference does next (optimized_train.py:210-219 / :226-233): `scaler.unscale_` + its
+inf check, `clip_grad_norm_`, `optimizer.step()` all see the already-averaged gradient, every rank takes the same skip / clip
+decision, and no rank can miss the collective.  `module.ddp_sync = False` turns it off (gradient accumulation over micro-batches).
 """
-import ctypes as C
+import contextlib
 
 import torch
 
@@ -31,10 +32,31 @@ class _TrainCtx:
         self.y = self.l1_target = self.l1_scale = self.l1_marker = None
 
 
+def _on_device_of(t):
+    """Make t's GPU the current one for the launches below; a CPU tensor (the bridge over torch stand-ins of the ops) needs none."""
+    return torch.cuda.device(t.device) if t.is_cuda else contextlib.nullcontext()
+
+
+def _alias_grads(flat, params):
+    """Make each parameter's `.grad` its consecutive view of `flat`, in order: the layout `_flat_grad_sink` accepts."""
+    off = 0
+    for p in params:
+        p.grad = flat[off:off + p.numel()].view_as(p)
+        off += p.numel()
+
+
+def _zero_grads(flat, params):
+    """zero_grad of a flat gradient bucket (FusedAdamW, FlatGradBucket): zero it, stamp it all-zero as of this version -- the
+    stamp `_flat_grad_sink` reads, so that backward may write straight into it -- and alias the `.grad`s again."""
+    flat.zero_()
+    flat._dg_zero_version = flat._version
+    _alias_grads(flat, params)
+
+
 def _flat_grad_sink(params, want=None):
     """The flat fp32 buffer whose consecutive views are the `.grad`s of the parameters flagged in `want` (default: those that
     require a gradient), in parameters() order -- the FusedAdamW / FlatGradBucket layout over the trainable parameters -- if it is
-    known to be all-zero since its last zero_grad and nothing else would observe the per-parameter accumulation; else None.
+    known to be all-zero since its last `_zero_grads` and nothing else would observe the per-parameter accumulation; else None.
     No other parameter's `.grad` may live in it."""
     if want is None:
         want = [p.requires_grad for p in params]
@@ -76,103 +98,66 @@ def _gather_index(module, params, want, device):
     return cache[key]
 
 
-class _LightweightUNetFn(torch.autograd.Function):
+class _TrainFn(torch.autograd.Function):
+    """The autograd node of a training forward, shared by LightweightUNet and OptimizedUNet.  The model computes:
+      module._train_forward(x) -> (y, saved)
+      module._train_backward(saved, grad_y, tctx, want_p, grad_x, sink) -> flat
+        the parameter gradients flagged in `want_p` (parameters() order) into `sink` when given, else into a buffer of the model's
+        own in the full parameters() layout or the compact one over `want_p`; returns the buffer that holds them.  dL/dx into
+        `grad_x` (fp32, x's shape) when given.
+    This node decides which gradients are wanted and where they land -- the optimizer's flat bucket when `_flat_grad_sink` finds it
+    safe (no per-parameter accumulate kernels), else the model's buffer handed to autograd -- and ends with the data-parallel mean
+    all-reduce of the parameter gradients."""
+
     @staticmethod
     def forward(ctx, module, tctx, x, *params):
-        lib = _lib.load()
-        x_dtype = x.dtype
-        x = x.detach().float().contiguous()
-        N, _, H, W = x.shape
-        with torch.cuda.device(x.device):
-            pc = module._refresh(train=True)
-            ws = torch.empty(module.workspace_bytes(N, H, W), dtype=torch.uint8, device=x.device)  # kept for backward
-            y = torch.empty((N, module.out_channels, H, W), dtype=torch.float32, device=x.device)
-            _lib.check(lib.dg_lw_forward(C.byref(pc), x.data_ptr(), y.data_ptr(), N, H, W, ws.data_ptr(), ws.numel(),
-                                         None, None, torch.cuda.current_stream().cuda_stream))
-        ctx.module, ctx.ws, ctx.x, ctx.tctx = module, ws, x, tctx
-        ctx.x_dtype = x_dtype
-        ctx.n_inputs = len(params)
+        with _on_device_of(x):
+            y, ctx.saved = module._train_forward(x)
+        ctx.module, ctx.tctx, ctx.n_inputs = module, tctx, len(params)
+        ctx.x_meta = (x.shape, x.dtype, x.device)
         ctx.direct = getattr(module, "_dg_direct_grads", False)
-        tctx.y = y
+        if tctx is not None:
+            tctx.y = y
         return y
 
     @staticmethod
     def backward(ctx, grad_y):
-        lib = _lib.load()
-        module, x, tctx = ctx.module, ctx.x, ctx.tctx
-        N, _, H, W = x.shape
+        module, tctx = ctx.module, ctx.tctx
+        if ctx.saved is None:
+            raise RuntimeError(f"{type(module).__name__}: backward through the same forward twice (the saved activations were "
+                               "released)")
         params = list(module.parameters())
-        total = sum(p.numel() for p in params)
-        # Only what autograd asks for is computed: dL/dx when x needs it, the gradients of parameters that require one, and the
-        # backward stops below the lowest of them.  GraphedTrainStep's parameters are not autograd inputs: it wants the trainable ones.
+        # Only what autograd asks for is computed: dL/dx when x needs it, the gradients of parameters that require one.
+        # GraphedTrainStep's parameters are not autograd inputs: it wants the trainable ones.
         want_x = ctx.needs_input_grad[2]
         want_p = [p.requires_grad for p in params] if ctx.direct else list(ctx.needs_input_grad[3:])
-        if len(want_p) != 64:
-            raise RuntimeError(f"gradient layout mismatch: {len(want_p)} parameter tensors, the library's backward has 64")
-        mask = sum(1 << k for k, w in enumerate(want_p) if w)
-        select = want_x or not all(want_p)
-        with torch.cuda.device(x.device):
-            pc = module._refresh(train=True)
-            nb = C.c_size_t(0)
-            _lib.check(lib.dg_lw_backward_workspace_bytes(C.byref(pc), N, H, W, C.byref(nb)))
-            bws = torch.empty(nb.value, dtype=torch.uint8, device=x.device)
-            cnt = C.c_size_t(0)
-            _lib.check(lib.dg_lw_num_params(C.byref(pc), C.byref(cnt)))
-            if cnt.value != total:
-                raise RuntimeError(f"gradient layout mismatch: library {cnt.value} vs module {total}")
-            # gradients go straight into the optimizer's flat bucket when that is safe (fresh after zero_grad, no hooks): no
-            # per-parameter accumulate kernels.  A bucket over a subset of the parameters is filled by one gather from the
-            # native full layout.  A fully frozen net gets no flat buffer at all.
-            sink = _flat_grad_sink(params, want_p) if total > 0 and mask else None
+        shape, x_dtype, dev = ctx.x_meta
+        grad_x = torch.empty(shape, dtype=torch.float32, device=dev) if want_x else None
+        with _on_device_of(grad_y):
+            # the optimizer's flat bucket when it is safe to write into (fresh after zero_grad, no hooks); a fully frozen net gets
+            # no gradient buffer at all
+            sink = _flat_grad_sink(params, want_p) if any(want_p) else None
             if ctx.direct and sink is None:
                 raise RuntimeError("GraphedTrainStep: the gradients must land in the optimizer's flat bucket (FusedAdamW.zero_grad "
                                    "inside the step, no per-parameter hooks)")
-            if sink is not None and sink.numel() == total:
-                flat = sink
-            else:
-                flat = torch.empty(total, dtype=torch.float32, device=x.device) if mask else None
-            grad_x = torch.empty_like(x) if want_x else None
-            stream = torch.cuda.current_stream().cuda_stream
-            fused_l1 = (tctx.l1_target is not None and tctx.l1_marker is not None and grad_y.data_ptr() == tctx.l1_marker.data_ptr()
-                        and all(s == 0 for s in grad_y.stride()))
-            if not fused_l1:
-                grad_y = grad_y.detach().float().contiguous()
-            if select:
-                req = _lib.DgLwBwdRequest()
-                if fused_l1:
-                    req.y, req.target, req.loss_grad = tctx.y.data_ptr(), tctx.l1_target.data_ptr(), tctx.l1_scale.data_ptr()
-                else:
-                    req.grad_y = grad_y.data_ptr()
-                req.grads = flat.data_ptr() if flat is not None else None
-                req.param_mask = mask
-                req.grad_x = grad_x.data_ptr() if grad_x is not None else None
-                _lib.check(lib.dg_lw_backward_select(C.byref(pc), x.data_ptr(), C.byref(req), N, H, W, ctx.ws.data_ptr(),
-                                                     ctx.ws.numel(), bws.data_ptr(), bws.numel(), stream))
-            elif fused_l1:   # loss = L1Loss (below): the seed sign(y - t) * dloss / numel is generated inside the head backward
-                _lib.check(lib.dg_lw_backward_l1(C.byref(pc), x.data_ptr(), tctx.y.data_ptr(), tctx.l1_target.data_ptr(),
-                                                 tctx.l1_scale.data_ptr(), N, H, W, ctx.ws.data_ptr(), ctx.ws.numel(),
-                                                 bws.data_ptr(), bws.numel(), flat.data_ptr(), stream))
-            else:
-                _lib.check(lib.dg_lw_backward(C.byref(pc), x.data_ptr(), grad_y.data_ptr(), N, H, W, ctx.ws.data_ptr(),
-                                              ctx.ws.numel(), bws.data_ptr(), bws.numel(), flat.data_ptr(), stream))
-        ctx.ws = None
-        tctx.y = tctx.l1_target = tctx.l1_scale = tctx.l1_marker = None
-        if grad_x is not None and grad_x.dtype != ctx.x_dtype:
-            grad_x = grad_x.to(ctx.x_dtype)
-        if flat is None:
+            flat = module._train_backward(ctx.saved, grad_y, tctx, want_p, grad_x, sink)
+        ctx.saved = None
+        if tctx is not None:
+            tctx.y = tctx.l1_target = tctx.l1_scale = tctx.l1_marker = None
+        if grad_x is not None and grad_x.dtype != x_dtype:
+            grad_x = grad_x.to(x_dtype)
+        if not any(want_p):
             return (None, None, grad_x) + (None,) * ctx.n_inputs
-        if sink is not None and sink is not flat:
-            torch.index_select(flat, 0, _gather_index(module, params, want_p, flat.device), out=sink)
-            flat = sink
         sync_gradients(flat, getattr(module, "ddp_sync", True))   # parameter gradients only: dL/dx is per rank's own batch
         if sink is not None:
             sink._dg_zero_version = None      # the bucket now holds a gradient: a second backward must accumulate the ordinary way
             return (None, None, grad_x) + (None,) * ctx.n_inputs
+        full = flat.numel() == sum(p.numel() for p in params)
         grads, off = [], 0
         for p, want in zip(params, want_p):
             n = p.numel()
-            grads.append(flat[off:off + n].view_as(p) if want else None)   # a frozen range of `flat` is never written
-            off += n
+            grads.append(flat[off:off + n].view_as(p) if want else None)   # a frozen range is never written
+            off += n if want or full else 0
         return (None, None, grad_x, *grads)
 
 
@@ -231,8 +216,11 @@ def sync_gradients(flat, enabled=True, group=None):
     return flat
 
 
-def lightweight_forward_train(module, x):
-    tctx = _TrainCtx()
+def train_forward(module, x):
+    """The forward of `module` (LightweightUNet, OptimizedUNet) recorded for autograd through `_TrainFn`.  Only a module whose
+    backward consumes `L1Loss`'s seed (class flag `_fused_l1`) gets an output that `L1Loss` fuses: any other module would be handed
+    the stride-0 dL/dloss marker as if it were dL/dy."""
+    tctx = _TrainCtx() if getattr(module, "_fused_l1", False) else None
     if getattr(module, "_dg_direct_grads", False):
         if x.requires_grad:
             raise NotImplementedError("GraphedTrainStep computes parameter gradients only, not the input image's")
@@ -240,12 +228,12 @@ def lightweight_forward_train(module, x):
         # on (the default stream if an eager step's graph is still alive), and the engine would synchronise the capturing stream
         # with it at the end of backward (cudaErrorStreamCaptureIsolation).  A fresh leaf anchors the node instead; the gradients
         # go straight into the optimizer's flat bucket.
-        anchor = torch.zeros((), device=x.device, requires_grad=True)
-        y = _LightweightUNetFn.apply(module, tctx, x, anchor)
+        inputs = (torch.zeros((), device=x.device, requires_grad=True),)
+    else:
+        inputs = tuple(module.parameters())
+    y = _TrainFn.apply(module, tctx, x, *inputs)
+    if tctx is not None:
         y._dg_train_ctx = tctx
-        return y
-    y = _LightweightUNetFn.apply(module, tctx, x, *module.parameters())
-    y._dg_train_ctx = tctx
     return y
 
 
@@ -288,19 +276,12 @@ class FusedAdamW(torch.optim.Optimizer):
                 self.flat_p[off:off + k].copy_(p.reshape(-1))
                 p.data = self.flat_p[off:off + k].view_as(p)     # parameters become views of the flat buffer
                 off += k
-        self._attach_grads()
+        _alias_grads(self.flat_g, ps)
 
     def add_param_group(self, param_group):
         if getattr(self, "param_groups", None):
             raise ValueError("FusedAdamW supports a single param group")
         super().add_param_group(param_group)
-
-    def _attach_grads(self):
-        off = 0
-        for p in self._ps:
-            k = p.numel()
-            p.grad = self.flat_g[off:off + k].view_as(p)
-            off += k
 
     def _publish_state(self):
         """Expose the flat moments through `self.state` in torch.optim.AdamW's layout (views, no copies)."""
@@ -360,9 +341,7 @@ class FusedAdamW(torch.optim.Optimizer):
 
     def zero_grad(self, set_to_none=True):
         # the reference calls zero_grad(set_to_none=True) (optimized_train.py:201); keep the flat aliasing instead
-        self.flat_g.zero_()
-        self.flat_g._dg_zero_version = self.flat_g._version   # all-zero as of this version: backward may write into it directly
-        self._attach_grads()
+        _zero_grads(self.flat_g, self._ps)
 
     def _gather(self):
         off = 0

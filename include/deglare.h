@@ -173,7 +173,7 @@ int dg_channel_attention(const double* act_sum, double plane, const float* w1, c
                          int32_t hidden, float* scale, dg_stream_t stream);
 
 /* ---- per-op backward (autograd of the pieces above; OptimizedUNet training, src/optimized_model.py:118-158 under
- * optimized_train.py:210/226, is orchestrated above the C-ABI from these; LightweightUNet uses dg_lw_backward) --------
+ * optimized_train.py:210/226, is orchestrated above the C-ABI from these; LightweightUNet uses dg_lw_backward_select) -
  * Notation per conv i: R = its raw output, y = GroupNorm(R), A = SiLU(y).  Gradient tensors are fp32 NHWC.
  *
  * dg_head1x1_bwd: backward of dg_head1x1 (src/optimized_model.py:74,158) for grad_y = dL/d(out) fp32 [N,cout,H,W] (cout <= 4):

@@ -135,7 +135,7 @@ def test_selective_backward_computes_only_what_requests_read(golden, monkeypatch
 def test_selective_backward_compact_layout_and_bridge(golden, monkeypatch):
     """`flat` holding only the requested tensors (the optimizer's bucket over the trainable subset) gets the same values as the
     full layout, and the autograd bridge returns gradients only for parameters that require one."""
-    from image_enhancement_deglaring_b200.model_optimized import _OptimizedUNetFn
+    from image_enhancement_deglaring_b200.train import train_forward
     net, sd = _net(golden, monkeypatch)
     x = _rand((1, 1, 32, 32), 3)
     gy = torch.randn(1, 1, 32, 32, generator=torch.Generator().manual_seed(4)) / x.numel()
@@ -159,7 +159,7 @@ def test_selective_backward_compact_layout_and_bridge(golden, monkeypatch):
         net._backward(keep, gy, torch.zeros(7), want)
     for k, p in net.named_parameters():
         p.requires_grad_(DECODER(k))
-    y = _OptimizedUNetFn.apply(net, x, *net.parameters())
+    y = train_forward(net, x)
     (y * gy).sum().backward()
     for k, p in net.named_parameters():
         if DECODER(k):
@@ -170,12 +170,9 @@ def test_selective_backward_compact_layout_and_bridge(golden, monkeypatch):
 
 def _bucket(params, order):
     """A fresh FusedAdamW-style flat bucket whose views are the .grads of `order`."""
-    flat = torch.zeros(sum(p.numel() for p in order))
-    off = 0
-    for p in order:
-        p.grad = flat[off:off + p.numel()].view_as(p)
-        off += p.numel()
-    flat._dg_zero_version = flat._version
+    from image_enhancement_deglaring_b200.train import _zero_grads
+    flat = torch.empty(sum(p.numel() for p in order))
+    _zero_grads(flat, order)
     return flat
 
 

@@ -58,18 +58,20 @@ def test_orchestration_reproduces_oracle_gradients(golden, monkeypatch, shape, s
 
 
 def test_autograd_bridge_returns_gradients_in_parameter_order(golden, monkeypatch):
-    from image_enhancement_deglaring_b200.model_optimized import _OptimizedUNetFn
+    from image_enhancement_deglaring_b200.train import train_forward
     net, sd = _net(golden, monkeypatch)
     x, t = _rand((1, 1, 32, 32), 3), _rand((1, 1, 32, 32), 4)
     r = tpo.train_step(sd, x, t, forward=tpo.optimized_forward, max_norm=0.0)
-    y = _OptimizedUNetFn.apply(net, x, *net.parameters())
+    y = train_forward(net, x)
     loss = torch.nn.L1Loss()(y, t)
-    loss.backward()
+    loss.backward(retain_graph=True)
     assert abs(float(loss.detach()) - r["loss"]) <= 1e-5 * max(1.0, r["loss"])
     for k, p in net.named_parameters():
         ref = r["grads"][k]
         assert p.grad is not None and p.grad.shape == ref.shape, k
         assert float((p.grad - ref).abs().max()) <= 2e-5 + 1e-3 * float(ref.abs().max()), k
+    with pytest.raises(RuntimeError, match="backward through the same forward twice"):
+        loss.backward()              # the saved activations were released by the first backward
     with pytest.raises(RuntimeError, match="CUDA"):
         net(x)                       # the public forward still refuses CPU tensors: no CPU fallback in the product
 
@@ -80,7 +82,7 @@ def _opt_ddp_worker(rank, world, port, out):
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
     from image_enhancement_deglaring_b200 import ops
-    from image_enhancement_deglaring_b200.model_optimized import _OptimizedUNetFn
+    from image_enhancement_deglaring_b200.train import train_forward
     for name in opt_standins.STANDINS:
         setattr(ops, name, getattr(opt_standins, name))
     g = np.load(os.path.join(os.path.dirname(__file__), "golden", "opt_rand.npz"), allow_pickle=False)
@@ -89,7 +91,7 @@ def _opt_ddp_worker(rank, world, port, out):
     net = dg.OptimizedUNet()
     net.load_state_dict(sd, strict=True)
     x, t = _rand((2, 1, 16, 32), 3), _rand((2, 1, 16, 32), 4)
-    y = _OptimizedUNetFn.apply(net, x[rank:rank + 1], *net.parameters())      # one image per rank
+    y = train_forward(net, x[rank:rank + 1])      # one image per rank
     torch.nn.L1Loss()(y, t[rank:rank + 1]).backward()
     flat = torch.cat([p.grad.reshape(-1) for p in net.parameters()])
     gathered = [torch.empty_like(flat) for _ in range(world)]
